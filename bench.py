@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
         --master-port 29500 bench.py --gpus 8 --steps 5 --warmup 3
     python bench.py --impl reference ...      # CPU arm: the oracle (restated interior point, NOT Ipopt)
+    python bench.py ... --dump-outputs DIR    # also the last timed step's results as DIR/*.npy, to compare two builds
 
 A step = one pass of the hot path (cold-start solve of every problem of the batch) over one
 synthetic batch: BASELINE.json configs[2], 65,536 problems per GPU at N=20 along paths 1-3
@@ -46,7 +47,32 @@ def parse():
     ap.add_argument("--x0", dest="start", default="zero", choices=["zero", "rollout"],
                     help="start point: zero = the reference's start=0.0 (the metric); rollout = MPCB200_START_ROLLOUT "
                          "(opt-in; what the horizon sweep of configs[4] uses at N = 40 / 80)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (u0, cost, status, iters, restorations, "
+                         "one row per problem) as DIR/<name>.npy in float64, with the problems' ids in DIR/index.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT = 64 << 20   # bytes of .npy data written by --dump-outputs
+
+
+def dump_outputs(out_dir, index, arrays):
+    """Writes arrays (one row per problem; index = the problems' ids in the synthetic stream) as out_dir/<name>.npy in
+    float64.  When they exceed DUMP_LIMIT in all, a fixed, seeded sample of the rows is written instead."""
+    index = np.asarray(index)
+    n = index.shape[0]
+    row_bytes = 8 * (1 + sum(int(np.prod(a.shape[1:])) for a in arrays.values()))
+    rows = np.arange(n)
+    if n * row_bytes > DUMP_LIMIT - 4096 * (1 + len(arrays)):     # room for the .npy headers
+        k = (DUMP_LIMIT - 4096 * (1 + len(arrays))) // row_bytes
+        rows = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "index.npy"), index[rows].astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(np.asarray(a)[rows], dtype=np.float64))
 
 
 class ClockSampler(object):
@@ -211,9 +237,13 @@ def run_reference(args):
         cpu_baseline(N, min(sample, 256), cores, start=args.start)
     t_tot, conv_tot = 0.0, 0
     for s in range(args.steps):
-        v, dt, conv, _ = cpu_baseline(N, sample, cores, start_b0=s * sample, start=args.start)
+        v, dt, conv, r = cpu_baseline(N, sample, cores, start_b0=s * sample, start=args.start)
         t_tot += dt
         conv_tot += conv
+    if args.dump_outputs:
+        s = args.steps - 1
+        dump_outputs(args.dump_outputs, np.arange(s * sample, (s + 1) * sample),
+                     {"u0": r["u0"], "cost": r["cost"], "status": r["status"], "iters": r["iters"], "restorations": r["n_resto"]})
     val = conv_tot / t_tot
     line = {
         "impl": "reference", "metric": "converged MPC solves/sec at batch 64K, N=20", "value": val,
@@ -355,6 +385,12 @@ def main():
     u0, cost, status, iters, resto = sharding.unpack_records_np(d_rec.cpu().numpy())
     u0 = u0.copy(); cost = cost.copy()
     optimal_local = int((status == 0).sum())
+    if args.dump_outputs and rank == 0:
+        # the records of the last timed step: this rank's, or every rank's after the all-gather
+        ru0, rcost, rstatus, riters, rresto = (sharding.unpack_records_np(d_all.cpu().numpy()) if world > 1
+                                               else (u0, cost, status, iters, resto))
+        dump_outputs(args.dump_outputs, np.arange(ru0.shape[0]),
+                     {"u0": ru0, "cost": rcost, "status": rstatus, "iters": riters, "restorations": rresto})
 
     # ---- parity against the oracle on EVERY problem of this rank's slice (SURVEY 8d: converged = Optimal AND within
     # tolerance of the oracle); at one GPU this run is also the cpu_baseline (the oracle timed on the box's cores)
