@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define MPCB200_VERSION 2
+#define MPCB200_VERSION 3
 
 /* error codes */
 #define MPCB200_OK          0
@@ -137,6 +137,19 @@ int mpcb200_solve_batch(mpcb200_handle* h, int64_t B,
                         double* traj, int32_t mem_space);
 
 /*
+ * mpcb200_solve_batch with one cost-weight row per problem: w [B][8] in update_cost order (cx, cy, cp, cv, cda, cdd, ca, cd),
+ * so one batch can hold controllers with different tunings (a weight sweep is one call).  The handle's own weights
+ * (mpcb200_set_cost) are neither used nor changed by this call.  A weight is valid by mpcb200_set_cost's rule (not negative, not
+ * NaN): with MPCB200_HOST pointers a bad row is refused (MPCB200_EINVAL, the message names the problem and the weight index); with
+ * MPCB200_DEVICE pointers that problem alone comes back with MPCB200_ERROR, zero commands, cost 0, 0 iterations and 0 restorations.
+ * Everything else -- both device layouts (mpcb200_set_large_batch_path), multi-GPU slicing, the small-batch path,
+ * mpcb200_get_stats and mpcb200_get_restorations -- as in mpcb200_solve_batch.  w is required.
+ */
+int mpcb200_solve_batch_w(mpcb200_handle* h, int64_t B, const double* state, const double* ref, const double* v_des,
+                          const double* u_prev, double* warm, const double* w,
+                          double* u0, double* cost, int32_t* status, int32_t* iters, double* traj, int32_t mem_space);
+
+/*
  * mpcb200_solve_batch whose per-problem results come back as ONE packed 32-byte record
  *   rec [B][4] doubles = { accel_cmd, steer_angle_cmd, cost, (int32 status | restorations << 8, int32 iters) }
  * written by the solve kernel itself: the unit of the multi-GPU exchange (one all-gather of these records is the only
@@ -194,6 +207,13 @@ int mpcb200_rollout(mpcb200_handle* h, int64_t B, int32_t T,
                     int32_t track_using_time, double target_vel,
                     double* log, double* final_state);
 
+/* mpcb200_rollout with one cost-weight row per vehicle, w [B][8] in update_cost order, used in every control period of that
+ * vehicle (a closed-loop tuning sweep in one call).  Rows are checked as by mpcb200_solve_batch_w with host pointers.  The first
+ * solve of every vehicle still starts from the module-load solution of the default problem (the node loads the module before any
+ * update_cost).  Host pointers only; same kernels, same fused / per-period switch and same sharding as mpcb200_rollout. */
+int mpcb200_rollout_w(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of,
+                      int32_t track_using_time, double target_vel, const double* w, double* log, double* final_state);
+
 /*
  * Frenet-frame variant of the same solver: scripts/mpc_utils/MKZMPCPathFollowerFrenet.jl (the model the Gazebo
  * lane-keep node gazebo_sim_mpc_cmd_pub_frenet.jl:112-153 drives).  Same vehicle constants, horizon, bounds, rate
@@ -214,6 +234,11 @@ int mpcb200_set_cost_frenet(mpcb200_handle* h, const double w[7]);
 int mpcb200_solve_batch_frenet(mpcb200_handle* h, int64_t B, const double* state, const double* k_coeffs,
                                const double* v_des, const double* u_prev, double* warm, double* u0,
                                double* cost, int32_t* status, int32_t* iters, double* traj, int32_t mem_space);
+/* mpcb200_solve_batch_frenet with one cost-weight row per problem: w [B][7] in the update_cost order of
+ * MKZMPCPathFollowerFrenet.jl (cey, cep, cev, cda, cdd, ca, cd); validation and everything else as mpcb200_solve_batch_w. */
+int mpcb200_solve_batch_frenet_w(mpcb200_handle* h, int64_t B, const double* state, const double* k_coeffs,
+                                 const double* v_des, const double* u_prev, double* warm, const double* w,
+                                 double* u0, double* cost, int32_t* status, int32_t* iters, double* traj, int32_t mem_space);
 
 /*
  * Closed loop on the Frenet-frame module, on the device (scripts/nodes_gazebo_sim/gazebo_sim_mpc_cmd_pub_frenet.jl:112-153

@@ -56,14 +56,17 @@ def lib():
     L.mpcb200_set_stream.argtypes = [vp, vp]
     L.mpcb200_set_large_batch_path.argtypes = [vp, C.c_int64]
     L.mpcb200_solve_batch.argtypes = [vp, C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int32]
+    L.mpcb200_solve_batch_w.argtypes = [vp, C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int32]
     L.mpcb200_solve_batch_records.argtypes = [vp, C.c_int64, vp, vp, vp, vp, vp, vp, vp, C.c_int32]
     L.mpcb200_get_restorations.argtypes = [vp, C.c_int64, vp]
     L.mpcb200_create_frenet.argtypes = [C.POINTER(vp), C.POINTER(Config)]
     L.mpcb200_set_cost_frenet.argtypes = [vp, dp]
     L.mpcb200_solve_batch_frenet.argtypes = [vp, C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int32]
+    L.mpcb200_solve_batch_frenet_w.argtypes = [vp, C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int32]
     L.mpcb200_solve_batch_on_path.argtypes = [vp, C.c_int64, vp, vp, C.c_int32, C.c_double, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int32]
     L.mpcb200_set_path.argtypes = [vp, C.c_int32, C.c_int32, dp, dp, dp, dp, dp]
     L.mpcb200_rollout.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_int32, C.c_double, dp, dp]
+    L.mpcb200_rollout_w.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_int32, C.c_double, dp, dp, dp]
     L.mpcb200_rollout_frenet.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_double, C.c_double, C.c_int32, dp, dp]
     L.mpcb200_get_stats.argtypes = [vp, C.POINTER(Stats)]
     L.mpcb200_fp64_peak.argtypes = [vp, dp]
@@ -98,6 +101,21 @@ def _ptr(a):
     if isinstance(a, np.ndarray):
         return a.ctypes.data
     return a.data_ptr()  # torch tensor
+
+
+def _weight_rows(weights, B, n, who):
+    """Per-problem cost weights: (B, n) float64 numpy array (host calls)."""
+    w = np.ascontiguousarray(weights, dtype=np.float64)
+    if w.shape != (B, n):
+        raise ValueError("%s: weights must be (B,%d) = (%d,%d), got %s" % (who, n, B, n, w.shape))
+    return w
+
+
+def _weight_rows_device(weights, B, n, who):
+    """Per-problem cost weights on the device: a (B, n) tensor, passed as it is (float64, contiguous)."""
+    if tuple(weights.shape) != (B, n):
+        raise ValueError("%s: weights must be (B,%d) = (%d,%d), got %s" % (who, n, B, n, tuple(weights.shape)))
+    return weights
 
 
 class Solver(object):
@@ -141,9 +159,11 @@ class Solver(object):
     def set_stream(self, cuda_stream_ptr):
         self._check(lib().mpcb200_set_stream(self._h, C.c_void_p(cuda_stream_ptr)))
 
-    def solve_batch(self, state, ref, u_prev, v_des=None, warm=None, want_traj=False, want_aux=True):
+    def solve_batch(self, state, ref, u_prev, v_des=None, warm=None, want_traj=False, want_aux=True, weights=None):
         """Host (numpy) arrays in, numpy arrays out.  state (B,4); ref (B,3,N+1); u_prev (B,2)
-        = (d_f_current, acc_current); v_des (B,) or None; warm (B,6N+4) in/out or None."""
+        = (d_f_current, acc_current); v_des (B,) or None; warm (B,6N+4) in/out or None.
+        weights (B,8) in update_cost order (cx, cy, cp, cv, cda, cdd, ca, cd), one row per problem (mpcb200_solve_batch_w),
+        or None: the handle's weights (set_cost)."""
         N = self.N
         state = np.ascontiguousarray(state, dtype=np.float64)
         B = state.shape[0]
@@ -164,8 +184,13 @@ class Solver(object):
         status = np.empty(B, dtype=np.int32) if want_aux else None
         iters = np.empty(B, dtype=np.int32) if want_aux else None
         traj = np.empty((B, 6 * N + 4)) if want_traj else None
-        self._check(lib().mpcb200_solve_batch(self._h, B, _ptr(state), _ptr(ref), _ptr(v_des), _ptr(u_prev), _ptr(warm),
-                                              _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), HOST))
+        if weights is None:
+            self._check(lib().mpcb200_solve_batch(self._h, B, _ptr(state), _ptr(ref), _ptr(v_des), _ptr(u_prev), _ptr(warm),
+                                                  _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), HOST))
+        else:
+            w = _weight_rows(weights, B, 8, "solve_batch")
+            self._check(lib().mpcb200_solve_batch_w(self._h, B, _ptr(state), _ptr(ref), _ptr(v_des), _ptr(u_prev), _ptr(warm), _ptr(w),
+                                                    _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), HOST))
         return {"u0": u0, "cost": cost, "status": status, "iters": iters, "traj": traj}
 
     def solve_batch_on_path(self, state, path_of, u_prev, track_using_time=True, target_vel=1.0, v_des=None, warm=None,
@@ -232,11 +257,17 @@ class Solver(object):
         return out
 
     def solve_batch_device(self, B, state, ref, u_prev, u0, v_des=None, warm=None, cost=None, status=None,
-                           iters=None, traj=None):
+                           iters=None, traj=None, weights=None):
         """Device pointers (torch CUDA tensors, float64 / int32, contiguous); only enqueues on the
-        handle's stream."""
-        self._check(lib().mpcb200_solve_batch(self._h, B, _ptr(state), _ptr(ref), _ptr(v_des), _ptr(u_prev), _ptr(warm),
-                                              _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), DEVICE))
+        handle's stream.  weights: (B,8) float64 tensor, one row per problem (a bad row gives that problem
+        status ERROR), or None: the handle's weights."""
+        if weights is None:
+            self._check(lib().mpcb200_solve_batch(self._h, B, _ptr(state), _ptr(ref), _ptr(v_des), _ptr(u_prev), _ptr(warm),
+                                                  _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), DEVICE))
+        else:
+            w = _weight_rows_device(weights, B, 8, "solve_batch_device")
+            self._check(lib().mpcb200_solve_batch_w(self._h, B, _ptr(state), _ptr(ref), _ptr(v_des), _ptr(u_prev), _ptr(warm), _ptr(w),
+                                                    _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), DEVICE))
 
     def set_path(self, path_id, traj_table):
         """traj_table: the (n,7) table of GPSRefTrajectory.trajectory (ref_gps_traj.py:106); path_id 0..2."""
@@ -244,9 +275,10 @@ class Solver(object):
         dp = C.POINTER(C.c_double)
         self._check(lib().mpcb200_set_path(self._h, int(path_id), int(traj_table.shape[0]), *[c.ctypes.data_as(dp) for c in cols]))
 
-    def rollout(self, pose0, path_of, T, track_using_time=True, target_vel=1.0, want_log=True):
+    def rollout(self, pose0, path_of, T, track_using_time=True, target_vel=1.0, want_log=True, weights=None):
         """Closed-loop Monte-Carlo rollout on the device (mpcb200_rollout).  pose0 (B,3); path_of (B,) in 0..2
-        (ids given to set_path).  Returns log (T,B,8) = x,y,psi,v,acc_cmd,df_cmd,status,iters and final (B,8)."""
+        (ids given to set_path).  Returns log (T,B,8) = x,y,psi,v,acc_cmd,df_cmd,status,iters and final (B,8).
+        weights (B,8): each vehicle's cost weights for all its control periods (mpcb200_rollout_w), or None: the handle's."""
         pose0 = np.ascontiguousarray(np.atleast_2d(pose0), dtype=np.float64)
         B = pose0.shape[0]
         path_of = np.ascontiguousarray(path_of, dtype=np.int32)
@@ -255,9 +287,13 @@ class Solver(object):
         log = np.empty((T, B, 8)) if want_log else None
         final = np.empty((B, 8))
         dp = C.POINTER(C.c_double)
-        self._check(lib().mpcb200_rollout(self._h, B, int(T), pose0.ctypes.data_as(dp), path_of.ctypes.data_as(C.POINTER(C.c_int32)),
-                                          int(bool(track_using_time)), float(target_vel),
-                                          None if log is None else log.ctypes.data_as(dp), final.ctypes.data_as(dp)))
+        args = [pose0.ctypes.data_as(dp), path_of.ctypes.data_as(C.POINTER(C.c_int32)), int(bool(track_using_time)), float(target_vel)]
+        outs = [None if log is None else log.ctypes.data_as(dp), final.ctypes.data_as(dp)]
+        if weights is None:
+            self._check(lib().mpcb200_rollout(self._h, B, int(T), *args, *outs))
+        else:
+            w = _weight_rows(weights, B, 8, "rollout")
+            self._check(lib().mpcb200_rollout_w(self._h, B, int(T), *args, w.ctypes.data_as(dp), *outs))
         return {"log": log, "final_state": final}
 
     def stats(self):
@@ -288,9 +324,10 @@ class FrenetSolver(Solver):
         """Batches of at least `min_batch` problems use the thread-per-problem kernel (TppSolverT<1>); 0: never; < 0: the default rule."""
         self._check(lib().mpcb200_set_large_batch_path(self._h, int(min_batch)))
 
-    def solve_batch(self, state, k_coeffs, u_prev, v_des=None, warm=None, want_traj=False, want_aux=True):
+    def solve_batch(self, state, k_coeffs, u_prev, v_des=None, warm=None, want_traj=False, want_aux=True, weights=None):
         """state (B,4) = s, ey, epsi, v; k_coeffs (B,4) highest degree first; u_prev (B,2) = (d_f_current, acc_current);
-        warm / traj (B,6N+4) = s, ey, v, epsi, d_f, acc."""
+        warm / traj (B,6N+4) = s, ey, v, epsi, d_f, acc.  weights (B,7) in set_cost's order (cey, cep, cev, cda, cdd, ca, cd),
+        one row per problem (mpcb200_solve_batch_frenet_w), or None: the handle's weights."""
         N = self.N
         state = np.ascontiguousarray(state, dtype=np.float64)
         B = state.shape[0]
@@ -311,8 +348,13 @@ class FrenetSolver(Solver):
         status = np.empty(B, dtype=np.int32) if want_aux else None
         iters = np.empty(B, dtype=np.int32) if want_aux else None
         traj = np.empty((B, 6 * N + 4)) if want_traj else None
-        self._check(lib().mpcb200_solve_batch_frenet(self._h, B, _ptr(state), _ptr(k_coeffs), _ptr(v_des), _ptr(u_prev), _ptr(warm),
-                                                     _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), HOST))
+        if weights is None:
+            self._check(lib().mpcb200_solve_batch_frenet(self._h, B, _ptr(state), _ptr(k_coeffs), _ptr(v_des), _ptr(u_prev), _ptr(warm),
+                                                         _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), HOST))
+        else:
+            w = _weight_rows(weights, B, 7, "solve_batch")
+            self._check(lib().mpcb200_solve_batch_frenet_w(self._h, B, _ptr(state), _ptr(k_coeffs), _ptr(v_des), _ptr(u_prev), _ptr(warm),
+                                                           _ptr(w), _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), HOST))
         return {"u0": u0, "cost": cost, "status": status, "iters": iters, "traj": traj}
 
     def rollout(self, pose0, path_of, T, window=40.0, target_vel=8.0, ey_from_path=True, want_log=True):
@@ -331,7 +373,14 @@ class FrenetSolver(Solver):
                                                  None if log is None else log.ctypes.data_as(dp), final.ctypes.data_as(dp)))
         return {"log": log, "final_state": final}
 
-    def solve_batch_device(self, B, state, k_coeffs, u_prev, u0, v_des=None, warm=None, cost=None, status=None, iters=None, traj=None):
-        """Device pointers (torch CUDA tensors or ints); asynchronous on the handle's stream."""
-        self._check(lib().mpcb200_solve_batch_frenet(self._h, B, _ptr(state), _ptr(k_coeffs), _ptr(v_des), _ptr(u_prev), _ptr(warm),
-                                                     _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), DEVICE))
+    def solve_batch_device(self, B, state, k_coeffs, u_prev, u0, v_des=None, warm=None, cost=None, status=None, iters=None, traj=None,
+                           weights=None):
+        """Device pointers (torch CUDA tensors or ints); asynchronous on the handle's stream.  weights: (B,7) float64 tensor, one row
+        per problem (a bad row gives that problem status ERROR), or None: the handle's weights."""
+        if weights is None:
+            self._check(lib().mpcb200_solve_batch_frenet(self._h, B, _ptr(state), _ptr(k_coeffs), _ptr(v_des), _ptr(u_prev), _ptr(warm),
+                                                         _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), DEVICE))
+        else:
+            w = _weight_rows_device(weights, B, 7, "solve_batch_device")
+            self._check(lib().mpcb200_solve_batch_frenet_w(self._h, B, _ptr(state), _ptr(k_coeffs), _ptr(v_des), _ptr(u_prev), _ptr(warm),
+                                                           _ptr(w), _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), DEVICE))

@@ -29,21 +29,25 @@ constexpr int WARPS_PER_BLOCK = 4;
 // 168 registers per thread: three blocks (12 warps) per SM at the N = 20 shared-memory footprint.
 // The iterate's bound multipliers, the step and the model evaluation live in per-thread shared-memory
 // fields (mpc_kernel.cuh, LF_*), which is what lets the solver fit.
+//
+// PW (every solve kernel below): 1 = each problem's cost weights from io.w (mpcb200_solve_batch_w / _frenet_w), 0 = KCfg::w.
+// A compile-time switch, so that the PW = 0 instantiations the unweighted entry points launch are the code they always were.
 #ifndef MPC_MIN_BLOCKS
 #define MPC_MIN_BLOCKS 3
 #endif
+template <int PW>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, MPC_MIN_BLOCKS)
 mpc_solve_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const long long B, unsigned long long* counter) {
     extern __shared__ double smem_all[];
     const int warp = threadIdx.x >> 5;
-    const smem_t smem = smem_base(smem_all + (size_t)warp * smem_doubles_per_team(cfg.N));
+    const smem_t smem = smem_base(smem_all + (size_t)warp * smem_doubles_per_team(cfg.N, 0, PW));
     TeamSolver<1>::init_work(smem, cfg.N);
     for (;;) {
         unsigned long long b = 0;
         if ((threadIdx.x & 31) == 0) b = atomicAdd(counter, 1ULL);
         b = __shfl_sync(0xffffffffu, b, 0);
         if (b >= (unsigned long long)B) break;
-        solve_problem<1>(cfg, io, rg, (long)b, smem);
+        solve_problem<1, 0, PW>(cfg, io, rg, (long)b, smem);
         __syncwarp();
     }
 }
@@ -52,19 +56,19 @@ mpc_solve_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const long
 // 62-double records, 21.3 KB of shared memory per problem at N = 20.  Two builds: blocks of four warps at 255 registers
 // (two per SM) and blocks of three at 168 registers with spill code (up to four per SM: 12 warps at the N = 8 footprint);
 // mpcb200_create_frenet picks per horizon (see there)
-template <int WPB>
+template <int WPB, int PW = 0>
 __global__ void __launch_bounds__(WPB * 32, WPB == 3 ? 3 : 2)
 mpc_solve_frenet_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const long long B, unsigned long long* counter) {
     extern __shared__ double smem_all[];
     const int warp = threadIdx.x >> 5;
-    const smem_t smem = smem_base(smem_all + (size_t)warp * smem_doubles_per_team(cfg.N, 1));
+    const smem_t smem = smem_base(smem_all + (size_t)warp * smem_doubles_per_team(cfg.N, 1, PW));
     TeamSolver<1, 1>::init_work(smem, cfg.N);
     for (;;) {
         unsigned long long b = 0;
         if ((threadIdx.x & 31) == 0) b = atomicAdd(counter, 1ULL);
         b = __shfl_sync(0xffffffffu, b, 0);
         if (b >= (unsigned long long)B) break;
-        solve_problem<1, 1>(cfg, io, rg, (long)b, smem);
+        solve_problem<1, 1, PW>(cfg, io, rg, (long)b, smem);
         __syncwarp();
     }
 }
@@ -75,7 +79,7 @@ mpc_solve_frenet_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, con
 #define MPC_LONG_MIN_BLOCKS2 6
 #define MPC_LONG_MIN_BLOCKS3 2
 #endif
-template <int W, int MODEL = 0>
+template <int W, int MODEL = 0, int PW = 0>
 __global__ void __launch_bounds__(W * 32, MODEL ? 2 : (W == 2 ? MPC_LONG_MIN_BLOCKS2 : MPC_LONG_MIN_BLOCKS3))
 mpc_solve_long_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const long long B, unsigned long long* counter) {
     extern __shared__ double smem_all[];
@@ -88,7 +92,7 @@ mpc_solve_long_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const
         const unsigned long long b = next_problem;
         __syncthreads();
         if (b >= (unsigned long long)B) break;
-        solve_problem<W, MODEL>(cfg, io, rg, (long)b, smem);
+        solve_problem<W, MODEL, PW>(cfg, io, rg, (long)b, smem);
     }
 }
 
@@ -101,19 +105,20 @@ mpc_solve_long_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const
 #define MPC_TPP_BLOCK 256
 #define MPC_TPP_MIN_BLOCKS 1
 #endif
-template <int MODEL>
+template <int MODEL, int PW = 0>
 __global__ void __launch_bounds__(MPC_TPP_BLOCK, MPC_TPP_MIN_BLOCKS)
 mpc_solve_tpp_kernel(const KCfg cfg, const BatchPtrs io, const long long B, double* st, double* filt, unsigned long long* counter,
                      const double v_des0) {
     const long slot = (long)blockIdx.x * blockDim.x + threadIdx.x;
     const TppMemT<MODEL> mem(st, filt, cfg.N, slot);
-    TppSolverT<MODEL> sv(cfg, mem);
+    TppSolverT<MODEL, PW> sv(cfg, mem);
     bool alive = true;   // the counter has not run past the batch for this lane yet
     long b = -1;
     while (__syncthreads_or(alive)) {
         if (alive && b < 0) {
             const unsigned long long nb = atomicAdd(counter, 1ULL);
             if (nb >= (unsigned long long)B) alive = false;
+            else if (PW && io.w && !row_weights_ok(io.w, (long)nb, MODEL)) write_error_answer(io, (long)nb);   // the lane takes the next one
             else { b = (long)nb; sv.begin(io, b, v_des0); }
         }
         const bool done = sv.tick(b >= 0);
@@ -148,12 +153,7 @@ on_path_invalid_kernel(const long long B, const RefGen rg, const BatchPtrs io) {
     if (b >= B) return;
     const int pid = rg.path_of[b];
     if (!(pid < 0 || pid > 2 || rg.paths[pid].n < 2)) return;
-    if (io.u0) { io.u0[2 * b] = 0.0; io.u0[2 * b + 1] = 0.0; }
-    if (io.cost) io.cost[b] = 0.0;
-    if (io.status) io.status[b] = 4;
-    if (io.iters) io.iters[b] = 0;
-    if (io.rec) { st_global_v2(io.rec + 4 * b, 0.0, 0.0); st_global_v2(io.rec + 4 * b + 2, 0.0, int2_as_double(4, 0)); }
-    if (io.resto) io.resto[b] = 0;
+    write_error_answer(io, b);
 }
 
 // ---- Closed-loop fleets with the thread-per-problem layout: one control period = three launches over the whole fleet
@@ -206,14 +206,16 @@ rollout_waypoints_kernel(const KCfg cfg, const long long B, const long long Bp, 
 // MODEL 0: reference samples already in the slots, stop latch, the first solve from the module-load solution `warm0`.
 // MODEL 1 (closed loop of the Frenet node, gazebo_sim_mpc_cmd_pub_frenet.jl:112-153): `fref` = [6][Bp] curvature polynomial (4),
 // e_y, psi_start per vehicle from rollout_frenet_ref_kernel; state (0, e_y, -psi_start, v); the first solve from all zeros.
-template <int MODEL>
+// PW: each vehicle's cost weights from out.w (mpcb200_rollout_w), the slot keeps its vehicle and so its row
+template <int MODEL, int PW = 0>
 __global__ void __launch_bounds__(MPC_TPP_BLOCK, MPC_TPP_MIN_BLOCKS)
 rollout_solve_tpp_kernel(const KCfg cfg, const long long B, const long long Bp, double* veh, const int* stop, double* tpp_state, double* tpp_filt,
                          const double* warm0, const double des_speed, BatchPtrs out, double* log_row, const double* fref, const int first) {
     const long long v = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const bool valid = v < B;
     const TppMemT<MODEL> mem(tpp_state, tpp_filt, cfg.N, (long)(valid ? v : 0));
-    TppSolverT<MODEL> sv(cfg, mem);
+    TppSolverT<MODEL, PW> sv(cfg, mem);
+    if (PW && valid && out.w) sv.wr = out.w + 8 * v;
     const bool stopped = valid && !MODEL && stop[v] != 0;
     bool live = valid && !stopped;
     double st4[4] = {0.0, 0.0, 0.0, 0.0};
@@ -274,12 +276,14 @@ __global__ void rollout_final_kernel(const long long B, const long long Bp, cons
 #ifndef MPC_ROLLOUT_MIN_BLOCKS
 #define MPC_ROLLOUT_MIN_BLOCKS 3
 #endif
+// PW (this kernel and mpc_rollout_long_kernel): each vehicle's cost weights from args.w (mpcb200_rollout_w)
+template <int PW>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, MPC_ROLLOUT_MIN_BLOCKS)
 mpc_rollout_kernel(const KCfg cfg, const RolloutArgs args, unsigned long long* counter) {
     extern __shared__ double smem_all[];
     const int warp = threadIdx.x >> 5;
-    const smem_t smem = smem_base(smem_all + (size_t)warp * smem_doubles_per_team(cfg.N));
-    const smem_t px = smem_base(smem_all + (size_t)WARPS_PER_BLOCK * smem_doubles_per_team(cfg.N));   // plant exchange area
+    const smem_t smem = smem_base(smem_all + (size_t)warp * smem_doubles_per_team(cfg.N, 0, PW));
+    const smem_t px = smem_base(smem_all + (size_t)WARPS_PER_BLOCK * smem_doubles_per_team(cfg.N, 0, PW));   // plant exchange area
     __shared__ unsigned long long next_group;
     TeamSolver<1>::init_work(smem, cfg.N);
     for (;;) {   // the block takes WARPS_PER_BLOCK vehicles at a time and steps them together
@@ -288,18 +292,18 @@ mpc_rollout_kernel(const KCfg cfg, const RolloutArgs args, unsigned long long* c
         const unsigned long long b0 = next_group;
         __syncthreads();
         if (b0 >= (unsigned long long)args.B) break;
-        rollout_group<1>(cfg, args, (long)b0, smem, px, WARPS_PER_BLOCK);
+        rollout_group<1, PW>(cfg, args, (long)b0, smem, px, WARPS_PER_BLOCK);
     }
 }
 
 // Closed-loop rollouts at long horizons (32 <= N <= 95): one vehicle per block of W = 2 or 3 warps
-template <int W>
+template <int W, int PW = 0>
 __global__ void __launch_bounds__(W * 32, W == 2 ? 4 : 2)
 mpc_rollout_long_kernel(const KCfg cfg, const RolloutArgs args, unsigned long long* counter) {
     extern __shared__ double smem_all[];
     __shared__ unsigned long long next_vehicle;
     const smem_t smem = smem_base(smem_all);
-    const smem_t px = smem_base(smem_all + (size_t)smem_doubles_per_team(cfg.N));
+    const smem_t px = smem_base(smem_all + (size_t)smem_doubles_per_team(cfg.N, 0, PW));
     TeamSolver<W>::init_work(smem, cfg.N);
     for (;;) {
         if (threadIdx.x == 0) next_vehicle = atomicAdd(counter, 1ULL);
@@ -307,7 +311,7 @@ mpc_rollout_long_kernel(const KCfg cfg, const RolloutArgs args, unsigned long lo
         const unsigned long long b0 = next_vehicle;
         __syncthreads();
         if (b0 >= (unsigned long long)args.B) break;
-        rollout_group<W>(cfg, args, (long)b0, smem, px, 1);
+        rollout_group<W, PW>(cfg, args, (long)b0, smem, px, 1);
     }
 }
 
@@ -368,6 +372,9 @@ struct mpcb200_handle {
     DevBuf d_tpp_state, d_tpp_filt;   /* thread-per-problem path: slot state [warp][stage][field][lane], filters */
     DevBuf d_genref;                  /* ... on a path: the generated waypoints [B][3][N+1] when the caller did not ask for them */
     DevBuf d_veh, d_vstop;            /* ... closed-loop fleets: vehicle state [12][Bp], stop latches */
+    DevBuf d_w;                       /* per-problem weight rows of a weighted call (host pointers) */
+    int blocks_per_sm_w = 0;          /* resident blocks per SM of the PW = 1 solve kernel of this handle (8 more doubles per team) */
+    int rollout_blocks_per_sm_w = 0;  /* ... of the PW = 1 fused rollout kernel */
     int tpp_blocks_per_sm = 0;        /* resident blocks of mpc_solve_tpp_kernel per SM */
     int tpp_block = MPC_TPP_BLOCK;    /* threads per block of mpc_solve_tpp_kernel (a multiple of 32, <= MPC_TPP_BLOCK) */
     bool tpp_block_forced = false;    /* ... given by MPCB200_TPP_BLOCK: no per-batch choice */
@@ -392,7 +399,8 @@ struct mpcb200_handle {
     void* h_stage = nullptr;      /* its pinned host mirror */
     size_t h_stage_cap = 0;
     /* small batches on the handle's own stream: copy in -> kernel -> copy out captured once per shape as a CUDA graph
-     * (one cudaGraphLaunch instead of five driver calls per solve); dropped when a buffer, the weights or the stream change */
+     * (one cudaGraphLaunch instead of five driver calls per solve); dropped when a buffer, the handle's weights or the stream
+     * change.  A shape is B and which optional buffers the call has, per-problem weight rows included */
     struct SmallGraph { int64_t B; int flags; cudaGraphExec_t exec; };
     SmallGraph graphs[8];
     int n_graphs = 0;
@@ -462,6 +470,43 @@ static KCfg make_kcfg(const mpcb200_handle* h) {
     kcfg_finalize(k);
     k.roles = h->d_roles;
     return k;
+}
+
+/* problems per block of the warp / block-per-problem solve kernel */
+static int teams_per_block(const mpcb200_handle* h) { return (h->team_warps != 1) ? 1 : (h->model ? h->frenet_wpb : WARPS_PER_BLOCK); }
+
+/* the warp / block-per-problem solve kernel of a handle (model, team size, Frenet block size) and its threads per block */
+typedef void (*TeamKernel)(const KCfg, const BatchPtrs, const RefGen, const long long, unsigned long long*);
+template <int PW>
+static TeamKernel team_kernel(const mpcb200_handle* h, int* threads) {
+    *threads = 32 * h->team_warps;
+    if (h->model && h->team_warps == 2) return mpc_solve_long_kernel<2, 1, PW>;
+    if (h->model && h->team_warps == 3) return mpc_solve_long_kernel<3, 1, PW>;
+    if (h->model) { *threads = 32 * h->frenet_wpb; return (h->frenet_wpb == 3) ? mpc_solve_frenet_kernel<3, PW> : mpc_solve_frenet_kernel<4, PW>; }
+    if (h->team_warps == 1) { *threads = 32 * WARPS_PER_BLOCK; return mpc_solve_kernel<PW>; }
+    return (h->team_warps == 2) ? mpc_solve_long_kernel<2, 0, PW> : mpc_solve_long_kernel<3, 0, PW>;
+}
+
+/* the fused closed-loop kernel of an XY handle */
+typedef void (*RolloutKernel)(const KCfg, const RolloutArgs, unsigned long long*);
+template <int PW>
+static RolloutKernel rollout_kernel(const mpcb200_handle* h) {
+    if (h->team_warps == 1) return mpc_rollout_kernel<PW>;
+    return (h->team_warps == 2) ? mpc_rollout_long_kernel<2, PW> : mpc_rollout_long_kernel<3, PW>;
+}
+
+/* dynamic shared memory of the fused rollout kernel: the teams and the plant exchange area */
+static size_t rollout_smem_bytes(const mpcb200_handle* h, bool pw) {
+    return h->smem_bytes + (h->team_warps == 1 ? 0 : ROLLOUT_PX * sizeof(double)) + (pw ? (size_t)teams_per_block(h) * 8 * sizeof(double) : 0);
+}
+
+/* shared-memory limit, carveout and resident blocks per SM of one kernel */
+static cudaError_t prepare_kernel(const void* fn, int device, int threads, size_t bytes, int* blocks_per_sm) {
+    cudaError_t e = raise_dyn_smem(fn, device, bytes);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, fn, threads, bytes);
+    if (*blocks_per_sm < 1) *blocks_per_sm = 1;
+    return e;
 }
 
 extern "C" {
@@ -613,12 +658,12 @@ static int create_impl(mpcb200_handle** out, const mpcb200_config* cfg, int mode
         if (h->frenet_rollout_blocks_per_sm < 1) h->frenet_rollout_blocks_per_sm = 1;
     } else if (h->team_warps == 1) {
         h->smem_bytes = ((size_t)WARPS_PER_BLOCK * smem_doubles_per_team(cfg->N) + WARPS_PER_BLOCK * ROLLOUT_PX) * sizeof(double);
-        TRY_OR_FREE(raise_dyn_smem((const void*)mpc_solve_kernel, h->device, (size_t)(h->smem_bytes)));
-        TRY_OR_FREE(cudaFuncSetAttribute(mpc_solve_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        TRY_OR_FREE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->blocks_per_sm, mpc_solve_kernel, WARPS_PER_BLOCK * 32, h->smem_bytes));
-        TRY_OR_FREE(raise_dyn_smem((const void*)mpc_rollout_kernel, h->device, (size_t)(h->smem_bytes)));
-        TRY_OR_FREE(cudaFuncSetAttribute(mpc_rollout_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        TRY_OR_FREE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->rollout_blocks_per_sm, mpc_rollout_kernel, WARPS_PER_BLOCK * 32, h->smem_bytes));
+        TRY_OR_FREE(raise_dyn_smem((const void*)mpc_solve_kernel<0>, h->device, (size_t)(h->smem_bytes)));
+        TRY_OR_FREE(cudaFuncSetAttribute(mpc_solve_kernel<0>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        TRY_OR_FREE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->blocks_per_sm, mpc_solve_kernel<0>, WARPS_PER_BLOCK * 32, h->smem_bytes));
+        TRY_OR_FREE(raise_dyn_smem((const void*)mpc_rollout_kernel<0>, h->device, (size_t)(h->smem_bytes)));
+        TRY_OR_FREE(cudaFuncSetAttribute(mpc_rollout_kernel<0>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        TRY_OR_FREE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->rollout_blocks_per_sm, mpc_rollout_kernel<0>, WARPS_PER_BLOCK * 32, h->smem_bytes));
         if (h->rollout_blocks_per_sm < 1) h->rollout_blocks_per_sm = 1;
     } else {
         h->smem_bytes = (size_t)smem_doubles_per_team(cfg->N) * sizeof(double);
@@ -637,6 +682,8 @@ static int create_impl(mpcb200_handle** out, const mpcb200_config* cfg, int mode
         /* thread-per-problem path for large batches (any horizon): needs B >> resident lanes to keep them busy */
         const void* tk = model ? (const void*)mpc_solve_tpp_kernel<1> : (const void*)mpc_solve_tpp_kernel<0>;
         TRY_OR_FREE(cudaFuncSetAttribute(tk, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1));
+        const void* tkw = model ? (const void*)mpc_solve_tpp_kernel<1, 1> : (const void*)mpc_solve_tpp_kernel<0, 1>;
+        TRY_OR_FREE(cudaFuncSetAttribute(tkw, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxL1));
         TRY_OR_FREE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->tpp_blocks_per_sm, tk, MPC_TPP_BLOCK, 0));
         if (h->tpp_blocks_per_sm < 1) h->tpp_blocks_per_sm = 1;
         if (const char* e = getenv("MPCB200_TPP_BLOCKS_PER_SM")) { int v = atoi(e); if (v >= 1 && v < h->tpp_blocks_per_sm) h->tpp_blocks_per_sm = v; }  /* tuning aid */
@@ -645,6 +692,14 @@ static int create_impl(mpcb200_handle** out, const mpcb200_config* cfg, int mode
          * kernel at 16 K / 32 K / 64 K / 128 K problems; N = 12, 16: break-even at ~128 K; N = 20: 0.65x at 64 K, 0.97x at 256 K */
         h->tpp_min_batch = tpp_default_min_batch(model, cfg->N);
         if (const char* e = getenv("MPCB200_TPP_MIN_BATCH")) { h->tpp_min_batch = atoll(e); h->tpp_default_rule = false; }   /* tuning aid; 0 switches the path off */
+    }
+    {
+        /* the PW = 1 kernels of the weighted entry points: 8 more doubles of shared memory per team */
+        int threads = 0;
+        const void* fw = (const void*)team_kernel<1>(h, &threads);
+        TRY_OR_FREE(prepare_kernel(fw, h->device, threads, h->smem_bytes + (size_t)teams_per_block(h) * 8 * sizeof(double), &h->blocks_per_sm_w));
+        if (!model)
+            TRY_OR_FREE(prepare_kernel((const void*)rollout_kernel<1>(h), h->device, threads, rollout_smem_bytes(h, true), &h->rollout_blocks_per_sm_w));
     }
     if (h->blocks_per_sm < 1) h->blocks_per_sm = 1;
     if (const char* e = getenv("MPCB200_BLOCKS_PER_SM")) { int v = atoi(e); if (v >= 1 && v < h->blocks_per_sm) h->blocks_per_sm = v; }  /* tuning aid */
@@ -660,7 +715,8 @@ int mpcb200_destroy(mpcb200_handle* h) {
     cudaSetDevice(h->device);
     DevBuf* bufs[] = {&h->d_state, &h->d_ref, &h->d_vdes, &h->d_uprev, &h->d_warm, &h->d_u0, &h->d_cost, &h->d_status, &h->d_iters, &h->d_traj,
                       &h->d_path[0], &h->d_path[1], &h->d_path[2], &h->d_pose, &h->d_pathof, &h->d_log, &h->d_final, &h->d_stop, &h->d_stage,
-                      &h->d_rec, &h->d_resto, &h->d_seed, &h->d_fit, &h->d_tpp_state, &h->d_tpp_filt, &h->d_veh, &h->d_vstop, &h->d_genref};
+                      &h->d_rec, &h->d_resto, &h->d_seed, &h->d_fit, &h->d_tpp_state, &h->d_tpp_filt, &h->d_veh, &h->d_vstop, &h->d_genref,
+                      &h->d_w};
     for (DevBuf* b : bufs) if (b->p) cudaFree(b->p);
     if (h->d_counter) cudaFree(h->d_counter);
     if (h->d_roles) cudaFree(h->d_roles);
@@ -743,12 +799,8 @@ static int launch_solve(mpcb200_handle* h, int64_t B, const BatchPtrs& io, const
             h->stats.kernel_launches += 1;
         }
         const double v_des0 = rg.path_of ? rg.target_vel : 0.0;   /* des_speed when the caller gives no v_des, mpc_cmd_pub.jl:58-62,116 */
-        if (h->model)
-            mpc_solve_tpp_kernel<1><<<(int)blocks, tb, 0, h->stream>>>(make_kcfg(h), io2, (long long)B, (double*)h->d_tpp_state.p,
-                                                                      (double*)h->d_tpp_filt.p, counter, v_des0);
-        else
-            mpc_solve_tpp_kernel<0><<<(int)blocks, tb, 0, h->stream>>>(make_kcfg(h), io2, (long long)B, (double*)h->d_tpp_state.p,
-                                                                      (double*)h->d_tpp_filt.p, counter, v_des0);
+        auto tk = h->model ? (io.w ? mpc_solve_tpp_kernel<1, 1> : mpc_solve_tpp_kernel<1, 0>) : (io.w ? mpc_solve_tpp_kernel<0, 1> : mpc_solve_tpp_kernel<0, 0>);
+        tk<<<(int)blocks, tb, 0, h->stream>>>(make_kcfg(h), io2, (long long)B, (double*)h->d_tpp_state.p, (double*)h->d_tpp_filt.p, counter, v_des0);
         CUDA_TRY(h, cudaGetLastError());
         h->stats.kernel_launches += 1;
         if (rg.path_of) {
@@ -758,25 +810,16 @@ static int launch_solve(mpcb200_handle* h, int64_t B, const BatchPtrs& io, const
         }
         return 0;
     }
-    const int teams_per_block = (h->team_warps != 1) ? 1 : (h->model ? h->frenet_wpb : WARPS_PER_BLOCK);
-    long long blocks_needed = (B + teams_per_block - 1) / teams_per_block;
-    long long max_blocks = (long long)h->num_sms * h->blocks_per_sm;
+    const int tpb = teams_per_block(h);
+    const bool pw = io.w != nullptr;
+    long long blocks_needed = (B + tpb - 1) / tpb;
+    long long max_blocks = (long long)h->num_sms * (pw ? h->blocks_per_sm_w : h->blocks_per_sm);
     int grid = (int)(blocks_needed < max_blocks ? blocks_needed : max_blocks);
     if (grid < 1) grid = 1;
-    if (h->model && h->team_warps == 2)
-        mpc_solve_long_kernel<2, 1><<<grid, 64, h->smem_bytes, h->stream>>>(make_kcfg(h), io, rg, (long long)B, counter);
-    else if (h->model && h->team_warps == 3)
-        mpc_solve_long_kernel<3, 1><<<grid, 96, h->smem_bytes, h->stream>>>(make_kcfg(h), io, rg, (long long)B, counter);
-    else if (h->model && h->frenet_wpb == 3)
-        mpc_solve_frenet_kernel<3><<<grid, 96, h->smem_bytes, h->stream>>>(make_kcfg(h), io, rg, (long long)B, counter);
-    else if (h->model)
-        mpc_solve_frenet_kernel<4><<<grid, 128, h->smem_bytes, h->stream>>>(make_kcfg(h), io, rg, (long long)B, counter);
-    else if (h->team_warps == 1)
-        mpc_solve_kernel<<<grid, WARPS_PER_BLOCK * 32, h->smem_bytes, h->stream>>>(make_kcfg(h), io, rg, (long long)B, counter);
-    else if (h->team_warps == 2)
-        mpc_solve_long_kernel<2><<<grid, 64, h->smem_bytes, h->stream>>>(make_kcfg(h), io, rg, (long long)B, counter);
-    else
-        mpc_solve_long_kernel<3><<<grid, 96, h->smem_bytes, h->stream>>>(make_kcfg(h), io, rg, (long long)B, counter);
+    int threads = 0;
+    const TeamKernel tk = pw ? team_kernel<1>(h, &threads) : team_kernel<0>(h, &threads);
+    const size_t smem = h->smem_bytes + (pw ? (size_t)tpb * 8 * sizeof(double) : 0);
+    tk<<<grid, threads, smem, h->stream>>>(make_kcfg(h), io, rg, (long long)B, counter);
     CUDA_TRY(h, cudaGetLastError());
     h->stats.kernel_launches += 1;
     return 0;
@@ -801,7 +844,11 @@ struct SolveArgs {
     const double* v_des; const double* u_prev; double* warm;
     double* u0; double* cost; int32_t* status; int32_t* iters; double* traj;
     double* ref_out; int32_t* stop; double* rec;
+    const double* w;   /* [B][8] ([B][7] Frenet) per-problem weights, or NULL: the handle's */
 };
+
+/* doubles per weight row of a handle's model */
+static size_t weight_row(int model) { return model ? 7 : 8; }
 
 /* a contiguous slice [lo, lo + n) of a call's problems */
 static SolveArgs slice_args(const SolveArgs& a, int64_t lo, int N, int model) {
@@ -821,6 +868,7 @@ static SolveArgs slice_args(const SolveArgs& a, int64_t lo, int N, int model) {
     if (a.ref_out) s.ref_out = a.ref_out + 3 * ((size_t)N + 1) * lo;
     if (a.stop) s.stop = a.stop + lo;
     if (a.rec) s.rec = a.rec + 4 * lo;
+    if (a.w) s.w = a.w + weight_row(model) * lo;
     return s;
 }
 
@@ -838,8 +886,9 @@ static const int64_t SMALL_BATCH = 64;
 static int solve_small_host(mpcb200_handle* h, int64_t B, const SolveArgs& a) {
     const int N = h->cfg.N;
     const size_t nt = 6 * (size_t)N + 4, nr = h->model ? 4 : 3 * ((size_t)N + 1);
-    /* layout in doubles: [counter, pad] state ref uprev vdes | warm | u0 cost traj status/iters(int32 pairs) resto rec */
-    const size_t o_state = 2, o_ref = o_state + 4 * B, o_uprev = o_ref + nr * B, o_vdes = o_uprev + 2 * B, o_warm = o_vdes + B;
+    const size_t nw = a.w ? weight_row(h->model) : 0;
+    /* layout in doubles: [counter, pad] state ref uprev vdes w | warm | u0 cost traj status/iters(int32 pairs) resto rec */
+    const size_t o_state = 2, o_ref = o_state + 4 * B, o_uprev = o_ref + nr * B, o_vdes = o_uprev + 2 * B, o_w = o_vdes + B, o_warm = o_w + nw * B;
     const size_t o_u0 = o_warm + nt * B, o_cost = o_u0 + 2 * B, o_traj = o_cost + B, o_stat = o_traj + nt * B, o_iter = o_stat + (B + 1) / 2;
     const size_t o_resto = o_iter + (B + 1) / 2, o_rec = o_resto + (B + 1) / 2;
     const size_t total = o_rec + (a.rec ? 4 * B : 0);
@@ -860,12 +909,13 @@ static int solve_small_host(mpcb200_handle* h, int64_t B, const SolveArgs& a) {
     memcpy(hs + o_ref, a.ref, nr * B * sizeof(double));
     memcpy(hs + o_uprev, a.u_prev, 2 * B * sizeof(double));
     if (a.v_des) memcpy(hs + o_vdes, a.v_des, B * sizeof(double));
+    if (a.w) memcpy(hs + o_w, a.w, nw * B * sizeof(double));
     if (a.warm) memcpy(hs + o_warm, a.warm, nt * B * sizeof(double));
     const size_t in_doubles = a.warm ? o_u0 : o_warm;
     cudaStream_t s = h->stream;
     BatchPtrs io{ds + o_state, ds + o_ref, a.v_des ? ds + o_vdes : nullptr, ds + o_uprev, a.warm ? ds + o_warm : nullptr, ds + o_u0,
                  ds + o_cost, (int*)(ds + o_stat), (int*)(ds + o_iter), a.traj ? ds + o_traj : nullptr,
-                 a.rec ? ds + o_rec : nullptr, (int*)(ds + o_resto)};
+                 a.rec ? ds + o_rec : nullptr, (int*)(ds + o_resto), a.w ? ds + o_w : nullptr};
     RefGen rg;
     memset(&rg, 0, sizeof(rg));
     const size_t out_from = a.warm ? o_warm : o_u0;
@@ -881,7 +931,7 @@ static int solve_small_host(mpcb200_handle* h, int64_t B, const SolveArgs& a) {
     };
     bool launched = false;
     if (h->graphs_ok && s == h->own_stream) {
-        const int flags = (a.v_des ? 1 : 0) | (a.warm ? 2 : 0) | (a.traj ? 4 : 0) | (a.rec ? 8 : 0);
+        const int flags = (a.v_des ? 1 : 0) | (a.warm ? 2 : 0) | (a.traj ? 4 : 0) | (a.rec ? 8 : 0) | (a.w ? 16 : 0);   /* (the rows are data) */
         cudaGraphExec_t exec = nullptr;
         for (int i = 0; i < h->n_graphs; i++) if (h->graphs[i].B == B && h->graphs[i].flags == flags) exec = h->graphs[i].exec;
         if (!exec) {
@@ -948,6 +998,8 @@ static int host_enqueue(mpcb200_handle* h, int64_t B, const SolveArgs& a, const 
     if (a.traj && (rc = ensure(h, h->d_traj, bt))) return rc;
     if (a.rec && (rc = ensure(h, h->d_rec, B * 4 * sizeof(double)))) return rc;
     if ((rc = ensure(h, h->d_resto, B * sizeof(int32_t)))) return rc;
+    const size_t bw = B * weight_row(h->model) * sizeof(double);
+    if (a.w && (rc = ensure(h, h->d_w, bw))) return rc;
     cudaStream_t s = h->stream;
     CUDA_TRY(h, cudaMemcpyAsync(h->d_state.p, a.state, bs, cudaMemcpyHostToDevice, s));
     h->stats.h2d_bytes += bs;
@@ -957,11 +1009,12 @@ static int host_enqueue(mpcb200_handle* h, int64_t B, const SolveArgs& a, const 
     h->stats.h2d_bytes += bu;
     if (a.v_des) { CUDA_TRY(h, cudaMemcpyAsync(h->d_vdes.p, a.v_des, B * sizeof(double), cudaMemcpyHostToDevice, s)); h->stats.h2d_bytes += B * sizeof(double); }
     if (a.warm) { CUDA_TRY(h, cudaMemcpyAsync(h->d_warm.p, a.warm, bt, cudaMemcpyHostToDevice, s)); h->stats.h2d_bytes += bt; }
+    if (a.w) { CUDA_TRY(h, cudaMemcpyAsync(h->d_w.p, a.w, bw, cudaMemcpyHostToDevice, s)); h->stats.h2d_bytes += bw; }
     BatchPtrs io{(const double*)h->d_state.p, on_path ? nullptr : (const double*)h->d_ref.p, a.v_des ? (const double*)h->d_vdes.p : nullptr,
                  (const double*)h->d_uprev.p, a.warm ? (double*)h->d_warm.p : nullptr, (double*)h->d_u0.p,
                  a.cost ? (double*)h->d_cost.p : nullptr, a.status ? (int*)h->d_status.p : nullptr,
                  a.iters ? (int*)h->d_iters.p : nullptr, a.traj ? (double*)h->d_traj.p : nullptr,
-                 a.rec ? (double*)h->d_rec.p : nullptr, (int*)h->d_resto.p};
+                 a.rec ? (double*)h->d_rec.p : nullptr, (int*)h->d_resto.p, a.w ? (const double*)h->d_w.p : nullptr};
     RefGen rg = rg0;
     if (on_path) {
         fill_paths(h, rg.paths);   /* this device's copies of the tables */
@@ -1018,6 +1071,12 @@ static int solve_batch_impl(mpcb200_handle* h, int64_t B, const SolveArgs& a, in
     if (!a.state || (!a.ref && !on_path) || !a.u_prev || (!a.u0 && !a.rec))
         return fail(h, MPCB200_EINVAL, "%s: state, %s, u_prev and %s are required", who, on_path ? "path_of" : "ref", a.rec ? "rec" : "u0");
     if (on_path && h->model) return fail(h, MPCB200_EINVAL, "%s: not available for the Frenet-frame variant", who);
+    if (a.w && mem_space == MPCB200_HOST) {   /* (device rows are checked by the kernel: MPCB200_ERROR for that problem) */
+        const size_t nw = weight_row(h->model);
+        for (int64_t b = 0; b < B; b++)
+            for (size_t i = 0; i < nw; i++)
+                if (!(a.w[b * nw + i] >= 0.0)) return fail(h, MPCB200_EINVAL, "%s: weight %d of problem %lld is negative or NaN", who, (int)i, (long long)b);
+    }
     CUDA_TRY(h, cudaSetDevice(h->device));
     RefGen rg;
     memset(&rg, 0, sizeof(rg));
@@ -1034,7 +1093,7 @@ static int solve_batch_impl(mpcb200_handle* h, int64_t B, const SolveArgs& a, in
     if (mem_space == MPCB200_DEVICE) {
         int rc;
         if ((rc = ensure(h, h->d_resto, B * sizeof(int32_t)))) return rc;
-        BatchPtrs io{a.state, a.ref, a.v_des, a.u_prev, a.warm, a.u0, a.cost, a.status, a.iters, a.traj, a.rec, (int*)h->d_resto.p};
+        BatchPtrs io{a.state, a.ref, a.v_des, a.u_prev, a.warm, a.u0, a.cost, a.status, a.iters, a.traj, a.rec, (int*)h->d_resto.p, a.w};
         rg.path_of = a.path_of; rg.ref_out = a.ref_out; rg.stop = a.stop;
         return launch_solve(h, B, io, rg);
     }
@@ -1086,13 +1145,26 @@ int mpcb200_get_restorations(mpcb200_handle* h, int64_t B, int32_t* out) {
     return MPCB200_OK;
 }
 
+/* mpcb200_solve_batch_frenet and mpcb200_solve_batch_frenet_w (w == NULL: the handle's weights) */
+static int solve_frenet(const char* who, mpcb200_handle* h, int64_t B, const double* state, const double* k_coeffs, const double* v_des,
+                        const double* u_prev, double* warm, const double* w, double* u0, double* cost, int32_t* status, int32_t* iters,
+                        double* traj, int32_t mem_space) {
+    if (h && !h->model) return fail(h, MPCB200_EINVAL, "%s: the handle was not created with mpcb200_create_frenet", who);
+    const SolveArgs a{who, state, k_coeffs, nullptr, 1, 0.0, v_des, u_prev, warm, u0, cost, status, iters, traj, nullptr, nullptr, nullptr, w};
+    return solve_batch_impl(h, B, a, mem_space);
+}
+
 int mpcb200_solve_batch_frenet(mpcb200_handle* h, int64_t B, const double* state, const double* k_coeffs, const double* v_des,
                                const double* u_prev, double* warm, double* u0, double* cost, int32_t* status, int32_t* iters,
                                double* traj, int32_t mem_space) {
-    if (h && !h->model) return fail(h, MPCB200_EINVAL, "mpcb200_solve_batch_frenet: the handle was not created with mpcb200_create_frenet");
-    const SolveArgs a{"mpcb200_solve_batch_frenet", state, k_coeffs, nullptr, 1, 0.0, v_des, u_prev, warm, u0, cost, status, iters, traj,
-                      nullptr, nullptr, nullptr};
-    return solve_batch_impl(h, B, a, mem_space);
+    return solve_frenet("mpcb200_solve_batch_frenet", h, B, state, k_coeffs, v_des, u_prev, warm, nullptr, u0, cost, status, iters, traj, mem_space);
+}
+
+int mpcb200_solve_batch_frenet_w(mpcb200_handle* h, int64_t B, const double* state, const double* k_coeffs, const double* v_des,
+                                 const double* u_prev, double* warm, const double* w, double* u0, double* cost, int32_t* status,
+                                 int32_t* iters, double* traj, int32_t mem_space) {
+    if (h && !w) return fail(h, MPCB200_EINVAL, "mpcb200_solve_batch_frenet_w: w is required");
+    return solve_frenet("mpcb200_solve_batch_frenet_w", h, B, state, k_coeffs, v_des, u_prev, warm, w, u0, cost, status, iters, traj, mem_space);
 }
 
 int mpcb200_set_cost_frenet(mpcb200_handle* h, const double w[7]) {
@@ -1106,13 +1178,26 @@ int mpcb200_set_cost_frenet(mpcb200_handle* h, const double w[7]) {
     return MPCB200_OK;
 }
 
+/* mpcb200_solve_batch and mpcb200_solve_batch_w (w == NULL: the handle's weights) */
+static int solve_xy(const char* who, mpcb200_handle* h, int64_t B, const double* state, const double* ref, const double* v_des,
+                    const double* u_prev, double* warm, const double* w, double* u0, double* cost, int32_t* status, int32_t* iters,
+                    double* traj, int32_t mem_space) {
+    if (h && h->model) return fail(h, MPCB200_EINVAL, "%s: Frenet handle; use mpcb200_solve_batch_frenet", who);
+    const SolveArgs a{who, state, ref, nullptr, 1, 0.0, v_des, u_prev, warm, u0, cost, status, iters, traj, nullptr, nullptr, nullptr, w};
+    return solve_batch_impl(h, B, a, mem_space);
+}
+
 int mpcb200_solve_batch(mpcb200_handle* h, int64_t B, const double* state, const double* ref, const double* v_des,
                         const double* u_prev, double* warm, double* u0, double* cost, int32_t* status, int32_t* iters,
                         double* traj, int32_t mem_space) {
-    if (h && h->model) return fail(h, MPCB200_EINVAL, "mpcb200_solve_batch: Frenet handle; use mpcb200_solve_batch_frenet");
-    const SolveArgs a{"mpcb200_solve_batch", state, ref, nullptr, 1, 0.0, v_des, u_prev, warm, u0, cost, status, iters, traj,
-                      nullptr, nullptr, nullptr};
-    return solve_batch_impl(h, B, a, mem_space);
+    return solve_xy("mpcb200_solve_batch", h, B, state, ref, v_des, u_prev, warm, nullptr, u0, cost, status, iters, traj, mem_space);
+}
+
+int mpcb200_solve_batch_w(mpcb200_handle* h, int64_t B, const double* state, const double* ref, const double* v_des,
+                          const double* u_prev, double* warm, const double* w, double* u0, double* cost, int32_t* status,
+                          int32_t* iters, double* traj, int32_t mem_space) {
+    if (h && !w) return fail(h, MPCB200_EINVAL, "mpcb200_solve_batch_w: w is required");
+    return solve_xy("mpcb200_solve_batch_w", h, B, state, ref, v_des, u_prev, warm, w, u0, cost, status, iters, traj, mem_space);
 }
 
 int mpcb200_solve_batch_records(mpcb200_handle* h, int64_t B, const double* state, const double* ref, const double* v_des,
@@ -1201,7 +1286,7 @@ static int ensure_seed(mpcb200_handle* h) {
 
 /* one device's share of a rollout: vehicles [lo, lo + n) of B; enqueue ... */
 static int rollout_enqueue(mpcb200_handle* h, int64_t n, int32_t T, const double* pose0, const int32_t* path_of, int32_t track_using_time,
-                           double target_vel, bool want_log, bool want_final) {
+                           double target_vel, const double* w, bool want_log, bool want_final) {
     CUDA_TRY(h, cudaSetDevice(h->device));
     int rc;
     if ((rc = ensure_seed(h))) return rc;
@@ -1214,6 +1299,11 @@ static int rollout_enqueue(mpcb200_handle* h, int64_t n, int32_t T, const double
     CUDA_TRY(h, cudaMemcpyAsync(h->d_pose.p, pose0, (size_t)n * 3 * sizeof(double), cudaMemcpyHostToDevice, s));
     CUDA_TRY(h, cudaMemcpyAsync(h->d_pathof.p, path_of, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     h->stats.h2d_bytes += (size_t)n * (3 * sizeof(double) + sizeof(int32_t));
+    if (w) {
+        if ((rc = ensure(h, h->d_w, (size_t)n * 8 * sizeof(double)))) return rc;
+        CUDA_TRY(h, cudaMemcpyAsync(h->d_w.p, w, (size_t)n * 8 * sizeof(double), cudaMemcpyHostToDevice, s));
+        h->stats.h2d_bytes += (size_t)n * 8 * sizeof(double);
+    }
     RolloutArgs a;
     memset(&a, 0, sizeof(a));
     a.pose0 = (const double*)h->d_pose.p; a.path_of = (const int*)h->d_pathof.p;
@@ -1221,6 +1311,7 @@ static int rollout_enqueue(mpcb200_handle* h, int64_t n, int32_t T, const double
     a.T = T; a.track_using_time = track_using_time; a.target_vel = target_vel;
     a.log = want_log ? (double*)h->d_log.p : nullptr; a.final_state = want_final ? (double*)h->d_final.p : nullptr; a.B = (long)n;
     a.warm0 = (const double*)h->d_seed.p;
+    a.w = w ? (const double*)h->d_w.p : nullptr;
     /* large fleets at short horizons: one control period = plant / waypoints / thread-per-problem solve over the whole fleet.
      * Measured at N = 8, 200 periods (profiles/r02_logs/r02_rollout_thresholds.log): a period of the pipeline takes ~0.9 ms up to
      * 8,192 vehicles (the slowest vehicle's dozen solver trips) and grows slowly after that, the fused kernel takes 0.5 / 0.8 /
@@ -1241,7 +1332,8 @@ static int rollout_enqueue(mpcb200_handle* h, int64_t n, int32_t T, const double
         if ((rc = ensure(h, h->d_iters, (size_t)n * sizeof(int32_t)))) return rc;
         BatchPtrs out;
         memset(&out, 0, sizeof(out));
-        out.u0 = (double*)h->d_u0.p; out.status = (int*)h->d_status.p; out.iters = (int*)h->d_iters.p;
+        out.u0 = (double*)h->d_u0.p; out.status = (int*)h->d_status.p; out.iters = (int*)h->d_iters.p; out.w = a.w;
+        auto sk = a.w ? rollout_solve_tpp_kernel<0, 1> : rollout_solve_tpp_kernel<0, 0>;
         RefGen rg;
         memset(&rg, 0, sizeof(rg));
         fill_paths(h, rg.paths);
@@ -1258,9 +1350,8 @@ static int rollout_enqueue(mpcb200_handle* h, int64_t n, int32_t T, const double
             rollout_plant_kernel<<<pgrid, 128, 0, s>>>((long long)n, Bp, veh, a.pose0, t == 0);
             rollout_waypoints_kernel<<<wgrid, 128, 0, s>>>(kc, (long long)n, Bp, veh, a.path_of, rg, (double*)h->d_tpp_state.p, (double*)h->d_tpp_filt.p,
                                                           (int*)h->d_vstop.p, t == 0);
-            rollout_solve_tpp_kernel<0><<<(int)sblocks, tb, 0, s>>>(kc, (long long)n, Bp, veh, (const int*)h->d_vstop.p, (double*)h->d_tpp_state.p,
-                                                                   (double*)h->d_tpp_filt.p, t == 0 ? a.warm0 : nullptr, des_speed, out,
-                                                                   a.log ? a.log + (size_t)t * n * 8 : nullptr, nullptr, t == 0);
+            sk<<<(int)sblocks, tb, 0, s>>>(kc, (long long)n, Bp, veh, (const int*)h->d_vstop.p, (double*)h->d_tpp_state.p, (double*)h->d_tpp_filt.p,
+                                           t == 0 ? a.warm0 : nullptr, des_speed, out, a.log ? a.log + (size_t)t * n * 8 : nullptr, nullptr, t == 0);
             CUDA_TRY(h, cudaGetLastError());
         }
         if (a.final_state) rollout_final_kernel<<<pgrid, 128, 0, s>>>((long long)n, Bp, veh, a.final_state);
@@ -1272,15 +1363,11 @@ static int rollout_enqueue(mpcb200_handle* h, int64_t n, int32_t T, const double
     CUDA_TRY(h, cudaMemsetAsync(h->d_counter, 0, sizeof(unsigned long long), s));
     const int per_block = (h->team_warps == 1) ? WARPS_PER_BLOCK : 1;
     long long blocks_needed = (n + per_block - 1) / per_block;
-    long long max_blocks = (long long)h->num_sms * h->rollout_blocks_per_sm;
+    long long max_blocks = (long long)h->num_sms * (w ? h->rollout_blocks_per_sm_w : h->rollout_blocks_per_sm);
     int grid = (int)(blocks_needed < max_blocks ? blocks_needed : max_blocks);
+    const RolloutKernel rk = w ? rollout_kernel<1>(h) : rollout_kernel<0>(h);
     CUDA_TRY(h, cudaEventRecord(h->ev0, s));
-    if (h->team_warps == 1)
-        mpc_rollout_kernel<<<grid, WARPS_PER_BLOCK * 32, h->smem_bytes, s>>>(make_kcfg(h), a, h->d_counter);
-    else if (h->team_warps == 2)
-        mpc_rollout_long_kernel<2><<<grid, 64, h->smem_bytes + ROLLOUT_PX * sizeof(double), s>>>(make_kcfg(h), a, h->d_counter);
-    else
-        mpc_rollout_long_kernel<3><<<grid, 96, h->smem_bytes + ROLLOUT_PX * sizeof(double), s>>>(make_kcfg(h), a, h->d_counter);
+    rk<<<grid, 32 * (h->team_warps == 1 ? WARPS_PER_BLOCK : h->team_warps), rollout_smem_bytes(h, w != nullptr), s>>>(make_kcfg(h), a, h->d_counter);
     CUDA_TRY(h, cudaGetLastError());
     CUDA_TRY(h, cudaEventRecord(h->ev1, s));
     h->stats.kernel_launches += 1;
@@ -1304,17 +1391,22 @@ static int rollout_collect(mpcb200_handle* h, int64_t lo, int64_t n, int64_t B, 
     return MPCB200_OK;
 }
 
-int mpcb200_rollout(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, int32_t track_using_time,
-                    double target_vel, double* log, double* final_state) {
+/* mpcb200_rollout and mpcb200_rollout_w (w == NULL: the handle's weights) */
+static int rollout_impl(const char* who, mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of,
+                        int32_t track_using_time, double target_vel, const double* w, double* log, double* final_state) {
     if (!h) return MPCB200_EINVAL;
-    if (B < 0 || T < 0) return fail(h, MPCB200_EINVAL, "mpcb200_rollout: B=%lld T=%d", (long long)B, T);
-    if (h->model) return fail(h, MPCB200_EINVAL, "mpcb200_rollout: not available for the Frenet-frame variant");
+    if (B < 0 || T < 0) return fail(h, MPCB200_EINVAL, "%s: B=%lld T=%d", who, (long long)B, T);
+    if (h->model) return fail(h, MPCB200_EINVAL, "%s: not available for the Frenet-frame variant", who);
     memset(&h->stats, 0, sizeof(h->stats));
     if (B == 0 || T == 0) return MPCB200_OK;
-    if (!pose0 || !path_of) return fail(h, MPCB200_EINVAL, "mpcb200_rollout: pose0 and path_of are required");
+    if (!pose0 || !path_of) return fail(h, MPCB200_EINVAL, "%s: pose0 and path_of are required", who);
     for (int64_t b = 0; b < B; b++)
         if (path_of[b] < 0 || path_of[b] > 2 || h->path_n[path_of[b]] == 0)
-            return fail(h, MPCB200_EINVAL, "mpcb200_rollout: vehicle %lld uses path %d, which was not set with mpcb200_set_path", (long long)b, path_of[b]);
+            return fail(h, MPCB200_EINVAL, "%s: vehicle %lld uses path %d, which was not set with mpcb200_set_path", who, (long long)b, path_of[b]);
+    if (w)
+        for (int64_t b = 0; b < B; b++)
+            for (int i = 0; i < 8; i++)
+                if (!(w[8 * b + i] >= 0.0)) return fail(h, MPCB200_EINVAL, "%s: weight %d of vehicle %lld is negative or NaN", who, i, (long long)b);
     /* a vehicle stays on one GPU for all T steps: contiguous slices of the fleet, every device at once */
     const int parts = (B >= 2 * (int64_t)(h->n_sub + 1)) ? h->n_sub + 1 : 1;
     mpcb200_handle* dev[8];
@@ -1325,8 +1417,8 @@ int mpcb200_rollout(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0
     for (int i = 0; i < parts; i++) {
         shard_range(B, parts, i, &lo[i], &hi[i]);
         if (i) memset(&dev[i]->stats, 0, sizeof(mpcb200_stats));
-        if ((rc = rollout_enqueue(dev[i], hi[i] - lo[i], T, pose0 + 3 * lo[i], path_of + lo[i], track_using_time, target_vel, log != nullptr,
-                                  final_state != nullptr)))
+        if ((rc = rollout_enqueue(dev[i], hi[i] - lo[i], T, pose0 + 3 * lo[i], path_of + lo[i], track_using_time, target_vel,
+                                  w ? w + 8 * lo[i] : nullptr, log != nullptr, final_state != nullptr)))
             return sub_fail(h, dev[i], rc);
     }
     for (int i = 0; i < parts; i++)
@@ -1338,6 +1430,17 @@ int mpcb200_rollout(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0
     }
     CUDA_TRY(h, cudaSetDevice(h->device));
     return MPCB200_OK;
+}
+
+int mpcb200_rollout(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, int32_t track_using_time,
+                    double target_vel, double* log, double* final_state) {
+    return rollout_impl("mpcb200_rollout", h, B, T, pose0, path_of, track_using_time, target_vel, nullptr, log, final_state);
+}
+
+int mpcb200_rollout_w(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, int32_t track_using_time,
+                      double target_vel, const double* w, double* log, double* final_state) {
+    if (h && !w && B > 0 && T > 0) return fail(h, MPCB200_EINVAL, "mpcb200_rollout_w: w is required");
+    return rollout_impl("mpcb200_rollout_w", h, B, T, pose0, path_of, track_using_time, target_vel, w, log, final_state);
 }
 
 int mpcb200_rollout_frenet(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, double window,

@@ -197,7 +197,18 @@ MPC_HD constexpr int sds_of(int model) { return model ? SDS_F : SDS; }
 MPC_HD int team_warps(int N) { return (N + 1 + 31) / 32; }   // warps that share one problem
 MPC_HD constexpr int w_sd_of(int W, int model) { return model ? 160 + (W > 1 ? XCH_SIZE : 0) : W_SD_OF(W); }   // MODEL 1: exchange area at 160
 MPC_HD int lf_offset(int N, int model = 0) { return w_sd_of(team_warps(N), model) + (N + 1) * sds_of(model) + N * KST_STRIDE; }
-MPC_HD int smem_doubles_per_team(int N, int model = 0) { return lf_offset(N, model) + LF_DOUBLES * (N + 2); }   // even: 16-byte alignment of the next team
+MPC_HD int smem_doubles_per_team(int N, int model = 0, int pw = 0) { return lf_offset(N, model) + LF_DOUBLES * (N + 2) + (pw ? 8 : 0); }   // even: 16-byte alignment of the next team
+// PW (per-problem weights) teams keep their problem's eight weights in update_cost order behind the rest of the team's area
+MPC_HD int wt_offset(int N, int model) { return smem_doubles_per_team(N, model); }
+// weight i (update_cost order of the XY model) of problem b in a caller's weight array: [B][8], or [B][7] for the Frenet-frame
+// variant (cey, cep, cev, cda, cdd, ca, cd: the XY slots 1..7; nothing on s)
+MPC_HD double row_weight(const double* w, long b, int i, int model) { return model ? (i ? w[7 * b + i - 1] : 0.0) : w[8 * b + i]; }
+// the rule of mpcb200_set_cost: not negative and not NaN
+MPC_HD bool row_weights_ok(const double* w, long b, int model) {
+    bool ok = true;
+    for (int i = 0; i < 8; i++) ok = ok && row_weight(w, b, i, model) >= 0.0;
+    return ok;
+}
 
 MPC_DEV double dmax_(double a, double b) { return a > b ? a : b; }
 MPC_DEV double dmin_(double a, double b) { return a < b ? a : b; }
@@ -556,7 +567,9 @@ MPC_HD void riccati_roles_shfl(int l, int N, int W_SD, int* out) {
 
 // W = warps per team (1: a warp per problem; 2, 3: a block per problem)
 // MODEL 0: XY kinematic bicycle (MKZMPCPathFollower.jl); MODEL 1: Frenet-frame variant (MKZMPCPathFollowerFrenet.jl)
-template <int W, int MODEL = 0>
+// PW: the cost weights are this problem's (wt_offset in the team's shared memory, staged by solve_problem / rollout_group) instead
+// of the kernel parameter KCfg::w.  PW = 0 reads the kernel parameter, as the unweighted entry points always have.
+template <int W, int MODEL = 0, int PW = 0>
 struct TeamSolver {
     static constexpr int W_XCHG = MODEL ? 160 : W_XCH;   // exchange area of multi-warp teams
     static constexpr int W_SD = w_sd_of(W, MODEL);   // first stage record
@@ -764,10 +777,11 @@ struct TeamSolver {
     }
 
     // cheap per-use reconstruction of lane constants (keeps them out of the register file)
-    MPC_DEV double wx() const { return (k >= 1 && k <= N) ? c.w[0] : 0.0; }
-    MPC_DEV double wy() const { return (k >= 1 && k <= N) ? c.w[1] : 0.0; }
-    MPC_DEV double wp() const { return (k >= 1 && k <= N) ? c.w[2] : 0.0; }
-    MPC_DEV double wv() const { return (k >= 1 && k <= N - 1) ? c.w[3] : 0.0; }
+    MPC_DEV double wt(int i) const { return PW ? lds(sm, SO(wt_offset(N, MODEL) + i)) : c.w[i]; }   // cost weight i (update_cost order)
+    MPC_DEV double wx() const { return (k >= 1 && k <= N) ? wt(0) : 0.0; }
+    MPC_DEV double wy() const { return (k >= 1 && k <= N) ? wt(1) : 0.0; }
+    MPC_DEV double wp() const { return (k >= 1 && k <= N) ? wt(2) : 0.0; }
+    MPC_DEV double wv() const { return (k >= 1 && k <= N - 1) ? wt(3) : 0.0; }
     MPC_DEV double rHi(int i) const { return (k == 0) ? c.rHiFirst[i] : c.rHiLater[i]; }
     MPC_DEV double cst(int i) const { return lds(sm, SO(W_CONST + i)); }  // state[0..3], u_prev[0..1], v_des
     MPC_DEV int rec() const { return SO(W_SD + (isS ? k : 0) * SDSZ); }    // this lane's own stage record
@@ -866,8 +880,8 @@ struct TeamSolver {
             const double ex = sx - ref_x(), ey = sy - ref_y(), ep = sp - ref_p(), evv = sv - cst(6);
             f = wx() * ex * ex + wy() * ey * ey + wp() * ep * ep + wv() * evv * evv;
             if (isU) {
-                f += c.w[6] * ua * ua + c.w[7] * ud * ud;
-                if (k >= 1) { const double da = ua - pa, dd = ud - pd; f += c.w[4] * da * da + c.w[5] * dd * dd; }
+                f += wt(6) * ua * ua + wt(7) * ud * ud;
+                if (k >= 1) { const double da = ua - pa, dd = ud - pd; f += wt(4) * da * da + wt(5) * dd * dd; }
             }
         }
         double p = 1.0;
@@ -899,10 +913,10 @@ struct TeamSolver {
         g.v = s2 * wv() * (L.sv - cst(6));
         g.a = 0.0; g.d = 0.0;
         if (isU) {
-            g.a = s2 * c.w[6] * L.ua;
-            g.d = s2 * c.w[7] * L.ud;
-            if (k >= 1) { g.a += s2 * c.w[4] * (L.ua - pa); g.d += s2 * c.w[5] * (L.ud - pd); }
-            if (k + 1 < N) { g.a -= s2 * c.w[4] * (na - L.ua); g.d -= s2 * c.w[5] * (nd - L.ud); }
+            g.a = s2 * wt(6) * L.ua;
+            g.d = s2 * wt(7) * L.ud;
+            if (k >= 1) { g.a += s2 * wt(4) * (L.ua - pa); g.d += s2 * wt(5) * (L.ud - pd); }
+            if (k + 1 < N) { g.a -= s2 * wt(4) * (na - L.ua); g.d -= s2 * wt(5) * (nd - L.ud); }
         }
         return g;
     }
@@ -1008,11 +1022,11 @@ struct TeamSolver {
             Hxx = s2 * wx() + dw; Hyy = s2 * wy() + dw; Hpp = s2 * wp() + hpp + dw; Hvv = s2 * wv() + Sv + dw;
             if (MODEL) { Hxx += hss; Hyy += hee; }
             if (isU) {
-                if (k >= 1) { Ca = s2 * c.w[4]; Cd = s2 * c.w[5]; }
+                if (k >= 1) { Ca = s2 * wt(4); Cd = s2 * wt(5); }
                 if (isR) { Ca += SrW[1]; Cd += SrW[0]; }
             }
-            Haa = isU ? s2 * c.w[6] + Sa + dw + Ca : 1.0;
-            Hdd = isU ? s2 * c.w[7] + Sd + dw + Cd + hdd : 1.0;
+            Haa = isU ? s2 * wt(6) + Sa + dw + Ca : 1.0;
+            Hdd = isU ? s2 * wt(7) + Sd + dw + Cd + hdd : 1.0;
             gsv = gv + bv;
             if (isU) { gua = ga + ba; gud = gd + bd; }
         }
@@ -1960,8 +1974,8 @@ struct TeamSolver {
             const double ex = L.sx - ref_x(), ey = L.sy - ref_y(), ep = L.sp - ref_p(), evv = L.sv - cst(6);
             double f = wx() * ex * ex + wy() * ey * ey + wp() * ep * ep + wv() * evv * evv;
             if (isU) {
-                f += c.w[6] * L.ua * L.ua + c.w[7] * L.ud * L.ud;
-                if (k >= 1) { const double da = L.ua - pa, dd = L.ud - pd; f += c.w[4] * da * da + c.w[5] * dd * dd; }
+                f += wt(6) * L.ua * L.ua + wt(7) * L.ud * L.ud;
+                if (k >= 1) { const double da = L.ua - pa, dd = L.ud - pd; f += wt(4) * da * da + wt(5) * dd * dd; }
             }
             res.cost = tsum(f);
         }
@@ -1984,7 +1998,19 @@ struct BatchPtrs {
     double* rec;           // [B][4] or null: the packed 32-byte result record {acc, df, cost: f64; status, iters: i32} that the
                            //   multi-GPU all-gather moves (SURVEY 8e); its status word carries the restoration count in bits 8..15
     int* resto;            // [B] or null: restorations by rollout this solve went through (0 for almost every problem)
+    const double* w;       // [B][8] ([B][7] Frenet) or null: the problem's own cost weights (row_weight); null = KCfg::w
 };
+
+// The answer to a problem that cannot be solved as given (a path id never set, a weight row that is negative or NaN -- device
+// pointers cannot be checked on the host): MPCB200_ERROR, zero commands, cost 0, no iterations, no restorations
+MPC_DEV void write_error_answer(const BatchPtrs& io, long b) {
+    if (io.u0) { io.u0[2 * b] = 0.0; io.u0[2 * b + 1] = 0.0; }
+    if (io.cost) io.cost[b] = 0.0;
+    if (io.status) io.status[b] = 4;
+    if (io.iters) io.iters[b] = 0;
+    if (io.rec) { st_global_v2(io.rec + 4 * b, 0.0, 0.0); st_global_v2(io.rec + 4 * b + 2, 0.0, int2_as_double(4, 0)); }
+    if (io.resto) io.resto[b] = 0;
+}
 
 // Optional on-device reference generation for a batch (path_of != null): the waypoints come from the
 // replicated path tables instead of io.ref.
@@ -1999,9 +2025,11 @@ struct RefGen {
 
 // MODEL 1 (Frenet-frame variant): io.state = (s, e_y, e_psi, v), io.ref = [B][4] curvature polynomial (highest degree
 // first), traj / warm = s, e_y, v, e_psi, d_f, acc (get_solver_results of MKZMPCPathFollowerFrenet.jl:188-206)
-template <int W, int MODEL = 0>
+// PW: the problem's weights come from io.w (KCfg::w when it is null); a row that breaks mpcb200_set_cost's rule gets
+// write_error_answer
+template <int W, int MODEL = 0, int PW = 0>
 MPC_DEV void solve_problem(const KCfg& cfg, const BatchPtrs& io, const RefGen& rg, long b, smem_t smem) {
-    TeamSolver<W, MODEL> S(cfg, smem);
+    TeamSolver<W, MODEL, PW> S(cfg, smem);
     const int k = S.k, N = cfg.N;
     const long nr = 3L * (N + 1), nt = 6L * N + 4;
     if (MODEL) {
@@ -2014,12 +2042,7 @@ MPC_DEV void solve_problem(const KCfg& cfg, const BatchPtrs& io, const RefGen& r
             // a path id that was never given to mpcb200_set_path (device pointers cannot be checked on the host):
             // the problem is answered with MPCB200_ERROR and zero commands instead of indexing outside the tables
             if (k == 0) {
-                if (io.u0) { io.u0[2 * b] = 0.0; io.u0[2 * b + 1] = 0.0; }
-                if (io.cost) io.cost[b] = 0.0;
-                if (io.status) io.status[b] = 4;
-                if (io.iters) io.iters[b] = 0;
-                if (io.rec) { st_global_v2(io.rec + 4 * b, 0.0, 0.0); st_global_v2(io.rec + 4 * b + 2, 0.0, int2_as_double(4, 0)); }
-                if (io.resto) io.resto[b] = 0;
+                write_error_answer(io, b);
                 if (rg.stop) rg.stop[b] = 0;
             }
             return;
@@ -2041,6 +2064,15 @@ MPC_DEV void solve_problem(const KCfg& cfg, const BatchPtrs& io, const RefGen& r
         else if (k < 6) cv = io.u_prev[2 * b + (k - 4)];
         else if (k == 6) cv = io.v_des ? io.v_des[b] : (rg.path_of ? rg.target_vel : 0.0);   // des_speed (clamped on the host), mpc_cmd_pub.jl:58-62,116
         if (k < 8) sts(smem, SO(W_CONST + k), cv);
+        if (PW) {
+            const double wk = (k < 8) ? (io.w ? row_weight(io.w, b, k, MODEL) : cfg.w[k]) : 0.0;
+            if (k < 8) sts(smem, SO(wt_offset(N, MODEL) + k), wk);
+            if (!S.tall(wk >= 0.0)) {
+                if (k == 0) write_error_answer(io, b);
+                S.tsync();
+                return;
+            }
+        }
         S.tsync();
     }
     // ---- start point
@@ -2093,6 +2125,7 @@ struct RolloutArgs {
     double* final_state;    // [B][8] or null
     long B;
     const double* warm0;    // [6N+4] or null: start point of every vehicle's FIRST solve (the module-load solution)
+    const double* w;        // [B][8] or null: each vehicle's cost weights for all its control periods (checked by the host); null = KCfg::w
 };
 
 // atan2(y, x) for x > 0 and sincos for small arguments: the plant's slip angles and steering angle are
@@ -2162,9 +2195,9 @@ MPC_DEV double sel8(const double* v, int i) {   // register-friendly v[i] for a 
 // rollout's instructions); states and commands cross through `px` ([vehicle][10] doubles) around two
 // block barriers per control period.  Warps whose vehicle index is past the fleet only keep the barriers.
 #define ROLLOUT_PX 10   // X, Y, psi, vx, vy, wz, acc, df, acc_des, df_des
-template <int W>
+template <int W, int PW = 0>
 MPC_DEV void rollout_group(const KCfg& cfg, const RolloutArgs& a, long b0, smem_t smem, smem_t px, int nwarps) {
-    TeamSolver<W> S(cfg, smem);
+    TeamSolver<W, 0, PW> S(cfg, smem);
     const int k = S.k, N = cfg.N;
     const int w = (W == 1) ? (thread_in_block() >> 5) : 0;   // vehicle of this thread within the block
     const int nveh = (W == 1) ? nwarps : 1;
@@ -2173,6 +2206,7 @@ MPC_DEV void rollout_group(const KCfg& cfg, const RolloutArgs& a, long b0, smem_
     const int pxw = SO(w * ROLLOUT_PX);
     const PathTable& path = a.paths[valid ? a.path_of[b] : 0];
     if (k < 8) sts(px, pxw + SO(k), (valid && k < 3) ? a.pose0[3 * b + k] : 0.0);
+    if (PW && k < 8) sts(smem, SO(wt_offset(N, 0) + k), (valid && a.w) ? a.w[8 * b + k] : cfg.w[k]);   // the vehicle keeps its row
     double st[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     double acc_des = 0.0, df_des = 0.0, up_d = 0.0, up_a = 0.0;   // commands, d_f_current, acc_current
     const double des_speed = a.target_vel > 0.0 ? a.target_vel : 0.0;

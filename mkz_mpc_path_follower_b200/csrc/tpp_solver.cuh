@@ -107,12 +107,15 @@ struct FalseT { static constexpr bool value = false; };
 MPC_DEV double nanmax(double v, double t) { return (t > v || t != t) ? t : v; }   // NaN wins, like warp_max
 MPC_DEV constexpr int sidx(int i, int j) { return (i <= j) ? (i * 6 - i * (i - 1) / 2 + (j - i)) : (j * 6 - j * (j - 1) / 2 + (i - j)); }
 
-template <int MODEL = 0>
+// PW: the cost weights are the problem's own row `wr` (BatchPtrs::w; KCfg::w when it is null), read from global memory where they are
+// used (64 bytes per problem against the ~43 KB of slot state a trip streams); PW = 0 reads the kernel parameter KCfg::w
+template <int MODEL = 0, int PW = 0>
 struct TppSolverT {
     static constexpr int TEVN = tev_n(MODEL), TF_FH = tf_fh(MODEL);
     const KCfg& c;
     const TppMemT<MODEL> m;
     const int N;
+    const double* wr;   // PW: this problem's weight row (row_weight layout of its model) or null
     double cst[7];   // state[4], u_prev (df, acc), v_des
     double kp[4];    // MODEL 1: the problem's curvature polynomial K(s), highest degree first
     // ---- interior-point driver state (TeamSolver::solve's locals)
@@ -125,14 +128,15 @@ struct TppSolverT {
     enum { PH_INIT = 0, PH_EVAL0, PH_LS, PH_BEGIN, PH_PD, PH_RESOLVE, PH_TRIAL, PH_SOC, PH_RESTO };
     enum { RUNNING = -100 };
 
-    MPC_DEV TppSolverT(const KCfg& cfg, const TppMemT<MODEL>& mem) : c(cfg), m(mem), N(cfg.N) {}
+    MPC_DEV TppSolverT(const KCfg& cfg, const TppMemT<MODEL>& mem) : c(cfg), m(mem), N(cfg.N), wr(nullptr) {}
 
     MPC_DEV bool isU(int k) const { return k < N; }
     MPC_DEV bool isR(int k) const { return (k == 0 || k >= 2) && k < N; }
-    MPC_DEV double wx(int k) const { return (k >= 1) ? c.w[0] : 0.0; }
-    MPC_DEV double wy(int k) const { return (k >= 1) ? c.w[1] : 0.0; }
-    MPC_DEV double wp(int k) const { return (k >= 1) ? c.w[2] : 0.0; }
-    MPC_DEV double wv(int k) const { return (k >= 1 && k <= N - 1) ? c.w[3] : 0.0; }
+    MPC_DEV double wt(int i) const { return (PW && wr) ? row_weight(wr, 0, i, MODEL) : c.w[i]; }   // cost weight i (update_cost order)
+    MPC_DEV double wx(int k) const { return (k >= 1) ? wt(0) : 0.0; }
+    MPC_DEV double wy(int k) const { return (k >= 1) ? wt(1) : 0.0; }
+    MPC_DEV double wp(int k) const { return (k >= 1) ? wt(2) : 0.0; }
+    MPC_DEV double wv(int k) const { return (k >= 1 && k <= N - 1) ? wt(3) : 0.0; }
     MPC_DEV double rHi(int k, int i) const { return (k == 0) ? c.rHiFirst[i] : c.rHiLater[i]; }
     MPC_DEV int evb(int which) const { return TF_EV + TEVN * which; }
     // reference sample of stage k; MODEL 1: the cost is on e_y, e_psi themselves (reference 0): nothing to read
@@ -190,6 +194,7 @@ struct TppSolverT {
     // ------------------------------------------------------------------
     MPC_DEV void begin(const BatchPtrs& io, long b, double v_des0 = 0.0) {
         const long nr = 3L * (N + 1), nt = 6L * N + 4;
+        if (PW) wr = io.w ? io.w + (MODEL ? 7 : 8) * b : nullptr;
         for (int i = 0; i < 4; i++) cst[i] = io.state[4 * b + i];
         cst[4] = io.u_prev[2 * b]; cst[5] = io.u_prev[2 * b + 1];
         cst[6] = io.v_des ? io.v_des[b] : v_des0;
@@ -212,7 +217,7 @@ struct TppSolverT {
 
     // A problem whose reference samples are already in the slot (written by the waypoint kernel of a closed-loop step) and
     // whose start point is either `warm0` ([6N+4], the layout of BatchPtrs::warm) or whatever the slot holds -- the
-    // previous solution of the same vehicle: the control loop's warm start without moving a byte.
+    // previous solution of the same vehicle: the control loop's warm start without moving a byte.  (PW: the caller sets wr.)
     MPC_DEV void begin_in_place(const double c7[7], const double* warm0) {
         for (int i = 0; i < 7; i++) cst[i] = c7[i];
         if (warm0) {
@@ -280,10 +285,10 @@ struct TppSolverT {
         g.v = s2 * wv(k) * (sv - cst[6]);
         g.a = 0.0; g.d = 0.0;
         if (u) {
-            g.a = s2 * c.w[6] * ua;
-            g.d = s2 * c.w[7] * ud;
-            if (k >= 1) { g.a += s2 * c.w[4] * (ua - pa); g.d += s2 * c.w[5] * (ud - pd); }
-            if (k + 1 < N) { g.a -= s2 * c.w[4] * (na - ua); g.d -= s2 * c.w[5] * (nd - ud); }
+            g.a = s2 * wt(6) * ua;
+            g.d = s2 * wt(7) * ud;
+            if (k >= 1) { g.a += s2 * wt(4) * (ua - pa); g.d += s2 * wt(5) * (ud - pd); }
+            if (k + 1 < N) { g.a -= s2 * wt(4) * (na - ua); g.d -= s2 * wt(5) * (nd - ud); }
         }
         return g;
     }
@@ -386,8 +391,8 @@ struct TppSolverT {
                 const double ex = sx - xr, ey = sy - yr, ep = sp - pr, evv = sv - cst[6];
                 double fk = wx(k) * ex * ex + wy(k) * ey * ey + wp(k) * ep * ep + wv(k) * evv * evv;
                 if (u) {
-                    fk += c.w[6] * ua * ua + c.w[7] * ud * ud;
-                    if (k >= 1) { const double da = ua - pa, dd = ud - pd; fk += c.w[4] * da * da + c.w[5] * dd * dd; }
+                    fk += wt(6) * ua * ua + wt(7) * ud * ud;
+                    if (k >= 1) { const double da = ua - pa, dd = ud - pd; fk += wt(4) * da * da + wt(5) * dd * dd; }
                 }
                 f += fk;
             }
@@ -468,10 +473,10 @@ struct TppSolverT {
                 g.x = s2 * wx(k) * (sx - xr); g.y = s2 * wy(k) * (sy - yr); g.p = s2 * wp(k) * (sp - pr); g.v = s2 * wv(k) * (sv - cst[6]);
                 g.a = 0.0; g.d = 0.0;
                 if (u) {
-                    g.a = s2 * c.w[6] * ua;
-                    g.d = s2 * c.w[7] * ud;
-                    if (k >= 1) { g.a += s2 * c.w[4] * (ua - pa); g.d += s2 * c.w[5] * (ud - pd); }
-                    if (k + 1 < N) { g.a -= s2 * c.w[4] * (na - ua); g.d -= s2 * c.w[5] * (nd - ud); }
+                    g.a = s2 * wt(6) * ua;
+                    g.d = s2 * wt(7) * ud;
+                    if (k >= 1) { g.a += s2 * wt(4) * (ua - pa); g.d += s2 * wt(5) * (ud - pd); }
+                    if (k + 1 < N) { g.a -= s2 * wt(4) * (na - ua); g.d -= s2 * wt(5) * (nd - ud); }
                 }
             }
             double Hxx, Hyy, Hpp, Hpv = 0.0, Hvv, Hpd = 0.0, Hvd = 0.0, Haa, Hdd, Ca = 0.0, Cd = 0.0;
@@ -532,11 +537,11 @@ struct TppSolverT {
                 Hxx = s2 * wx(k) + dw; Hyy = s2 * wy(k) + dw; Hpp = s2 * wp(k) + hpp + dw; Hvv = s2 * wv(k) + Sv + dw;
                 if (MODEL) { Hxx += hss; Hyy += hee; }
                 if (u) {
-                    if (k >= 1) { Ca = s2 * c.w[4]; Cd = s2 * c.w[5]; }
+                    if (k >= 1) { Ca = s2 * wt(4); Cd = s2 * wt(5); }
                     if (r) { Ca += SrW1; Cd += SrW0; }
                 }
-                Haa = u ? s2 * c.w[6] + Sa + dw + Ca : 1.0;
-                Hdd = u ? s2 * c.w[7] + Sd + dw + Cd + hdd : 1.0;
+                Haa = u ? s2 * wt(6) + Sa + dw + Ca : 1.0;
+                Hdd = u ? s2 * wt(7) + Sd + dw + Cd + hdd : 1.0;
                 gsv = g.v + bv;
                 if (u) { gua = g.a + ba; gud = g.d + bd; }
             }
@@ -916,10 +921,10 @@ struct TppSolverT {
                 g.x = s2 * wx(k) * (sx - xr); g.y = s2 * wy(k) * (sy - yr); g.p = s2 * wp(k) * (sp - pr); g.v = s2 * wv(k) * (sv - cst[6]);
                 g.a = 0.0; g.d = 0.0;
                 if (u) {
-                    g.a = s2 * c.w[6] * ua;
-                    g.d = s2 * c.w[7] * ud;
-                    if (k >= 1) { g.a += s2 * c.w[4] * (ua - pa); g.d += s2 * c.w[5] * (ud - pd); }
-                    if (k + 1 < N) { g.a -= s2 * c.w[4] * (na - ua); g.d -= s2 * c.w[5] * (nd - ud); }
+                    g.a = s2 * wt(6) * ua;
+                    g.d = s2 * wt(7) * ud;
+                    if (k >= 1) { g.a += s2 * wt(4) * (ua - pa); g.d += s2 * wt(5) * (ud - pd); }
+                    if (k + 1 < N) { g.a -= s2 * wt(4) * (na - ua); g.d -= s2 * wt(5) * (nd - ud); }
                 }
             }
             const double hn = u ? 1.0 : 0.0;
@@ -1320,8 +1325,8 @@ struct TppSolverT {
             const double ex = sx - ref(TF_XR, k), ey = sy - ref(TF_YR, k), ep = sp - ref(TF_PR, k), evv = sv - cst[6];
             double fk = wx(k) * ex * ex + wy(k) * ey * ey + wp(k) * ep * ep + wv(k) * evv * evv;
             if (isU(k)) {
-                fk += c.w[6] * ua * ua + c.w[7] * ud * ud;
-                if (k >= 1) { const double da = ua - pa, dd = ud - pd; fk += c.w[4] * da * da + c.w[5] * dd * dd; }
+                fk += wt(6) * ua * ua + wt(7) * ud * ud;
+                if (k >= 1) { const double da = ua - pa, dd = ud - pd; fk += wt(4) * da * da + wt(5) * dd * dd; }
             }
             f += fk;
             if (k == 0) { a0 = ua; d0 = ud; }
