@@ -495,8 +495,10 @@ static RolloutKernel rollout_kernel(const mpcb200_handle* h) {
     return (h->team_warps == 2) ? mpc_rollout_long_kernel<2, PW> : mpc_rollout_long_kernel<3, PW>;
 }
 
-/* dynamic shared memory of the fused rollout kernel: the teams and the plant exchange area */
+/* dynamic shared memory of the fused rollout kernel: the teams and the plant exchange area (the XY handle's smem_bytes already
+ * holds it at N <= 31; the Frenet kernel always runs WARPS_PER_BLOCK vehicles per block, whatever frenet_wpb is) */
 static size_t rollout_smem_bytes(const mpcb200_handle* h, bool pw) {
+    if (h->model) return WARPS_PER_BLOCK * ((size_t)smem_doubles_per_team(h->cfg.N, 1) + ROLLOUT_PX) * sizeof(double);
     return h->smem_bytes + (h->team_warps == 1 ? 0 : ROLLOUT_PX * sizeof(double)) + (pw ? (size_t)teams_per_block(h) * 8 * sizeof(double) : 0);
 }
 
@@ -544,6 +546,10 @@ static int64_t tpp_default_min_batch(int model, int N) {
     if (model) return (N <= 10) ? 16384 : 32768;
     return (N <= 10) ? 32768 : 0;
 }
+
+/* the module-default weights of MKZMPCPathFollower.jl:51-59 in update_cost order: an XY handle's weights until mpcb200_set_cost,
+ * and those of the module-load solve that seeds every rollout */
+static const double W_XY_DEFAULT[8] = {9.0, 9.0, 10.0, 0.0, 100.0, 1000.0, 0.0, 0.0};
 
 static int create_impl(mpcb200_handle** out, const mpcb200_config* cfg, int model);
 static int create_multi(mpcb200_handle** out, const mpcb200_config* cfg, int model);
@@ -597,11 +603,9 @@ static int create_impl(mpcb200_handle** out, const mpcb200_config* cfg, int mode
     h->device = cfg->device;
     h->err[0] = 0;
     memset(&h->stats, 0, sizeof(h->stats));
-    /* defaults of MKZMPCPathFollower.jl:51-59 in update_cost order */
-    const double w0[8] = {9.0, 9.0, 10.0, 0.0, 100.0, 1000.0, 0.0, 0.0};
     /* MKZMPCPathFollowerFrenet.jl:51-58 in the XY slots: nothing on s, C_ey, C_epsi, C_ev, C_dacc, C_ddf, C_acc, C_df */
     const double w1[8] = {0.0, 9.0, 10.0, 0.5, 100.0, 1000.0, 0.0, 0.0};
-    memcpy(h->w, model ? w1 : w0, sizeof(w0));
+    memcpy(h->w, model ? w1 : W_XY_DEFAULT, sizeof(w1));
     h->model = model;
 #define TRY_OR_FREE(expr)                                                                 \
     do {                                                                                  \
@@ -630,53 +634,27 @@ static int create_impl(mpcb200_handle** out, const mpcb200_config* cfg, int mode
         TRY_OR_FREE(cudaMalloc((void**)&h->d_roles, sizeof(roles)));
         TRY_OR_FREE(cudaMemcpy(h->d_roles, roles, sizeof(int) * (32 * rs + 32 * RS_STRIDE), cudaMemcpyHostToDevice));
     }
-    if (model && h->team_warps > 1) {
-        h->smem_bytes = (size_t)smem_doubles_per_team(cfg->N, 1) * sizeof(double);
-        const void* fn = (h->team_warps == 2) ? (const void*)mpc_solve_long_kernel<2, 1> : (const void*)mpc_solve_long_kernel<3, 1>;
-        TRY_OR_FREE(raise_dyn_smem((const void*)fn, h->device, (size_t)(h->smem_bytes)));
-        TRY_OR_FREE(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        TRY_OR_FREE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->blocks_per_sm, fn, h->team_warps * 32, h->smem_bytes));
-    } else if (model) {
-        const size_t team = (size_t)smem_doubles_per_team(cfg->N, 1) * sizeof(double);
+    const size_t team = (size_t)smem_doubles_per_team(cfg->N, model) * sizeof(double);
+    if (model && h->team_warps == 1) {
         int b4 = 0, b3 = 0;
-        TRY_OR_FREE(raise_dyn_smem((const void*)mpc_solve_frenet_kernel<4>, h->device, (size_t)(4 * team)));
-        TRY_OR_FREE(cudaFuncSetAttribute(mpc_solve_frenet_kernel<4>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        TRY_OR_FREE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b4, mpc_solve_frenet_kernel<4>, 4 * 32, 4 * team));
-        TRY_OR_FREE(raise_dyn_smem((const void*)mpc_solve_frenet_kernel<3>, h->device, (size_t)(3 * team)));
-        TRY_OR_FREE(cudaFuncSetAttribute(mpc_solve_frenet_kernel<3>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        TRY_OR_FREE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b3, mpc_solve_frenet_kernel<3>, 3 * 32, 3 * team));
+        TRY_OR_FREE(prepare_kernel((const void*)mpc_solve_frenet_kernel<4>, h->device, 4 * 32, 4 * team, &b4));
+        TRY_OR_FREE(prepare_kernel((const void*)mpc_solve_frenet_kernel<3>, h->device, 3 * 32, 3 * team, &b3));
         /* measured (tools/frenet_bench.py): N = 8: 12 warps at 168 registers 6.06 M solves/s vs 8 warps at 255 registers 5.80 M;
          * N = 20: 9 warps 2.88 M vs 8 warps 3.23 M -- the spill code of the 168-register build pays only for >= 1.4x the warps */
         h->frenet_wpb = (10 * 3 * b3 >= 14 * 4 * b4) ? 3 : 4;
         if (const char* e = getenv("MPCB200_FRENET_WPB")) { int v = atoi(e); if (v == 3 || v == 4) h->frenet_wpb = v; }  /* tuning aid */
         h->blocks_per_sm = (h->frenet_wpb == 3) ? b3 : b4;
         h->smem_bytes = h->frenet_wpb * team;
-        const size_t rb = WARPS_PER_BLOCK * team + WARPS_PER_BLOCK * ROLLOUT_PX * sizeof(double);
-        TRY_OR_FREE(raise_dyn_smem((const void*)mpc_rollout_frenet_kernel, h->device, (size_t)(rb)));
-        TRY_OR_FREE(cudaFuncSetAttribute(mpc_rollout_frenet_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        TRY_OR_FREE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->frenet_rollout_blocks_per_sm, mpc_rollout_frenet_kernel, WARPS_PER_BLOCK * 32, rb));
-        if (h->frenet_rollout_blocks_per_sm < 1) h->frenet_rollout_blocks_per_sm = 1;
-    } else if (h->team_warps == 1) {
-        h->smem_bytes = ((size_t)WARPS_PER_BLOCK * smem_doubles_per_team(cfg->N) + WARPS_PER_BLOCK * ROLLOUT_PX) * sizeof(double);
-        TRY_OR_FREE(raise_dyn_smem((const void*)mpc_solve_kernel<0>, h->device, (size_t)(h->smem_bytes)));
-        TRY_OR_FREE(cudaFuncSetAttribute(mpc_solve_kernel<0>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        TRY_OR_FREE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->blocks_per_sm, mpc_solve_kernel<0>, WARPS_PER_BLOCK * 32, h->smem_bytes));
-        TRY_OR_FREE(raise_dyn_smem((const void*)mpc_rollout_kernel<0>, h->device, (size_t)(h->smem_bytes)));
-        TRY_OR_FREE(cudaFuncSetAttribute(mpc_rollout_kernel<0>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        TRY_OR_FREE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->rollout_blocks_per_sm, mpc_rollout_kernel<0>, WARPS_PER_BLOCK * 32, h->smem_bytes));
-        if (h->rollout_blocks_per_sm < 1) h->rollout_blocks_per_sm = 1;
+        TRY_OR_FREE(prepare_kernel((const void*)mpc_rollout_frenet_kernel, h->device, WARPS_PER_BLOCK * 32, rollout_smem_bytes(h, false),
+                                   &h->frenet_rollout_blocks_per_sm));
     } else {
-        h->smem_bytes = (size_t)smem_doubles_per_team(cfg->N) * sizeof(double);
-        const void* fn = (h->team_warps == 2) ? (const void*)mpc_solve_long_kernel<2> : (const void*)mpc_solve_long_kernel<3>;
-        TRY_OR_FREE(raise_dyn_smem((const void*)fn, h->device, (size_t)(h->smem_bytes)));
-        TRY_OR_FREE(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        TRY_OR_FREE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->blocks_per_sm, fn, h->team_warps * 32, h->smem_bytes));
-        const void* fr = (h->team_warps == 2) ? (const void*)mpc_rollout_long_kernel<2> : (const void*)mpc_rollout_long_kernel<3>;
-        const size_t rb = h->smem_bytes + ROLLOUT_PX * sizeof(double);
-        TRY_OR_FREE(raise_dyn_smem((const void*)fr, h->device, (size_t)(rb)));
-        TRY_OR_FREE(cudaFuncSetAttribute(fr, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        TRY_OR_FREE(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&h->rollout_blocks_per_sm, fr, h->team_warps * 32, rb));
-        if (h->rollout_blocks_per_sm < 1) h->rollout_blocks_per_sm = 1;
+        /* one-warp XY teams: four per block, with the plant exchange area of the fused rollout kernel */
+        h->smem_bytes = (model || h->team_warps > 1) ? team : WARPS_PER_BLOCK * (team + ROLLOUT_PX * sizeof(double));
+        int threads = 0;
+        const void* fn = (const void*)team_kernel<0>(h, &threads);
+        TRY_OR_FREE(prepare_kernel(fn, h->device, threads, h->smem_bytes, &h->blocks_per_sm));
+        if (!model)
+            TRY_OR_FREE(prepare_kernel((const void*)rollout_kernel<0>(h), h->device, threads, rollout_smem_bytes(h, false), &h->rollout_blocks_per_sm));
     }
     {
         /* thread-per-problem path for large batches (any horizon): needs B >> resident lanes to keep them busy */
@@ -850,26 +828,57 @@ struct SolveArgs {
 /* doubles per weight row of a handle's model */
 static size_t weight_row(int model) { return model ? 7 : 8; }
 
-/* a contiguous slice [lo, lo + n) of a call's problems */
-static SolveArgs slice_args(const SolveArgs& a, int64_t lo, int N, int model) {
-    const size_t nt = 6 * (size_t)N + 4, nr = model ? 4 : 3 * ((size_t)N + 1);
-    SolveArgs s = a;
-    s.state = a.state + 4 * lo;
-    if (a.ref) s.ref = a.ref + nr * lo;
-    if (a.path_of) s.path_of = a.path_of + lo;
-    if (a.v_des) s.v_des = a.v_des + lo;
-    s.u_prev = a.u_prev + 2 * lo;
-    if (a.warm) s.warm = a.warm + nt * lo;
-    if (a.u0) s.u0 = a.u0 + 2 * lo;
-    if (a.cost) s.cost = a.cost + lo;
-    if (a.status) s.status = a.status + lo;
-    if (a.iters) s.iters = a.iters + lo;
-    if (a.traj) s.traj = a.traj + nt * lo;
-    if (a.ref_out) s.ref_out = a.ref_out + 3 * ((size_t)N + 1) * lo;
-    if (a.stop) s.stop = a.stop + lo;
-    if (a.rec) s.rec = a.rec + 4 * lo;
-    if (a.w) s.w = a.w + weight_row(model) * lo;
-    return s;
+/* The per-problem arrays of a solve call, one table entry each.  The order is that of the packed small-batch layout
+ * (solve_small_host): inputs, then warm (in and out), then outputs. */
+enum ArrayId { A_STATE, A_REF, A_PATH_OF, A_U_PREV, A_V_DES, A_W, A_WARM, A_U0, A_COST, A_TRAJ, A_STATUS, A_ITERS, A_REC, A_REF_OUT, A_STOP,
+               A_COUNT };
+enum { DIR_IN = 1, DIR_OUT = 2, DIR_INOUT = 3 };
+/* an array's slot in the packed small-batch layout: there when the caller gives the array (PACK_GIVEN); always there and
+ * copied, the kernel getting it only when given (PACK_SLOT); always there and always written by the kernel (PACK_ALWAYS), so
+ * that one captured graph serves callers who ask for the output and callers who do not */
+enum { PACK_GIVEN, PACK_SLOT, PACK_ALWAYS };
+struct CallArray {
+    char* host;     /* the caller's pointer, at the first problem of the slice (a device pointer for MPCB200_DEVICE); null: not given */
+    size_t row;     /* bytes per problem */
+    int dir;        /* DIR_* */
+    int pack;       /* PACK_* */
+    DevBuf* dev;    /* the handle's staging buffer for host pointers */
+};
+
+/* the table of a call's arrays from problem `lo` on, staged in handle h's buffers (d_ref also stages ref_out: on-path calls
+ * have no ref) */
+static void call_arrays(mpcb200_handle* h, const SolveArgs& a, int64_t lo, CallArray t[A_COUNT]) {
+    const size_t d = sizeof(double), i4 = sizeof(int32_t);
+    const size_t nt = (6 * (size_t)h->cfg.N + 4) * d, nr = 3 * ((size_t)h->cfg.N + 1) * d;
+    const CallArray all[A_COUNT] = {
+        {(char*)a.state, 4 * d, DIR_IN, PACK_GIVEN, &h->d_state},
+        {(char*)a.ref, h->model ? 4 * d : nr, DIR_IN, PACK_GIVEN, &h->d_ref},
+        {(char*)a.path_of, i4, DIR_IN, PACK_GIVEN, &h->d_pathof},
+        {(char*)a.u_prev, 2 * d, DIR_IN, PACK_GIVEN, &h->d_uprev},
+        {(char*)a.v_des, d, DIR_IN, PACK_SLOT, &h->d_vdes},
+        {(char*)a.w, weight_row(h->model) * d, DIR_IN, PACK_GIVEN, &h->d_w},
+        {(char*)a.warm, nt, DIR_INOUT, PACK_GIVEN, &h->d_warm},
+        {(char*)a.u0, 2 * d, DIR_OUT, PACK_ALWAYS, &h->d_u0},
+        {(char*)a.cost, d, DIR_OUT, PACK_ALWAYS, &h->d_cost},
+        {(char*)a.traj, nt, DIR_OUT, PACK_SLOT, &h->d_traj},
+        {(char*)a.status, i4, DIR_OUT, PACK_ALWAYS, &h->d_status},
+        {(char*)a.iters, i4, DIR_OUT, PACK_ALWAYS, &h->d_iters},
+        {(char*)a.rec, 4 * d, DIR_OUT, PACK_GIVEN, &h->d_rec},
+        {(char*)a.ref_out, nr, DIR_OUT, PACK_GIVEN, &h->d_ref},
+        {(char*)a.stop, i4, DIR_OUT, PACK_GIVEN, &h->d_stop},
+    };
+    for (int i = 0; i < A_COUNT; i++) {
+        t[i] = all[i];
+        if (t[i].host) t[i].host += t[i].row * lo;
+    }
+}
+
+/* the kernel arguments from one pointer per table entry (null: not in the call) */
+static BatchPtrs batch_ptrs(void* const p[A_COUNT], int* resto, RefGen& rg) {
+    rg.path_of = (const int*)p[A_PATH_OF]; rg.ref_out = (double*)p[A_REF_OUT]; rg.stop = (int*)p[A_STOP];
+    return BatchPtrs{(const double*)p[A_STATE], (const double*)p[A_REF], (const double*)p[A_V_DES], (const double*)p[A_U_PREV],
+                     (double*)p[A_WARM], (double*)p[A_U0], (double*)p[A_COST], (int*)p[A_STATUS], (int*)p[A_ITERS], (double*)p[A_TRAJ],
+                     (double*)p[A_REC], resto, (const double*)p[A_W]};
 }
 
 /* contiguous slice of `total` owned by part `i` of `parts`; sizes differ by at most one (same rule as sharding.shard_range) */
@@ -879,20 +888,64 @@ static void shard_range(int64_t total, int parts, int i, int64_t* lo, int64_t* h
     *hi = *lo + base + (i < rem ? 1 : 0);
 }
 
+/* Host pointers on a multi-GPU handle: one contiguous slice [lo[i], hi[i]) of the B problems per device dev[i] of the first
+ * n_dev, all working at once (one slice when there are fewer than two problems per device).  Clears the stats of the sub-handles
+ * that get a slice; returns the number of slices. */
+static int slice_call(mpcb200_handle* h, int64_t B, int n_dev, mpcb200_handle* dev[8], int64_t lo[8], int64_t hi[8]) {
+    const int parts = (B >= 2 * (int64_t)n_dev) ? n_dev : 1;
+    dev[0] = h;
+    for (int i = 0; i < h->n_sub; i++) dev[i + 1] = h->sub[i];
+    for (int i = 0; i < parts; i++) {
+        shard_range(B, parts, i, &lo[i], &hi[i]);
+        if (i) memset(&dev[i]->stats, 0, sizeof(mpcb200_stats));
+    }
+    return parts;
+}
+
+/* the sub-handles' counters into the handle the caller holds */
+static void merge_stats(mpcb200_handle* h, mpcb200_handle* const dev[8], int parts) {
+    for (int i = 1; i < parts; i++) {
+        h->stats.kernel_launches += dev[i]->stats.kernel_launches;
+        h->stats.h2d_bytes += dev[i]->stats.h2d_bytes; h->stats.d2h_bytes += dev[i]->stats.d2h_bytes;
+        if (dev[i]->stats.kernel_ms > h->stats.kernel_ms) h->stats.kernel_ms = dev[i]->stats.kernel_ms;   /* the devices run concurrently */
+    }
+}
+
+/* host path ids: each one set with mpcb200_set_path (`what`: "problem" or "vehicle") */
+static int check_path_ids(mpcb200_handle* h, const char* who, const char* what, int64_t B, const int32_t* path_of) {
+    for (int64_t b = 0; b < B; b++)
+        if (path_of[b] < 0 || path_of[b] > 2 || h->path_n[path_of[b]] == 0)
+            return fail(h, MPCB200_EINVAL, "%s: %s %lld uses path %d, which was not set with mpcb200_set_path", who, what, (long long)b, path_of[b]);
+    return MPCB200_OK;
+}
+
+/* host weight rows of nw doubles: mpcb200_set_cost's rule (device rows are checked by the kernel: MPCB200_ERROR for that problem) */
+static int check_weight_rows(mpcb200_handle* h, const char* who, const char* what, int64_t B, const double* w, size_t nw) {
+    for (int64_t b = 0; b < B; b++)
+        for (size_t i = 0; i < nw; i++)
+            if (!(w[b * nw + i] >= 0.0)) return fail(h, MPCB200_EINVAL, "%s: weight %d of %s %lld is negative or NaN", who, (int)i, what, (long long)b);
+    return MPCB200_OK;
+}
+
 /* Host pointers, small batch (the control loop's batch of one): latency is the driver calls, not the bytes.  All
  * inputs are packed into one pinned buffer (with the zeroed problem counter in front) and go over in ONE copy, all
  * outputs come back in ONE copy: 7 driver calls instead of ~16. */
 static const int64_t SMALL_BATCH = 64;
 static int solve_small_host(mpcb200_handle* h, int64_t B, const SolveArgs& a) {
-    const int N = h->cfg.N;
-    const size_t nt = 6 * (size_t)N + 4, nr = h->model ? 4 : 3 * ((size_t)N + 1);
-    const size_t nw = a.w ? weight_row(h->model) : 0;
-    /* layout in doubles: [counter, pad] state ref uprev vdes w | warm | u0 cost traj status/iters(int32 pairs) resto rec */
-    const size_t o_state = 2, o_ref = o_state + 4 * B, o_uprev = o_ref + nr * B, o_vdes = o_uprev + 2 * B, o_w = o_vdes + B, o_warm = o_w + nw * B;
-    const size_t o_u0 = o_warm + nt * B, o_cost = o_u0 + 2 * B, o_traj = o_cost + B, o_stat = o_traj + nt * B, o_iter = o_stat + (B + 1) / 2;
-    const size_t o_resto = o_iter + (B + 1) / 2, o_rec = o_resto + (B + 1) / 2;
-    const size_t total = o_rec + (a.rec ? 4 * B : 0);
-    const size_t bytes = total * sizeof(double);
+    CallArray t[A_COUNT];
+    call_arrays(h, a, 0, t);
+    /* layout in doubles: [counter, pad] inputs | warm | outputs, each slot a whole number of doubles, the restoration counts
+     * just before rec.  in_end: the end of what is copied in, out_from: the start of what is copied out (the warm slot is in both) */
+    size_t off[A_COUNT], o = 2, in_end = 2, out_from = 0, o_resto = 0;
+    for (int i = 0; i < A_COUNT; i++) {
+        if (i == A_REC) { o_resto = o; o += (B + 1) / 2; }
+        off[i] = o;
+        if (!t[i].host && t[i].pack == PACK_GIVEN) continue;
+        if ((t[i].dir & DIR_OUT) && !out_from) out_from = o;
+        o += (t[i].row * B + sizeof(double) - 1) / sizeof(double);
+        if (t[i].dir & DIR_IN) in_end = o;
+    }
+    const size_t total = o, bytes = total * sizeof(double);
     int rc;
     if (bytes > h->d_stage.cap || bytes > h->h_stage_cap) drop_graphs(h);   /* the graphs hold the old addresses */
     if ((rc = ensure(h, h->d_stage, bytes))) return rc;
@@ -905,23 +958,20 @@ static int solve_small_host(mpcb200_handle* h, int64_t B, const SolveArgs& a) {
     double* hs = (double*)h->h_stage;
     double* ds = (double*)h->d_stage.p;
     hs[0] = 0.0; hs[1] = 0.0;   /* the problem counter (all-zero bits) */
-    memcpy(hs + o_state, a.state, 4 * B * sizeof(double));
-    memcpy(hs + o_ref, a.ref, nr * B * sizeof(double));
-    memcpy(hs + o_uprev, a.u_prev, 2 * B * sizeof(double));
-    if (a.v_des) memcpy(hs + o_vdes, a.v_des, B * sizeof(double));
-    if (a.w) memcpy(hs + o_w, a.w, nw * B * sizeof(double));
-    if (a.warm) memcpy(hs + o_warm, a.warm, nt * B * sizeof(double));
-    const size_t in_doubles = a.warm ? o_u0 : o_warm;
+    void* p[A_COUNT];
+    int flags = 0;   /* the graph's shape: which arrays the kernel gets (the rows of w are data) */
+    for (int i = 0; i < A_COUNT; i++) {
+        if (t[i].host && (t[i].dir & DIR_IN)) memcpy(hs + off[i], t[i].host, t[i].row * B);
+        p[i] = (t[i].host || t[i].pack == PACK_ALWAYS) ? ds + off[i] : nullptr;
+        if (t[i].host && t[i].pack != PACK_ALWAYS) flags |= 1 << i;
+    }
     cudaStream_t s = h->stream;
-    BatchPtrs io{ds + o_state, ds + o_ref, a.v_des ? ds + o_vdes : nullptr, ds + o_uprev, a.warm ? ds + o_warm : nullptr, ds + o_u0,
-                 ds + o_cost, (int*)(ds + o_stat), (int*)(ds + o_iter), a.traj ? ds + o_traj : nullptr,
-                 a.rec ? ds + o_rec : nullptr, (int*)(ds + o_resto), a.w ? ds + o_w : nullptr};
     RefGen rg;
     memset(&rg, 0, sizeof(rg));
-    const size_t out_from = a.warm ? o_warm : o_u0;
+    const BatchPtrs io = batch_ptrs(p, (int*)(ds + o_resto), rg);
     /* the sequence copy in -> kernel -> copy out; `ext`: events recorded from inside a graph need the external flag to be timed */
     auto enqueue = [&](bool ext) -> int {
-        CUDA_TRY(h, cudaMemcpyAsync(ds, hs, in_doubles * sizeof(double), cudaMemcpyHostToDevice, s));
+        CUDA_TRY(h, cudaMemcpyAsync(ds, hs, in_end * sizeof(double), cudaMemcpyHostToDevice, s));
         CUDA_TRY(h, cudaEventRecordWithFlags(h->ev0, s, ext ? cudaEventRecordExternal : cudaEventRecordDefault));
         int r = launch_solve(h, B, io, rg, (unsigned long long*)ds);
         if (r) return r;
@@ -931,7 +981,6 @@ static int solve_small_host(mpcb200_handle* h, int64_t B, const SolveArgs& a) {
     };
     bool launched = false;
     if (h->graphs_ok && s == h->own_stream) {
-        const int flags = (a.v_des ? 1 : 0) | (a.warm ? 2 : 0) | (a.traj ? 4 : 0) | (a.rec ? 8 : 0) | (a.w ? 16 : 0);   /* (the rows are data) */
         cudaGraphExec_t exec = nullptr;
         for (int i = 0; i < h->n_graphs; i++) if (h->graphs[i].B == B && h->graphs[i].flags == flags) exec = h->graphs[i].exec;
         if (!exec) {
@@ -958,16 +1007,11 @@ static int solve_small_host(mpcb200_handle* h, int64_t B, const SolveArgs& a) {
         }
     }
     if (!launched && (rc = enqueue(false))) return rc;
-    h->stats.h2d_bytes += in_doubles * sizeof(double);
+    h->stats.h2d_bytes += in_end * sizeof(double);
     h->stats.d2h_bytes += (total - out_from) * sizeof(double);
     CUDA_TRY(h, cudaStreamSynchronize(s));
-    if (a.u0) memcpy(a.u0, hs + o_u0, 2 * B * sizeof(double));
-    if (a.cost) memcpy(a.cost, hs + o_cost, B * sizeof(double));
-    if (a.status) memcpy(a.status, hs + o_stat, B * sizeof(int32_t));
-    if (a.iters) memcpy(a.iters, hs + o_iter, B * sizeof(int32_t));
-    if (a.traj) memcpy(a.traj, hs + o_traj, nt * B * sizeof(double));
-    if (a.warm) memcpy(a.warm, hs + o_warm, nt * B * sizeof(double));
-    if (a.rec) memcpy(a.rec, hs + o_rec, 4 * B * sizeof(double));
+    for (int i = 0; i < A_COUNT; i++)
+        if (t[i].host && (t[i].dir & DIR_OUT)) memcpy(t[i].host, hs + off[i], t[i].row * B);
     memcpy(h->small_resto, hs + o_resto, B * sizeof(int32_t));   /* where mpcb200_get_restorations looks after a small batch */
     h->resto_on_host = true;
     float ms = 0.f;
@@ -977,51 +1021,25 @@ static int solve_small_host(mpcb200_handle* h, int64_t B, const SolveArgs& a) {
 }
 
 /* HOST pointers, one device: stage the slice through the handle's device buffers and launch (asynchronous) ... */
-static int host_enqueue(mpcb200_handle* h, int64_t B, const SolveArgs& a, const RefGen& rg0) {
+static int host_enqueue(mpcb200_handle* h, int64_t B, const SolveArgs& a, int64_t lo, const RefGen& rg0) {
     CUDA_TRY(h, cudaSetDevice(h->device));
-    const bool on_path = (a.path_of != nullptr);
-    const int N = h->cfg.N;
-    const size_t nt = 6 * (size_t)N + 4, nr = h->model ? 4 : 3 * ((size_t)N + 1);
-    const size_t bs = B * 4 * sizeof(double), br = B * nr * sizeof(double), bu = B * 2 * sizeof(double), bt = B * nt * sizeof(double);
+    CallArray t[A_COUNT];
+    call_arrays(h, a, lo, t);
     int rc;
-    if ((rc = ensure(h, h->d_state, bs))) return rc;
-    if ((!on_path || a.ref_out) && (rc = ensure(h, h->d_ref, br))) return rc;
-    if (on_path && (rc = ensure(h, h->d_pathof, B * sizeof(int32_t)))) return rc;
-    if (on_path && a.stop && (rc = ensure(h, h->d_stop, B * sizeof(int32_t)))) return rc;
-    if ((rc = ensure(h, h->d_uprev, bu))) return rc;
-    if ((rc = ensure(h, h->d_u0, bu))) return rc;
-    if (a.v_des && (rc = ensure(h, h->d_vdes, B * sizeof(double)))) return rc;
-    if (a.warm && (rc = ensure(h, h->d_warm, bt))) return rc;
-    if (a.cost && (rc = ensure(h, h->d_cost, B * sizeof(double)))) return rc;
-    if (a.status && (rc = ensure(h, h->d_status, B * sizeof(int32_t)))) return rc;
-    if (a.iters && (rc = ensure(h, h->d_iters, B * sizeof(int32_t)))) return rc;
-    if (a.traj && (rc = ensure(h, h->d_traj, bt))) return rc;
-    if (a.rec && (rc = ensure(h, h->d_rec, B * 4 * sizeof(double)))) return rc;
+    for (int i = 0; i < A_COUNT; i++)
+        if (t[i].host && (rc = ensure(h, *t[i].dev, t[i].row * B))) return rc;
     if ((rc = ensure(h, h->d_resto, B * sizeof(int32_t)))) return rc;
-    const size_t bw = B * weight_row(h->model) * sizeof(double);
-    if (a.w && (rc = ensure(h, h->d_w, bw))) return rc;
     cudaStream_t s = h->stream;
-    CUDA_TRY(h, cudaMemcpyAsync(h->d_state.p, a.state, bs, cudaMemcpyHostToDevice, s));
-    h->stats.h2d_bytes += bs;
-    if (on_path) { CUDA_TRY(h, cudaMemcpyAsync(h->d_pathof.p, a.path_of, B * sizeof(int32_t), cudaMemcpyHostToDevice, s)); h->stats.h2d_bytes += B * sizeof(int32_t); }
-    else { CUDA_TRY(h, cudaMemcpyAsync(h->d_ref.p, a.ref, br, cudaMemcpyHostToDevice, s)); h->stats.h2d_bytes += br; }
-    CUDA_TRY(h, cudaMemcpyAsync(h->d_uprev.p, a.u_prev, bu, cudaMemcpyHostToDevice, s));
-    h->stats.h2d_bytes += bu;
-    if (a.v_des) { CUDA_TRY(h, cudaMemcpyAsync(h->d_vdes.p, a.v_des, B * sizeof(double), cudaMemcpyHostToDevice, s)); h->stats.h2d_bytes += B * sizeof(double); }
-    if (a.warm) { CUDA_TRY(h, cudaMemcpyAsync(h->d_warm.p, a.warm, bt, cudaMemcpyHostToDevice, s)); h->stats.h2d_bytes += bt; }
-    if (a.w) { CUDA_TRY(h, cudaMemcpyAsync(h->d_w.p, a.w, bw, cudaMemcpyHostToDevice, s)); h->stats.h2d_bytes += bw; }
-    BatchPtrs io{(const double*)h->d_state.p, on_path ? nullptr : (const double*)h->d_ref.p, a.v_des ? (const double*)h->d_vdes.p : nullptr,
-                 (const double*)h->d_uprev.p, a.warm ? (double*)h->d_warm.p : nullptr, (double*)h->d_u0.p,
-                 a.cost ? (double*)h->d_cost.p : nullptr, a.status ? (int*)h->d_status.p : nullptr,
-                 a.iters ? (int*)h->d_iters.p : nullptr, a.traj ? (double*)h->d_traj.p : nullptr,
-                 a.rec ? (double*)h->d_rec.p : nullptr, (int*)h->d_resto.p, a.w ? (const double*)h->d_w.p : nullptr};
-    RefGen rg = rg0;
-    if (on_path) {
-        fill_paths(h, rg.paths);   /* this device's copies of the tables */
-        rg.path_of = (const int*)h->d_pathof.p;
-        rg.ref_out = a.ref_out ? (double*)h->d_ref.p : nullptr;
-        rg.stop = a.stop ? (int*)h->d_stop.p : nullptr;
+    void* p[A_COUNT];
+    for (int i = 0; i < A_COUNT; i++) {
+        p[i] = t[i].host ? t[i].dev->p : nullptr;
+        if (!t[i].host || !(t[i].dir & DIR_IN)) continue;
+        CUDA_TRY(h, cudaMemcpyAsync(p[i], t[i].host, t[i].row * B, cudaMemcpyHostToDevice, s));
+        h->stats.h2d_bytes += t[i].row * B;
     }
+    RefGen rg = rg0;
+    if (a.path_of) fill_paths(h, rg.paths);   /* this device's copies of the tables */
+    const BatchPtrs io = batch_ptrs(p, (int*)h->d_resto.p, rg);
     CUDA_TRY(h, cudaEventRecord(h->ev0, s));
     if ((rc = launch_solve(h, B, io, rg))) return rc;
     CUDA_TRY(h, cudaEventRecord(h->ev1, s));
@@ -1029,22 +1047,16 @@ static int host_enqueue(mpcb200_handle* h, int64_t B, const SolveArgs& a, const 
 }
 
 /* ... and bring the slice's results back into the caller's buffers (synchronises the device's stream) */
-static int host_collect(mpcb200_handle* h, int64_t B, const SolveArgs& a) {
+static int host_collect(mpcb200_handle* h, int64_t B, const SolveArgs& a, int64_t lo) {
     CUDA_TRY(h, cudaSetDevice(h->device));
-    const bool on_path = (a.path_of != nullptr);
-    const int N = h->cfg.N;
-    const size_t nt = 6 * (size_t)N + 4, nr = h->model ? 4 : 3 * ((size_t)N + 1);
-    const size_t br = B * nr * sizeof(double), bu = B * 2 * sizeof(double), bt = B * nt * sizeof(double);
+    CallArray t[A_COUNT];
+    call_arrays(h, a, lo, t);
     cudaStream_t s = h->stream;
-    if (a.u0) { CUDA_TRY(h, cudaMemcpyAsync(a.u0, h->d_u0.p, bu, cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += bu; }
-    if (a.cost) { CUDA_TRY(h, cudaMemcpyAsync(a.cost, h->d_cost.p, B * sizeof(double), cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += B * sizeof(double); }
-    if (a.status) { CUDA_TRY(h, cudaMemcpyAsync(a.status, h->d_status.p, B * sizeof(int32_t), cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += B * sizeof(int32_t); }
-    if (a.iters) { CUDA_TRY(h, cudaMemcpyAsync(a.iters, h->d_iters.p, B * sizeof(int32_t), cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += B * sizeof(int32_t); }
-    if (a.traj) { CUDA_TRY(h, cudaMemcpyAsync(a.traj, h->d_traj.p, bt, cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += bt; }
-    if (a.warm) { CUDA_TRY(h, cudaMemcpyAsync(a.warm, h->d_warm.p, bt, cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += bt; }
-    if (a.rec) { CUDA_TRY(h, cudaMemcpyAsync(a.rec, h->d_rec.p, B * 4 * sizeof(double), cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += B * 4 * sizeof(double); }
-    if (on_path && a.ref_out) { CUDA_TRY(h, cudaMemcpyAsync(a.ref_out, h->d_ref.p, br, cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += br; }
-    if (on_path && a.stop) { CUDA_TRY(h, cudaMemcpyAsync(a.stop, h->d_stop.p, B * sizeof(int32_t), cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += B * sizeof(int32_t); }
+    for (int i = 0; i < A_COUNT; i++) {
+        if (!t[i].host || !(t[i].dir & DIR_OUT)) continue;
+        CUDA_TRY(h, cudaMemcpyAsync(t[i].host, t[i].dev->p, t[i].row * B, cudaMemcpyDeviceToHost, s));
+        h->stats.d2h_bytes += t[i].row * B;
+    }
     CUDA_TRY(h, cudaStreamSynchronize(s));
     float ms = 0.f;
     CUDA_TRY(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
@@ -1071,12 +1083,8 @@ static int solve_batch_impl(mpcb200_handle* h, int64_t B, const SolveArgs& a, in
     if (!a.state || (!a.ref && !on_path) || !a.u_prev || (!a.u0 && !a.rec))
         return fail(h, MPCB200_EINVAL, "%s: state, %s, u_prev and %s are required", who, on_path ? "path_of" : "ref", a.rec ? "rec" : "u0");
     if (on_path && h->model) return fail(h, MPCB200_EINVAL, "%s: not available for the Frenet-frame variant", who);
-    if (a.w && mem_space == MPCB200_HOST) {   /* (device rows are checked by the kernel: MPCB200_ERROR for that problem) */
-        const size_t nw = weight_row(h->model);
-        for (int64_t b = 0; b < B; b++)
-            for (size_t i = 0; i < nw; i++)
-                if (!(a.w[b * nw + i] >= 0.0)) return fail(h, MPCB200_EINVAL, "%s: weight %d of problem %lld is negative or NaN", who, (int)i, (long long)b);
-    }
+    int rc;
+    if (a.w && mem_space == MPCB200_HOST && (rc = check_weight_rows(h, who, "problem", B, a.w, weight_row(h->model)))) return rc;
     CUDA_TRY(h, cudaSetDevice(h->device));
     RefGen rg;
     memset(&rg, 0, sizeof(rg));
@@ -1084,38 +1092,25 @@ static int solve_batch_impl(mpcb200_handle* h, int64_t B, const SolveArgs& a, in
         fill_paths(h, rg.paths);
         rg.track_using_time = a.track_using_time;
         rg.target_vel = a.target_vel > 0.0 ? a.target_vel : 0.0;   /* des_speed, mpc_cmd_pub.jl:58-62 */
-        if (mem_space == MPCB200_HOST) {
-            for (int64_t b = 0; b < B; b++)
-                if (a.path_of[b] < 0 || a.path_of[b] > 2 || h->path_n[a.path_of[b]] == 0)
-                    return fail(h, MPCB200_EINVAL, "%s: problem %lld uses path %d, which was not set with mpcb200_set_path", who, (long long)b, a.path_of[b]);
-        }
+        if (mem_space == MPCB200_HOST && (rc = check_path_ids(h, who, "problem", B, a.path_of))) return rc;
     }
     if (mem_space == MPCB200_DEVICE) {
-        int rc;
         if ((rc = ensure(h, h->d_resto, B * sizeof(int32_t)))) return rc;
-        BatchPtrs io{a.state, a.ref, a.v_des, a.u_prev, a.warm, a.u0, a.cost, a.status, a.iters, a.traj, a.rec, (int*)h->d_resto.p, a.w};
-        rg.path_of = a.path_of; rg.ref_out = a.ref_out; rg.stop = a.stop;
+        CallArray t[A_COUNT];
+        call_arrays(h, a, 0, t);
+        void* p[A_COUNT];
+        for (int i = 0; i < A_COUNT; i++) p[i] = t[i].host;
+        const BatchPtrs io = batch_ptrs(p, (int*)h->d_resto.p, rg);
         return launch_solve(h, B, io, rg);
     }
     if (!on_path && B <= SMALL_BATCH) return solve_small_host(h, B, a);
-    /* host pointers: one contiguous slice per device, all devices working at once */
-    const int parts = (B >= 2 * (int64_t)(h->n_sub + 1)) ? h->n_sub + 1 : 1;
     mpcb200_handle* dev[8];
-    dev[0] = h;
-    for (int i = 0; i < h->n_sub; i++) dev[i + 1] = h->sub[i];
-    int rc;
-    for (int i = 0; i < parts; i++) {
-        shard_range(B, parts, i, &h->slice_lo[i], &h->slice_hi[i]);
-        if (i) memset(&dev[i]->stats, 0, sizeof(mpcb200_stats));
-        if ((rc = host_enqueue(dev[i], h->slice_hi[i] - h->slice_lo[i], slice_args(a, h->slice_lo[i], h->cfg.N, h->model), rg))) return sub_fail(h, dev[i], rc);
-    }
+    const int parts = slice_call(h, B, h->n_sub + 1, dev, h->slice_lo, h->slice_hi);
     for (int i = 0; i < parts; i++)
-        if ((rc = host_collect(dev[i], h->slice_hi[i] - h->slice_lo[i], slice_args(a, h->slice_lo[i], h->cfg.N, h->model)))) return sub_fail(h, dev[i], rc);
-    for (int i = 1; i < parts; i++) {
-        h->stats.kernel_launches += dev[i]->stats.kernel_launches;
-        h->stats.h2d_bytes += dev[i]->stats.h2d_bytes; h->stats.d2h_bytes += dev[i]->stats.d2h_bytes;
-        if (dev[i]->stats.kernel_ms > h->stats.kernel_ms) h->stats.kernel_ms = dev[i]->stats.kernel_ms;   /* the devices run concurrently */
-    }
+        if ((rc = host_enqueue(dev[i], h->slice_hi[i] - h->slice_lo[i], a, h->slice_lo[i], rg))) return sub_fail(h, dev[i], rc);
+    for (int i = 0; i < parts; i++)
+        if ((rc = host_collect(dev[i], h->slice_hi[i] - h->slice_lo[i], a, h->slice_lo[i]))) return sub_fail(h, dev[i], rc);
+    merge_stats(h, dev, parts);
     h->last_sharded = parts > 1;
     for (int i = parts; i < 8; i++) h->slice_lo[i] = h->slice_hi[i] = 0;
     CUDA_TRY(h, cudaSetDevice(h->device));
@@ -1259,9 +1254,8 @@ static int ensure_seed(mpcb200_handle* h) {
     for (int k = 0; k <= N; k++) ref[k] = 15.0 * ((double)k * h->cfg.dt);
     v_des[0] = 15.0;
     double w_keep[8];
-    const double w0[8] = {9.0, 9.0, 10.0, 0.0, 100.0, 1000.0, 0.0, 0.0};
     memcpy(w_keep, h->w, sizeof(w_keep));
-    memcpy(h->w, w0, sizeof(w0));
+    memcpy(h->w, W_XY_DEFAULT, sizeof(W_XY_DEFAULT));
     const int start_keep = h->cfg.start_mode;
     h->cfg.start_mode = MPCB200_START_ZERO;
     drop_graphs(h);   /* weights and start mode are kernel parameters */
@@ -1284,38 +1278,68 @@ static int ensure_seed(mpcb200_handle* h) {
     return rc;
 }
 
+/* one closed-loop call: mpcb200_rollout and mpcb200_rollout_w (model 0) or mpcb200_rollout_frenet (model 1) */
+struct RolloutCall {
+    const char* who;
+    int model;
+    int64_t B; int32_t T;
+    const double* pose0; const int32_t* path_of;
+    double target_vel;
+    int32_t track_using_time; const double* w;   /* XY: waypoints by time or arc length; [B][8] weight rows or null */
+    double window; int32_t ey_from_path;          /* Frenet: length of the path ahead, e_y from the path or from the fit */
+    double* log; double* final_state;             /* [T][B][8], [B][8] or null */
+};
+
 /* one device's share of a rollout: vehicles [lo, lo + n) of B; enqueue ... */
-static int rollout_enqueue(mpcb200_handle* h, int64_t n, int32_t T, const double* pose0, const int32_t* path_of, int32_t track_using_time,
-                           double target_vel, const double* w, bool want_log, bool want_final) {
+static int rollout_enqueue(mpcb200_handle* h, const RolloutCall& c, int64_t lo, int64_t n) {
     CUDA_TRY(h, cudaSetDevice(h->device));
+    cudaStream_t s = h->stream;
     int rc;
-    if ((rc = ensure_seed(h))) return rc;
-    const size_t bl = (size_t)T * n * 8 * sizeof(double), bf = (size_t)n * 8 * sizeof(double);
+    if (!c.model && (rc = ensure_seed(h))) return rc;
+    if (c.model && h->fit_window != c.window) {   /* grids of nav_msgs_path_frenet.py:63,79: arange(0, window, 0.5) and arange(0, window, 0.25) */
+        const int n1 = (int)ceil(c.window / 0.5 - 1e-9), n2 = (int)ceil(c.window / 0.25 - 1e-9);
+        double* P = (double*)malloc(sizeof(double) * 4 * ((size_t)n1 + n2));
+        if (!P) return fail(h, MPCB200_ENOMEM, "%s: out of host memory", c.who);
+        cubic_fit_matrix(n1, 0.5, P); cubic_fit_matrix(n2, 0.25, P + 4 * (size_t)n1);
+        rc = ensure(h, h->d_fit, sizeof(double) * 4 * ((size_t)n1 + n2));
+        if (!rc) {
+            cudaError_t e = cudaMemcpyAsync(h->d_fit.p, P, sizeof(double) * 4 * ((size_t)n1 + n2), cudaMemcpyHostToDevice, s);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+            if (e != cudaSuccess) rc = fail(h, MPCB200_ECUDA, "%s: %s", c.who, cudaGetErrorString(e));
+        }
+        free(P);
+        if (rc) return rc;
+        h->fit_window = c.window; h->fit_n1 = n1; h->fit_n2 = n2;
+    }
     if ((rc = ensure(h, h->d_pose, (size_t)n * 3 * sizeof(double)))) return rc;
     if ((rc = ensure(h, h->d_pathof, (size_t)n * sizeof(int32_t)))) return rc;
-    if (want_log && (rc = ensure(h, h->d_log, bl))) return rc;
-    if (want_final && (rc = ensure(h, h->d_final, bf))) return rc;
-    cudaStream_t s = h->stream;
-    CUDA_TRY(h, cudaMemcpyAsync(h->d_pose.p, pose0, (size_t)n * 3 * sizeof(double), cudaMemcpyHostToDevice, s));
-    CUDA_TRY(h, cudaMemcpyAsync(h->d_pathof.p, path_of, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    if (c.log && (rc = ensure(h, h->d_log, (size_t)c.T * n * 8 * sizeof(double)))) return rc;
+    if (c.final_state && (rc = ensure(h, h->d_final, (size_t)n * 8 * sizeof(double)))) return rc;
+    CUDA_TRY(h, cudaMemcpyAsync(h->d_pose.p, c.pose0 + 3 * lo, (size_t)n * 3 * sizeof(double), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(h, cudaMemcpyAsync(h->d_pathof.p, c.path_of + lo, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     h->stats.h2d_bytes += (size_t)n * (3 * sizeof(double) + sizeof(int32_t));
-    if (w) {
+    if (c.w) {
         if ((rc = ensure(h, h->d_w, (size_t)n * 8 * sizeof(double)))) return rc;
-        CUDA_TRY(h, cudaMemcpyAsync(h->d_w.p, w, (size_t)n * 8 * sizeof(double), cudaMemcpyHostToDevice, s));
+        CUDA_TRY(h, cudaMemcpyAsync(h->d_w.p, c.w + 8 * lo, (size_t)n * 8 * sizeof(double), cudaMemcpyHostToDevice, s));
         h->stats.h2d_bytes += (size_t)n * 8 * sizeof(double);
     }
+    /* the kernel arguments of both models; only those of c.model are launched with */
     RolloutArgs a;
+    FrenetRolloutArgs fa;
     memset(&a, 0, sizeof(a));
-    a.pose0 = (const double*)h->d_pose.p; a.path_of = (const int*)h->d_pathof.p;
-    fill_paths(h, a.paths);
-    a.T = T; a.track_using_time = track_using_time; a.target_vel = target_vel;
-    a.log = want_log ? (double*)h->d_log.p : nullptr; a.final_state = want_final ? (double*)h->d_final.p : nullptr; a.B = (long)n;
-    a.warm0 = (const double*)h->d_seed.p;
-    a.w = w ? (const double*)h->d_w.p : nullptr;
-    /* large fleets at short horizons: one control period = plant / waypoints / thread-per-problem solve over the whole fleet.
-     * Measured at N = 8, 200 periods (profiles/r02_logs/r02_rollout_thresholds.log): a period of the pipeline takes ~0.9 ms up to
-     * 8,192 vehicles (the slowest vehicle's dozen solver trips) and grows slowly after that, the fused kernel takes 0.5 / 0.8 /
-     * 1.4 / 2.5 ms at 2,048 / 4,096 / 8,192 / 16,384 vehicles: the default rule switches at a quarter of the cold-start batch */
+    memset(&fa, 0, sizeof(fa));
+    a.pose0 = fa.pose0 = (const double*)h->d_pose.p; a.path_of = fa.path_of = (const int*)h->d_pathof.p;
+    fill_paths(h, a.paths); fill_paths(h, fa.paths);
+    a.T = fa.T = c.T; a.target_vel = fa.target_vel = c.target_vel; a.B = fa.B = (long)n;
+    a.log = fa.log = c.log ? (double*)h->d_log.p : nullptr; a.final_state = fa.final_state = c.final_state ? (double*)h->d_final.p : nullptr;
+    a.track_using_time = c.track_using_time; a.warm0 = (const double*)h->d_seed.p; a.w = c.w ? (const double*)h->d_w.p : nullptr;
+    fa.ey_from_path = c.ey_from_path;
+    fa.P1 = (const double*)h->d_fit.p; fa.P2 = fa.P1 + 4 * (size_t)h->fit_n1; fa.n1 = h->fit_n1; fa.n2 = h->fit_n2;
+    const KCfg kc = make_kcfg(h);
+    /* large fleets at short horizons: one control period = plant / reference / thread-per-problem solve over the whole fleet.
+     * Measured for the XY model at N = 8, 200 periods (profiles/r02_logs/r02_rollout_thresholds.log): a period of the pipeline takes
+     * ~0.9 ms up to 8,192 vehicles (the slowest vehicle's dozen solver trips) and grows slowly after that, the fused kernel takes
+     * 0.5 / 0.8 / 1.4 / 2.5 ms at 2,048 / 4,096 / 8,192 / 16,384 vehicles: the default rule switches at a quarter of the cold-start batch */
     const int64_t roll_from = h->tpp_default_rule ? h->tpp_min_batch / 4 : h->tpp_min_batch;
     if (h->tpp_min_batch > 0 && n >= roll_from) {
         const long long Bp = (n + 31) / 32 * 32;
@@ -1323,67 +1347,76 @@ static int rollout_enqueue(mpcb200_handle* h, int64_t n, int32_t T, const double
          * blocks mean less idle SMs in the last wave (16,384 vehicles: 0.89 instead of 1.07 ms per period; never slower) */
         const int tb = h->tpp_block < 128 ? h->tpp_block : 128;
         const long long sblocks = (n + tb - 1) / tb, S = sblocks * tb;
-        if ((rc = ensure(h, h->d_tpp_state, tpp_state_doubles(h->cfg.N, (long)S) * sizeof(double)))) return rc;
+        /* vehicle state [RV_NF][Bp], then for the Frenet model the reference of the period [6][Bp] */
+        const size_t veh_rows = c.model ? RV_NF + 6 : RV_NF;
+        if ((rc = ensure(h, h->d_tpp_state, tpp_state_doubles(h->cfg.N, (long)S, c.model) * sizeof(double)))) return rc;
         if ((rc = ensure(h, h->d_tpp_filt, tpp_filter_doubles((long)S) * sizeof(double)))) return rc;
-        if ((rc = ensure(h, h->d_veh, (size_t)RV_NF * Bp * sizeof(double)))) return rc;
-        if ((rc = ensure(h, h->d_vstop, (size_t)Bp * sizeof(int)))) return rc;
+        if ((rc = ensure(h, h->d_veh, veh_rows * Bp * sizeof(double)))) return rc;
+        if (!c.model && (rc = ensure(h, h->d_vstop, (size_t)Bp * sizeof(int)))) return rc;
         if ((rc = ensure(h, h->d_u0, (size_t)n * 2 * sizeof(double)))) return rc;
         if ((rc = ensure(h, h->d_status, (size_t)n * sizeof(int32_t)))) return rc;
         if ((rc = ensure(h, h->d_iters, (size_t)n * sizeof(int32_t)))) return rc;
         BatchPtrs out;
         memset(&out, 0, sizeof(out));
         out.u0 = (double*)h->d_u0.p; out.status = (int*)h->d_status.p; out.iters = (int*)h->d_iters.p; out.w = a.w;
-        auto sk = a.w ? rollout_solve_tpp_kernel<0, 1> : rollout_solve_tpp_kernel<0, 0>;
+        auto sk = c.model ? rollout_solve_tpp_kernel<1, 0> : (a.w ? rollout_solve_tpp_kernel<0, 1> : rollout_solve_tpp_kernel<0, 0>);
         RefGen rg;
         memset(&rg, 0, sizeof(rg));
         fill_paths(h, rg.paths);
-        rg.track_using_time = track_using_time;
-        const double des_speed = target_vel > 0.0 ? target_vel : 0.0;   /* mpc_cmd_pub.jl:58-62 */
+        rg.track_using_time = c.track_using_time;
+        /* XY: des_speed of mpc_cmd_pub.jl:58-62; the Frenet node uses its target speed as given */
+        const double des_speed = (c.model || c.target_vel > 0.0) ? c.target_vel : 0.0;
         rg.target_vel = des_speed;
-        const KCfg kc = make_kcfg(h);
         double* veh = (double*)h->d_veh.p;
+        double* fref = c.model ? veh + (size_t)RV_NF * Bp : nullptr;
+        int* stop = c.model ? nullptr : (int*)h->d_vstop.p;
+        double* st = (double*)h->d_tpp_state.p;
+        double* filt = (double*)h->d_tpp_filt.p;
         const int pgrid = (int)((n + 127) / 128);
         long long wblocks = (n + 3) / 4, wmax = (long long)h->num_sms * 16;
         const int wgrid = (int)(wblocks < wmax ? wblocks : wmax);
         CUDA_TRY(h, cudaEventRecord(h->ev0, s));
-        for (int t = 0; t < T; t++) {
+        for (int t = 0; t < c.T; t++) {
             rollout_plant_kernel<<<pgrid, 128, 0, s>>>((long long)n, Bp, veh, a.pose0, t == 0);
-            rollout_waypoints_kernel<<<wgrid, 128, 0, s>>>(kc, (long long)n, Bp, veh, a.path_of, rg, (double*)h->d_tpp_state.p, (double*)h->d_tpp_filt.p,
-                                                          (int*)h->d_vstop.p, t == 0);
-            sk<<<(int)sblocks, tb, 0, s>>>(kc, (long long)n, Bp, veh, (const int*)h->d_vstop.p, (double*)h->d_tpp_state.p, (double*)h->d_tpp_filt.p,
-                                           t == 0 ? a.warm0 : nullptr, des_speed, out, a.log ? a.log + (size_t)t * n * 8 : nullptr, nullptr, t == 0);
+            if (c.model) rollout_frenet_ref_kernel<<<wgrid, 128, 0, s>>>(kc, fa, Bp, veh, fref);
+            else rollout_waypoints_kernel<<<wgrid, 128, 0, s>>>(kc, (long long)n, Bp, veh, a.path_of, rg, st, filt, stop, t == 0);
+            sk<<<(int)sblocks, tb, 0, s>>>(kc, (long long)n, Bp, veh, stop, st, filt, (!c.model && t == 0) ? a.warm0 : nullptr, des_speed, out,
+                                           a.log ? a.log + (size_t)t * n * 8 : nullptr, fref, t == 0);
             CUDA_TRY(h, cudaGetLastError());
         }
         if (a.final_state) rollout_final_kernel<<<pgrid, 128, 0, s>>>((long long)n, Bp, veh, a.final_state);
         CUDA_TRY(h, cudaGetLastError());
         CUDA_TRY(h, cudaEventRecord(h->ev1, s));
-        h->stats.kernel_launches += 3 * (int64_t)T + (a.final_state ? 1 : 0);
+        h->stats.kernel_launches += 3 * (int64_t)c.T + (a.final_state ? 1 : 0);
         return MPCB200_OK;
     }
     CUDA_TRY(h, cudaMemsetAsync(h->d_counter, 0, sizeof(unsigned long long), s));
     const int per_block = (h->team_warps == 1) ? WARPS_PER_BLOCK : 1;
     long long blocks_needed = (n + per_block - 1) / per_block;
-    long long max_blocks = (long long)h->num_sms * (w ? h->rollout_blocks_per_sm_w : h->rollout_blocks_per_sm);
-    int grid = (int)(blocks_needed < max_blocks ? blocks_needed : max_blocks);
-    const RolloutKernel rk = w ? rollout_kernel<1>(h) : rollout_kernel<0>(h);
+    const int bps = c.model ? h->frenet_rollout_blocks_per_sm : (c.w ? h->rollout_blocks_per_sm_w : h->rollout_blocks_per_sm);
+    long long max_blocks = (long long)h->num_sms * bps;
+    const int grid = (int)(blocks_needed < max_blocks ? blocks_needed : max_blocks);
+    const int threads = 32 * (h->team_warps == 1 ? WARPS_PER_BLOCK : h->team_warps);
+    const size_t smem = rollout_smem_bytes(h, c.w != nullptr);
     CUDA_TRY(h, cudaEventRecord(h->ev0, s));
-    rk<<<grid, 32 * (h->team_warps == 1 ? WARPS_PER_BLOCK : h->team_warps), rollout_smem_bytes(h, w != nullptr), s>>>(make_kcfg(h), a, h->d_counter);
+    if (c.model) mpc_rollout_frenet_kernel<<<grid, threads, smem, s>>>(kc, fa, h->d_counter);
+    else (c.w ? rollout_kernel<1>(h) : rollout_kernel<0>(h))<<<grid, threads, smem, s>>>(kc, a, h->d_counter);
     CUDA_TRY(h, cudaGetLastError());
     CUDA_TRY(h, cudaEventRecord(h->ev1, s));
     h->stats.kernel_launches += 1;
     return MPCB200_OK;
 }
 
-/* ... and copy the share's rows of log [T][B][8] (a strided block when the fleet is sharded) and final [B][8] back */
-static int rollout_collect(mpcb200_handle* h, int64_t lo, int64_t n, int64_t B, int32_t T, double* log, double* final_state) {
+/* ... and copy the share's rows of log [T][B][8] (a strided block when the fleet is sliced) and final [B][8] back */
+static int rollout_collect(mpcb200_handle* h, const RolloutCall& c, int64_t lo, int64_t n) {
     CUDA_TRY(h, cudaSetDevice(h->device));
     cudaStream_t s = h->stream;
     const size_t row = (size_t)n * 8 * sizeof(double);
-    if (log) {
-        CUDA_TRY(h, cudaMemcpy2DAsync(log + (size_t)lo * 8, (size_t)B * 8 * sizeof(double), h->d_log.p, row, row, (size_t)T, cudaMemcpyDeviceToHost, s));
-        h->stats.d2h_bytes += row * T;
+    if (c.log) {
+        CUDA_TRY(h, cudaMemcpy2DAsync(c.log + (size_t)lo * 8, (size_t)c.B * 8 * sizeof(double), h->d_log.p, row, row, (size_t)c.T, cudaMemcpyDeviceToHost, s));
+        h->stats.d2h_bytes += row * c.T;
     }
-    if (final_state) { CUDA_TRY(h, cudaMemcpyAsync(final_state + (size_t)lo * 8, h->d_final.p, row, cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += row; }
+    if (c.final_state) { CUDA_TRY(h, cudaMemcpyAsync(c.final_state + (size_t)lo * 8, h->d_final.p, row, cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += row; }
     CUDA_TRY(h, cudaStreamSynchronize(s));
     float ms = 0.f;
     CUDA_TRY(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
@@ -1391,163 +1424,49 @@ static int rollout_collect(mpcb200_handle* h, int64_t lo, int64_t n, int64_t B, 
     return MPCB200_OK;
 }
 
-/* mpcb200_rollout and mpcb200_rollout_w (w == NULL: the handle's weights) */
-static int rollout_impl(const char* who, mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of,
-                        int32_t track_using_time, double target_vel, const double* w, double* log, double* final_state) {
+/* the body of mpcb200_rollout, mpcb200_rollout_w (w == NULL: the handle's weights) and mpcb200_rollout_frenet */
+static int rollout_impl(mpcb200_handle* h, const RolloutCall& c) {
+    const char* who = c.who;
     if (!h) return MPCB200_EINVAL;
-    if (B < 0 || T < 0) return fail(h, MPCB200_EINVAL, "%s: B=%lld T=%d", who, (long long)B, T);
-    if (h->model) return fail(h, MPCB200_EINVAL, "%s: not available for the Frenet-frame variant", who);
+    if (c.B < 0 || c.T < 0) return fail(h, MPCB200_EINVAL, "%s: B=%lld T=%d", who, (long long)c.B, c.T);
+    if (h->model != c.model)
+        return fail(h, MPCB200_EINVAL, c.model ? "%s: the handle was not created with mpcb200_create_frenet" : "%s: not available for the Frenet-frame variant", who);
+    if (c.model && h->team_warps != 1) return fail(h, MPCB200_EINVAL, "%s: N <= 31 (N=%d)", who, h->cfg.N);
+    if (c.model && !(c.window >= 4.0 && c.window <= 500.0)) return fail(h, MPCB200_EINVAL, "%s: window %.3g m outside [4, 500]", who, c.window);
     memset(&h->stats, 0, sizeof(h->stats));
-    if (B == 0 || T == 0) return MPCB200_OK;
-    if (!pose0 || !path_of) return fail(h, MPCB200_EINVAL, "%s: pose0 and path_of are required", who);
-    for (int64_t b = 0; b < B; b++)
-        if (path_of[b] < 0 || path_of[b] > 2 || h->path_n[path_of[b]] == 0)
-            return fail(h, MPCB200_EINVAL, "%s: vehicle %lld uses path %d, which was not set with mpcb200_set_path", who, (long long)b, path_of[b]);
-    if (w)
-        for (int64_t b = 0; b < B; b++)
-            for (int i = 0; i < 8; i++)
-                if (!(w[8 * b + i] >= 0.0)) return fail(h, MPCB200_EINVAL, "%s: weight %d of vehicle %lld is negative or NaN", who, i, (long long)b);
-    /* a vehicle stays on one GPU for all T steps: contiguous slices of the fleet, every device at once */
-    const int parts = (B >= 2 * (int64_t)(h->n_sub + 1)) ? h->n_sub + 1 : 1;
-    mpcb200_handle* dev[8];
-    dev[0] = h;
-    for (int i = 0; i < h->n_sub; i++) dev[i + 1] = h->sub[i];
-    int64_t lo[8], hi[8];
+    if (c.B == 0 || c.T == 0) return MPCB200_OK;
+    if (!c.pose0 || !c.path_of) return fail(h, MPCB200_EINVAL, "%s: pose0 and path_of are required", who);
     int rc;
-    for (int i = 0; i < parts; i++) {
-        shard_range(B, parts, i, &lo[i], &hi[i]);
-        if (i) memset(&dev[i]->stats, 0, sizeof(mpcb200_stats));
-        if ((rc = rollout_enqueue(dev[i], hi[i] - lo[i], T, pose0 + 3 * lo[i], path_of + lo[i], track_using_time, target_vel,
-                                  w ? w + 8 * lo[i] : nullptr, log != nullptr, final_state != nullptr)))
-            return sub_fail(h, dev[i], rc);
-    }
+    if ((rc = check_path_ids(h, who, "vehicle", c.B, c.path_of))) return rc;
+    if (c.w && (rc = check_weight_rows(h, who, "vehicle", c.B, c.w, 8))) return rc;
+    /* a vehicle stays on one GPU for all T steps: contiguous slices of the fleet, every device at once.  Frenet fleets run on
+     * devices[0] only, as mpc_b200.h documents */
+    mpcb200_handle* dev[8];
+    int64_t lo[8], hi[8];
+    const int parts = slice_call(h, c.B, c.model ? 1 : h->n_sub + 1, dev, lo, hi);
     for (int i = 0; i < parts; i++)
-        if ((rc = rollout_collect(dev[i], lo[i], hi[i] - lo[i], B, T, log, final_state))) return sub_fail(h, dev[i], rc);
-    for (int i = 1; i < parts; i++) {
-        h->stats.kernel_launches += dev[i]->stats.kernel_launches;
-        h->stats.h2d_bytes += dev[i]->stats.h2d_bytes; h->stats.d2h_bytes += dev[i]->stats.d2h_bytes;
-        if (dev[i]->stats.kernel_ms > h->stats.kernel_ms) h->stats.kernel_ms = dev[i]->stats.kernel_ms;
-    }
+        if ((rc = rollout_enqueue(dev[i], c, lo[i], hi[i] - lo[i]))) return sub_fail(h, dev[i], rc);
+    for (int i = 0; i < parts; i++)
+        if ((rc = rollout_collect(dev[i], c, lo[i], hi[i] - lo[i]))) return sub_fail(h, dev[i], rc);
+    merge_stats(h, dev, parts);
     CUDA_TRY(h, cudaSetDevice(h->device));
     return MPCB200_OK;
 }
 
 int mpcb200_rollout(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, int32_t track_using_time,
                     double target_vel, double* log, double* final_state) {
-    return rollout_impl("mpcb200_rollout", h, B, T, pose0, path_of, track_using_time, target_vel, nullptr, log, final_state);
+    return rollout_impl(h, {"mpcb200_rollout", 0, B, T, pose0, path_of, target_vel, track_using_time, nullptr, 0.0, 0, log, final_state});
 }
 
 int mpcb200_rollout_w(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, int32_t track_using_time,
                       double target_vel, const double* w, double* log, double* final_state) {
     if (h && !w && B > 0 && T > 0) return fail(h, MPCB200_EINVAL, "mpcb200_rollout_w: w is required");
-    return rollout_impl("mpcb200_rollout_w", h, B, T, pose0, path_of, track_using_time, target_vel, w, log, final_state);
+    return rollout_impl(h, {"mpcb200_rollout_w", 0, B, T, pose0, path_of, target_vel, track_using_time, w, 0.0, 0, log, final_state});
 }
 
 int mpcb200_rollout_frenet(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, double window,
                            double target_vel, int32_t ey_from_path, double* log, double* final_state) {
-    if (!h) return MPCB200_EINVAL;
-    if (B < 0 || T < 0) return fail(h, MPCB200_EINVAL, "mpcb200_rollout_frenet: B=%lld T=%d", (long long)B, T);
-    if (!h->model) return fail(h, MPCB200_EINVAL, "mpcb200_rollout_frenet: the handle was not created with mpcb200_create_frenet");
-    if (h->team_warps != 1) return fail(h, MPCB200_EINVAL, "mpcb200_rollout_frenet: N <= 31 (N=%d)", h->cfg.N);
-    if (!(window >= 4.0 && window <= 500.0)) return fail(h, MPCB200_EINVAL, "mpcb200_rollout_frenet: window %.3g m outside [4, 500]", window);
-    memset(&h->stats, 0, sizeof(h->stats));
-    if (B == 0 || T == 0) return MPCB200_OK;
-    if (!pose0 || !path_of) return fail(h, MPCB200_EINVAL, "mpcb200_rollout_frenet: pose0 and path_of are required");
-    for (int64_t b = 0; b < B; b++)
-        if (path_of[b] < 0 || path_of[b] > 2 || h->path_n[path_of[b]] == 0)
-            return fail(h, MPCB200_EINVAL, "mpcb200_rollout_frenet: vehicle %lld uses path %d, which was not set with mpcb200_set_path", (long long)b, path_of[b]);
-    CUDA_TRY(h, cudaSetDevice(h->device));
-    cudaStream_t s = h->stream;
-    int rc;
-    if (h->fit_window != window) {   /* grids of nav_msgs_path_frenet.py:63,79: arange(0, window, 0.5) and arange(0, window, 0.25) */
-        const int n1 = (int)ceil(window / 0.5 - 1e-9), n2 = (int)ceil(window / 0.25 - 1e-9);
-        double* P = (double*)malloc(sizeof(double) * 4 * ((size_t)n1 + n2));
-        if (!P) return fail(h, MPCB200_ENOMEM, "mpcb200_rollout_frenet: out of host memory");
-        cubic_fit_matrix(n1, 0.5, P); cubic_fit_matrix(n2, 0.25, P + 4 * (size_t)n1);
-        rc = ensure(h, h->d_fit, sizeof(double) * 4 * ((size_t)n1 + n2));
-        if (!rc) {
-            cudaError_t e = cudaMemcpyAsync(h->d_fit.p, P, sizeof(double) * 4 * ((size_t)n1 + n2), cudaMemcpyHostToDevice, s);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-            if (e != cudaSuccess) rc = fail(h, MPCB200_ECUDA, "mpcb200_rollout_frenet: %s", cudaGetErrorString(e));
-        }
-        free(P);
-        if (rc) return rc;
-        h->fit_window = window; h->fit_n1 = n1; h->fit_n2 = n2;
-    }
-    const size_t bl = (size_t)T * B * 8 * sizeof(double), bf = (size_t)B * 8 * sizeof(double);
-    if ((rc = ensure(h, h->d_pose, (size_t)B * 3 * sizeof(double)))) return rc;
-    if ((rc = ensure(h, h->d_pathof, (size_t)B * sizeof(int32_t)))) return rc;
-    if (log && (rc = ensure(h, h->d_log, bl))) return rc;
-    if (final_state && (rc = ensure(h, h->d_final, bf))) return rc;
-    CUDA_TRY(h, cudaMemcpyAsync(h->d_pose.p, pose0, (size_t)B * 3 * sizeof(double), cudaMemcpyHostToDevice, s));
-    CUDA_TRY(h, cudaMemcpyAsync(h->d_pathof.p, path_of, (size_t)B * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-    h->stats.h2d_bytes += (size_t)B * (3 * sizeof(double) + sizeof(int32_t));
-    FrenetRolloutArgs a;
-    memset(&a, 0, sizeof(a));
-    a.pose0 = (const double*)h->d_pose.p; a.path_of = (const int*)h->d_pathof.p;
-    fill_paths(h, a.paths);
-    a.T = T; a.ey_from_path = ey_from_path; a.target_vel = target_vel;
-    a.log = log ? (double*)h->d_log.p : nullptr; a.final_state = final_state ? (double*)h->d_final.p : nullptr; a.B = (long)B;
-    a.P1 = (const double*)h->d_fit.p; a.P2 = a.P1 + 4 * (size_t)h->fit_n1; a.n1 = h->fit_n1; a.n2 = h->fit_n2;
-    /* large fleets: one control period = plant / Frenet reference / thread-per-problem solve over the whole fleet (as mpcb200_rollout
-     * does for the XY model); the default switch is a quarter of the batch rule */
-    const int64_t roll_from = h->tpp_default_rule ? h->tpp_min_batch / 4 : h->tpp_min_batch;
-    if (h->tpp_min_batch > 0 && B >= roll_from) {
-        const long long Bp = (B + 31) / 32 * 32;
-        const int tb = h->tpp_block < 128 ? h->tpp_block : 128;
-        const long long sblocks = (B + tb - 1) / tb, S = sblocks * tb;
-        if ((rc = ensure(h, h->d_tpp_state, tpp_state_doubles(h->cfg.N, (long)S, 1) * sizeof(double)))) return rc;
-        if ((rc = ensure(h, h->d_tpp_filt, tpp_filter_doubles((long)S) * sizeof(double)))) return rc;
-        if ((rc = ensure(h, h->d_veh, (size_t)(RV_NF + 6) * Bp * sizeof(double)))) return rc;
-        if ((rc = ensure(h, h->d_u0, (size_t)B * 2 * sizeof(double)))) return rc;
-        if ((rc = ensure(h, h->d_status, (size_t)B * sizeof(int32_t)))) return rc;
-        if ((rc = ensure(h, h->d_iters, (size_t)B * sizeof(int32_t)))) return rc;
-        BatchPtrs out;
-        memset(&out, 0, sizeof(out));
-        out.u0 = (double*)h->d_u0.p; out.status = (int*)h->d_status.p; out.iters = (int*)h->d_iters.p;
-        const KCfg kc = make_kcfg(h);
-        double* veh = (double*)h->d_veh.p;
-        double* fref = veh + (size_t)RV_NF * Bp;
-        const int pgrid = (int)((B + 127) / 128);
-        long long wblocks = (B + 3) / 4, wmax = (long long)h->num_sms * 16;
-        const int wgrid = (int)(wblocks < wmax ? wblocks : wmax);
-        CUDA_TRY(h, cudaEventRecord(h->ev0, s));
-        for (int t = 0; t < T; t++) {
-            rollout_plant_kernel<<<pgrid, 128, 0, s>>>((long long)B, Bp, veh, a.pose0, t == 0);
-            rollout_frenet_ref_kernel<<<wgrid, 128, 0, s>>>(kc, a, Bp, veh, fref);
-            rollout_solve_tpp_kernel<1><<<(int)sblocks, tb, 0, s>>>(kc, (long long)B, Bp, veh, nullptr, (double*)h->d_tpp_state.p, (double*)h->d_tpp_filt.p,
-                                                                   nullptr, target_vel, out, a.log ? a.log + (size_t)t * B * 8 : nullptr, fref, t == 0);
-            CUDA_TRY(h, cudaGetLastError());
-        }
-        if (a.final_state) rollout_final_kernel<<<pgrid, 128, 0, s>>>((long long)B, Bp, veh, a.final_state);
-        CUDA_TRY(h, cudaGetLastError());
-        CUDA_TRY(h, cudaEventRecord(h->ev1, s));
-        h->stats.kernel_launches += 3 * (int64_t)T + (a.final_state ? 1 : 0);
-        if (log) { CUDA_TRY(h, cudaMemcpyAsync(log, h->d_log.p, bl, cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += bl; }
-        if (final_state) { CUDA_TRY(h, cudaMemcpyAsync(final_state, h->d_final.p, bf, cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += bf; }
-        CUDA_TRY(h, cudaStreamSynchronize(s));
-        float ms2 = 0.f;
-        CUDA_TRY(h, cudaEventElapsedTime(&ms2, h->ev0, h->ev1));
-        h->stats.kernel_ms = ms2;
-        return MPCB200_OK;
-    }
-    CUDA_TRY(h, cudaMemsetAsync(h->d_counter, 0, sizeof(unsigned long long), s));
-    long long blocks_needed = (B + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
-    long long max_blocks = (long long)h->num_sms * h->frenet_rollout_blocks_per_sm;
-    int grid = (int)(blocks_needed < max_blocks ? blocks_needed : max_blocks);
-    const size_t smem = (size_t)WARPS_PER_BLOCK * smem_doubles_per_team(h->cfg.N, 1) * sizeof(double) + WARPS_PER_BLOCK * ROLLOUT_PX * sizeof(double);
-    CUDA_TRY(h, cudaEventRecord(h->ev0, s));
-    mpc_rollout_frenet_kernel<<<grid, WARPS_PER_BLOCK * 32, smem, s>>>(make_kcfg(h), a, h->d_counter);
-    CUDA_TRY(h, cudaGetLastError());
-    CUDA_TRY(h, cudaEventRecord(h->ev1, s));
-    h->stats.kernel_launches += 1;
-    if (log) { CUDA_TRY(h, cudaMemcpyAsync(log, h->d_log.p, bl, cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += bl; }
-    if (final_state) { CUDA_TRY(h, cudaMemcpyAsync(final_state, h->d_final.p, bf, cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += bf; }
-    CUDA_TRY(h, cudaStreamSynchronize(s));
-    float ms = 0.f;
-    CUDA_TRY(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
-    h->stats.kernel_ms = ms;
-    return MPCB200_OK;
+    return rollout_impl(h, {"mpcb200_rollout_frenet", 1, B, T, pose0, path_of, target_vel, 0, nullptr, window, ey_from_path, log, final_state});
 }
 
 int mpcb200_get_stats(mpcb200_handle* h, mpcb200_stats* out) {
