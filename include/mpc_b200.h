@@ -58,7 +58,12 @@ extern "C" {
 #define MPCB200_START_ROLLOUT 1  /* states = bicycle-model rollout of the previous command from the
                                     measured state (not a reference behaviour; opt-in) */
 
-/* Replaces the module-level constants of MKZMPCPathFollower.jl:28-48. */
+/* Replaces the module-level constants of MKZMPCPathFollower.jl:28-48.  mpcb200_create refuses (MPCB200_EINVAL, the message
+ * names the field) a constant that is not finite, dt, dt_control, L_b, a_max, a_dmax, steer_dmax or tol <= 0, L_a < 0,
+ * v_max <= v_min, steer_max outside (0, 1.5) and max_iter < 0.
+ * tol: supported up to 1e-5.  Above that, Ipopt's barrier floor min(tol, 1e-4) / 11 (in the scaled problem) can lie above the
+ * unscaled complementarity tolerance 1e-4, and a solve that has reached the optimum of that barrier problem ends with
+ * MPCB200_ERROR (Ipopt: Search_Direction_Becomes_Too_Small), or UserLimit, instead of Optimal (DESIGN.md section 5). */
 typedef struct {
     int32_t N;            /* horizon (:34), 3 <= N <= 95: one warp per problem up to 31, one block of 2-3 warps beyond */
     int32_t max_iter;     /* iteration cap -> MPCB200_USERLIMIT */

@@ -587,10 +587,24 @@ static int create_impl(mpcb200_handle** out, const mpcb200_config* cfg, int mode
     if (!out || !cfg) return fail(nullptr, MPCB200_EINVAL, "mpcb200_create: NULL argument");
     *out = nullptr;
     if (cfg->N < 3 || cfg->N > 95) return fail(nullptr, MPCB200_EINVAL, "mpcb200_create: horizon N=%d outside [3,95]", cfg->N);
-    if (!(cfg->dt > 0) || !(cfg->dt_control > 0) || !(cfg->L_b > 0) || !(cfg->v_max > cfg->v_min) || !(cfg->a_max > 0) ||
-        !(cfg->steer_max > 0 && cfg->steer_max < 1.5) || !(cfg->a_dmax > 0) || !(cfg->steer_dmax > 0) || !(cfg->tol > 0) ||
-        cfg->max_iter < 0)
-        return fail(nullptr, MPCB200_EINVAL, "mpcb200_create: invalid model constants");
+    if (cfg->max_iter < 0) return fail(nullptr, MPCB200_EINVAL, "mpcb200_create: max_iter=%d is negative", cfg->max_iter);
+    /* every model constant must be finite: an infinite bound or step reaches kcfg_finalize, dtLb and rfrac as inf or NaN */
+    const struct { const char* name; double v; bool ok; const char* rule; } consts[] = {
+        {"dt", cfg->dt, cfg->dt > 0, "> 0"},
+        {"dt_control", cfg->dt_control, cfg->dt_control > 0, "> 0"},
+        {"L_a", cfg->L_a, cfg->L_a >= 0, ">= 0"},
+        {"L_b", cfg->L_b, cfg->L_b > 0, "> 0"},
+        {"v_min", cfg->v_min, true, "< v_max"},
+        {"v_max", cfg->v_max, cfg->v_max > cfg->v_min, "> v_min"},
+        {"a_max", cfg->a_max, cfg->a_max > 0, "> 0"},
+        {"steer_max", cfg->steer_max, cfg->steer_max > 0 && cfg->steer_max < 1.5, "in (0, 1.5)"},
+        {"a_dmax", cfg->a_dmax, cfg->a_dmax > 0, "> 0"},
+        {"steer_dmax", cfg->steer_dmax, cfg->steer_dmax > 0, "> 0"},
+        {"tol", cfg->tol, cfg->tol > 0, "> 0"},
+    };
+    for (const auto& k : consts)
+        if (!k.ok || !std::isfinite(k.v))
+            return fail(nullptr, MPCB200_EINVAL, "mpcb200_create: model constant %s = %g must be finite and %s", k.name, k.v, k.rule);
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
     if (e != cudaSuccess || ndev <= 0)

@@ -35,6 +35,39 @@ def test_default_config_matches_reference_constants():
     assert c.tol == 1e-8 and c.start_mode == capi.START_ZERO
 
 
+BAD_CONSTANTS = [(f, v) for f in ("dt", "dt_control", "L_a", "L_b", "v_min", "v_max", "a_max", "steer_max", "a_dmax", "steer_dmax", "tol")
+                 for v in (float("inf"), float("-inf"), float("nan"))] + [("L_a", -0.1), ("L_a", -1e-300)]
+
+
+@pytest.mark.parametrize("frenet", [False, True], ids=["xy", "frenet"])
+@pytest.mark.parametrize("field,value", BAD_CONSTANTS)
+def test_create_refuses_bad_constant(field, value, frenet):
+    """A constant that is not finite, or a negative L_a, is refused before any device is touched (MPCB200_EINVAL, the message
+    names the field): an infinite dt or bound or a NaN L_a would otherwise reach kcfg_finalize, dtLb and rfrac."""
+    from mkz_mpc_path_follower_b200 import capi
+    with pytest.raises(capi.MpcB200Error) as e:
+        (capi.FrenetSolver if frenet else capi.Solver)(8, **{field: value})
+    assert e.value.code == -1 and ("model constant %s = " % field) in str(e.value), str(e.value)
+
+
+def test_create_accepts_edge_constants():
+    """L_a = 0 (the rear axle as reference point) and large finite bounds are valid: without a GPU they get as far as the
+    device query (MPCB200_ENODEVICE)."""
+    try:
+        import torch
+        has_gpu = torch.cuda.is_available()
+    except Exception:
+        has_gpu = False
+    from mkz_mpc_path_follower_b200 import capi
+    for kw in (dict(L_a=0.0), dict(v_min=-1e300, v_max=1e300, a_max=1e300, a_dmax=1e300, steer_dmax=1e300, tol=1e300)):
+        if has_gpu:
+            capi.Solver(8, **kw).close()
+            continue
+        with pytest.raises(capi.MpcB200Error) as e:
+            capi.Solver(8, **kw)
+        assert e.value.code == -2, str(e.value)
+
+
 def test_no_cpu_fallback():
     """Without a CUDA device the product must fail loudly, not fall back."""
     try:
