@@ -1311,7 +1311,8 @@ static int rollout_enqueue(mpcb200_handle* h, const RolloutCall& c, int64_t lo, 
     int rc;
     if (!c.model && (rc = ensure_seed(h))) return rc;
     if (c.model && h->fit_window != c.window) {   /* grids of nav_msgs_path_frenet.py:63,79: arange(0, window, 0.5) and arange(0, window, 0.25) */
-        const int n1 = (int)ceil(c.window / 0.5 - 1e-9), n2 = (int)ceil(c.window / 0.25 - 1e-9);
+        int n1, n2;
+        fit_grid_sizes(c.window, &n1, &n2);
         double* P = (double*)malloc(sizeof(double) * 4 * ((size_t)n1 + n2));
         if (!P) return fail(h, MPCB200_ENOMEM, "%s: out of host memory", c.who);
         cubic_fit_matrix(n1, 0.5, P); cubic_fit_matrix(n2, 0.25, P + 4 * (size_t)n1);

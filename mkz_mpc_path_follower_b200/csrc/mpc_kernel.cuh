@@ -2288,6 +2288,13 @@ struct FrenetRolloutArgs {
 };
 
 // host side: the fit matrices of FrenetRolloutArgs
+// Sizes of the two fit grids, those of nav_msgs_path_frenet.py:63,79: np.arange(0, window, 0.5) and np.arange(0, window, 0.25)
+// have ceil(window / step) samples.  Dividing by 0.5 or 0.25 is exact, so no tolerance is needed (one would drop a sample of
+// a window just above a multiple of the step).
+inline void fit_grid_sizes(double window, int* n1, int* n2) {
+    *n1 = (int)ceil(window / 0.5);
+    *n2 = (int)ceil(window / 0.25);
+}
 // Least-squares cubic fit on the fixed grid x_g = g * step, g < n, as a 4 x n matrix P (coefficients, highest degree first,
 // = P * samples): P = (V'V)^-1 V' with the Vandermonde columns scaled to unit norm, normal equations in long double.
 inline void cubic_fit_matrix(int n, double step, double* P) {

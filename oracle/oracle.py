@@ -219,3 +219,50 @@ def closed_loop(cfg, path, pose0, T, track_using_time=True, target_vel=1.0, warm
     n = lib().mpc_oracle_closed_loop(C.byref(cfg), C.byref(path), _p(pose0), T, int(track_using_time),
                                      float(target_vel), int(warm_start), _p(log))
     return log[:n]
+
+
+def frenet_fit(xw, yw, window):
+    """The reference of the Frenet node from the path ahead, as nav_msgs_path_frenet.py:44-86 computes it: xw, yw sampled on
+    arange(0, window, 0.5) -> cubics X(s), Y(s) by np.polyfit (:65-70), their curvature on arange(0, window, 0.25) fitted by a
+    cubic (:44-58), psi_start = atan2(Y'(0), X'(0)) (:84).  Returns (K_coeffs[4] highest degree first, psi_start)."""
+    s_fit = np.arange(0.0, window, 0.5)
+    s_interp = np.arange(0.0, window, 0.25)
+    x_coeffs = np.polyfit(s_fit, xw, 3)
+    y_coeffs = np.polyfit(s_fit, yw, 3)
+    dx, dy = np.polyval(np.polyder(x_coeffs), s_interp), np.polyval(np.polyder(y_coeffs), s_interp)
+    ddx, ddy = np.polyval(np.polyder(x_coeffs, 2), s_interp), np.polyval(np.polyder(y_coeffs, 2), s_interp)
+    K = np.polyfit(s_interp, (dx * ddy - dy * ddx) / (dx * dx + dy * dy), 3)
+    psi_start = float(np.arctan2(np.polyval(np.polyder(y_coeffs), 0.0), np.polyval(np.polyder(x_coeffs), 0.0)))
+    return K, psi_start
+
+
+def closed_loop_frenet(cfg, traj_table, pose0, T, window, target_vel, ey_from_path=True):
+    """Closed loop on the Frenet-frame module (gazebo_sim_mpc_cmd_pub_frenet.jl:112-153) around the plant, one vehicle, with
+    nothing from the library: per control period the plant (plant_step) runs ten publishes, the path ahead is the next `window`
+    metres from the nearest sample (np.argmin, np.interp every 0.5 m, seen from the vehicle), frenet_fit gives K(s) and
+    psi_start, and solve_batch_frenet solves from (0, e_y, -psi_start, v) with the previous solution as its start (all zeros in
+    the first period) and cfg.max_iter as the cap.  e_y is the vehicle's offset from the fitted path start (ey_from_path) or 0.
+    traj_table: the (n,7) table of GPSRefTrajectory.trajectory.  Returns the (T, 8) log of the rollouts:
+    x, y, psi, v, acc_cmd, df_cmd, status, iters."""
+    N = cfg.N
+    Xp, Yp, sp = (np.ascontiguousarray(traj_table[:, i], dtype=np.float64) for i in (4, 5, 6))
+    s_fit = np.arange(0.0, window, 0.5)
+    st = np.array([pose0[0], pose0[1], pose0[2], 0.0, 0.0, 0.0, 0.0, 0.0])
+    acc_des = df_des = 0.0
+    u_prev = np.zeros((1, 2)); warm = np.zeros((1, 6 * N + 4)); log = np.zeros((T, 8))
+    for t in range(T):
+        for _ in range(10):
+            st = plant_step(st, acc_des, df_des)
+        i = int(np.argmin((Xp - st[0]) ** 2 + (Yp - st[1]) ** 2))
+        sq = sp[i] + s_fit
+        dx = np.interp(sq, sp, Xp) - st[0]; dy = np.interp(sq, sp, Yp) - st[1]
+        c, s = np.cos(st[2]), np.sin(st[2])
+        xw = c * dx + s * dy; yw = -s * dx + c * dy
+        K, psi_start = frenet_fit(xw, yw, window)
+        ey = -(-np.sin(psi_start) * xw[0] + np.cos(psi_start) * yw[0]) if ey_from_path else 0.0
+        state = np.array([[0.0, ey, -psi_start, st[3]]])
+        o = solve_batch_frenet(cfg, state, K[None], np.array([float(target_vel)]), u_prev, warm=warm)
+        acc_des, df_des = float(o["u0"][0, 0]), float(o["u0"][0, 1])
+        u_prev[0] = (df_des, acc_des)               # update_current_input(df_opt, a_opt) (:145)
+        log[t] = (st[0], st[1], st[2], st[3], acc_des, df_des, o["status"][0], o["iters"][0])
+    return log

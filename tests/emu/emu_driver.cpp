@@ -236,7 +236,8 @@ extern "C" int emu_rollout_frenet(const KCfg* cfg, long B, int T, const double* 
     std::vector<int> roles(32 * ROLE_STRIDE_F);
     for (int l = 0; l < 32; l++) riccati_roles(l, kc.N, w_sd_of(1, 1), roles.data() + l * ROLE_STRIDE_F, 1);
     kc.roles = roles.data();
-    const int n1 = (int)ceil(window / 0.5 - 1e-9), n2 = (int)ceil(window / 0.25 - 1e-9);
+    int n1, n2;
+    fit_grid_sizes(window, &n1, &n2);
     std::vector<double> P(4 * (size_t)(n1 + n2));
     cubic_fit_matrix(n1, 0.5, P.data()); cubic_fit_matrix(n2, 0.25, P.data() + 4 * (size_t)n1);
     FrenetRolloutArgs a;

@@ -294,38 +294,11 @@ def test_emulated_frenet_kernel_property(oracle):
     check()
 
 
-def _host_frenet_loop(oracle, cfg, traj_table, pose0, T, window, target_vel, ey_from_path=True):
-    """The control step of gazebo_sim_mpc_cmd_pub_frenet.jl:112-153 on the host, exactly as closed_loop.run_frenet runs
-    it, but with the ORACLE's Frenet solver in the place of the library (so that it runs without a GPU)."""
-    from mkz_mpc_path_follower_b200.vehicle_simulator import VehicleSimulator
-    N = cfg.N
-    sim = VehicleSimulator(X0=pose0[0], Y0=pose0[1], Psi0=pose0[2])
-    s_fit = np.arange(0.0, window, 0.5)
-    u_curr = np.zeros((1, 2)); warm = np.zeros((1, 6 * N + 4)); log = np.zeros((T, 8))
-    tr = traj_table
-    for t in range(T):
-        for _ in range(10):
-            sim.update_vehicle_model()
-        st = sim.state_est()[:4].copy()
-        i = int(np.argmin((tr[:, 4] - st[0]) ** 2 + (tr[:, 5] - st[1]) ** 2))
-        sq = tr[i, 6] + s_fit
-        dx = np.interp(sq, tr[:, 6], tr[:, 4]) - st[0]; dy = np.interp(sq, tr[:, 6], tr[:, 5]) - st[1]
-        c, s_ = np.cos(st[2]), np.sin(st[2])
-        xw = (c * dx + s_ * dy)[None]; yw = (-s_ * dx + c * dy)[None]
-        K, psi_start = frenet_ref.fit_windows(xw, yw, window)
-        ey = -(-np.sin(psi_start) * xw[:, 0] + np.cos(psi_start) * yw[:, 0]) if ey_from_path else np.zeros(1)
-        state = np.array([[0.0, ey[0], -psi_start[0], st[3]]])
-        o = oracle.solve_batch_frenet(cfg, state, K, np.array([float(target_vel)]), u_curr, warm=warm, n_threads=1)
-        sim.mpc_cmd(o["u0"][0, 0], o["u0"][0, 1])
-        u_curr[0] = (o["u0"][0, 1], o["u0"][0, 0])
-        log[t] = (st[0], st[1], st[2], st[3], o["u0"][0, 0], o["u0"][0, 1], o["status"][0], o["iters"][0])
-    return log
-
-
 def test_emulated_frenet_closed_loop(oracle):
     """rollout_group_frenet (mpcb200_rollout_frenet's kernel source) on the emulator: the path ahead, the two cubic
     least-squares fits of nav_msgs_path_frenet.py:44-86 as fixed matrices, state (0, e_y, -psi_start, v), warm-started
-    solve, command feedback -- against the same loop on the host (numpy fits, oracle solves)."""
+    solve, command feedback -- against oracle.closed_loop_frenet (np.polyfit fits, oracle solves, the oracle's plant).
+    test_frenet_closed_loop_emu.py runs it iterate for iterate at more horizons, windows and fleets."""
     import emu as E
     from mkz_mpc_path_follower_b200.gps_ref_traj import GPSRefTrajectory
     N, T, window, vt = 8, 6, 40.0, 8.0
@@ -336,7 +309,7 @@ def test_emulated_frenet_closed_loop(oracle):
     log, final = E.rollout_frenet(E.kcfg_from_oracle(cfg), g.trajectory, poses, T, window=window, target_vel=vt)
     assert E.race_count() == 0
     for b in range(poses.shape[0]):
-        h = _host_frenet_loop(oracle, cfg, g.trajectory, poses[b], T, window, vt)
+        h = oracle.closed_loop_frenet(cfg, g.trajectory, poses[b], T, window, vt)
         assert np.array_equal(log[:, b, 6], h[:, 6]) and (log[:, b, 6] == 0).all(), b
         assert np.abs(log[:, b, 7] - h[:, 7]).max() <= 1, b
         assert np.abs(log[:, b, 4:6] - h[:, 4:6]).max() <= 1e-6, (b, np.abs(log[:, b, 4:6] - h[:, 4:6]).max())

@@ -19,9 +19,9 @@ Which instantiation each row reaches (csrc/mpc_b200.cu: team_kernel, rollout_ker
                                    problems always take the packed small-batch path, which launches the team kernels)
 The team rows run B <= 64 host batches (the packed small-batch path and its CUDA graph); test_records_and_device_pointers runs
 the same kernels through the unpacked path, with mpcb200_solve_batch_records and with device pointers.  Not covered here:
-mpc_rollout_frenet_kernel and rollout_solve_tpp_kernel<1, 0> (the Frenet closed loop has no oracle counterpart; the host-loop
-test of test_gpu_parity.py checks it), and the reference generators of the on-path entry points, which launch the solve
-kernels above and are checked bit for bit against the host generator elsewhere.
+mpc_rollout_frenet_kernel and the Frenet per-period pipeline (rollout_frenet_ref_kernel, rollout_solve_tpp_kernel<1, 0>), which
+test_gpu_frenet_closed_loop.py checks iterate for iterate against oracle.closed_loop_frenet, and the reference generators of the
+on-path entry points, which launch the solve kernels above and are checked bit for bit against the host generator elsewhere.
 
 Bars: the GPU build contracts multiply-adds and uses its own sincos and reciprocal, so it does not round like the host build of
 the emulator (floor 1e-12).  The largest relative difference per row over k = 1, 2, 3, 5, 10 (k = 2, 5 for the constant sets;
