@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define MPCB200_VERSION 3
+#define MPCB200_VERSION 4
 
 /* error codes */
 #define MPCB200_OK          0
@@ -220,6 +220,33 @@ int mpcb200_rollout_w(mpcb200_handle* h, int64_t B, int32_t T, const double* pos
                       int32_t track_using_time, double target_vel, const double* w, double* log, double* final_state);
 
 /*
+ * Tracking metrics of a closed-loop rollout, accumulated on the device while it runs (the offline score of
+ * scripts/analysis/plot_path_tracking_error.py -- nearest-sample path error and heading error -- plus command smoothness, solver
+ * health and progress), so that scoring a large sweep needs neither the [T][B][8] log nor a host-side nearest-sample search.
+ * metrics [B][MPCB200_METRICS] is required; everything else -- validation, w ([B][8] rows as mpcb200_rollout_w, or NULL = the
+ * handle's weights), host pointers, the fused / per-period switch, multi-GPU slicing, log and final_state (either may be NULL) --
+ * is that of mpcb200_rollout / mpcb200_rollout_w, and log and final_state come out bit-identical to theirs.
+ *
+ * A period COUNTS when a solve ran in it (log status >= 0): every period before the stop latch (the period in which stop_cmd
+ * latches does not count).  For the pose (x, y, psi) logged for that period and its nearest path sample i (the one get_waypoints
+ * uses): e = sqrt((X_i - x)^2 + (Y_i - y)^2), h = mod(psi - psi_i + pi, 2 pi) - pi, and the command rates
+ * da = acc_cmd - acc_cmd_prev, dd = df_cmd - df_cmd_prev, "prev" being the previous counting period's command (0 for the first).
+ * Per vehicle, in this order (n = field 0; with n = 0 fields 1..9 are 0):
+ *    0 n_solved         counting periods             6 acc_rate_rms    sqrt(sum da^2 / n)
+ *    1 path_err_mean    sum e / n                    7 steer_rate_rms  sqrt(sum dd^2 / n)
+ *    2 path_err_rms     sqrt(sum e^2 / n)            8 n_not_optimal   counting periods with status != MPCB200_OPTIMAL
+ *    3 path_err_max     max e                        9 iters_total     sum of iterations
+ *    4 heading_err_rms  sqrt(sum h^2 / n)           10 s_last          arc length s_i of the last counting period (NaN if n = 0)
+ *    5 heading_err_max  max |h|                     11 stop_period     first period with status -1 (stop latch), -1 if none
+ * Every operation is rounded as numpy rounds it and the sums run in period order: closed_loop.tracking_metrics restates this on
+ * the host from a log.  metrics == NULL is MPCB200_EINVAL; with B == 0 or T == 0 nothing is written.
+ */
+#define MPCB200_METRICS 12   /* doubles per vehicle */
+int mpcb200_rollout_metrics(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of,
+                            int32_t track_using_time, double target_vel, const double* w,
+                            double* log, double* final_state, double* metrics);
+
+/*
  * Frenet-frame variant of the same solver: scripts/mpc_utils/MKZMPCPathFollowerFrenet.jl (the model the Gazebo
  * lane-keep node gazebo_sim_mpc_cmd_pub_frenet.jl:112-153 drives).  Same vehicle constants, horizon, bounds, rate
  * rows and interior-point iteration; states (s, e_y, e_psi, v) with ds/dt = v cos(e_psi + beta) / (1 - e_y K(s)),
@@ -257,6 +284,11 @@ int mpcb200_solve_batch_frenet_w(mpcb200_handle* h, int64_t B, const double* sta
  */
 int mpcb200_rollout_frenet(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of,
                            double window, double target_vel, int32_t ey_from_path, double* log, double* final_state);
+/* mpcb200_rollout_frenet with the tracking metrics of mpcb200_rollout_metrics (every period counts; stop_period is always -1).
+ * Per-vehicle weights are not available for Frenet rollouts: mpcb200_rollout_metrics refuses a Frenet handle (MPCB200_EINVAL). */
+int mpcb200_rollout_frenet_metrics(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of,
+                                   double window, double target_vel, int32_t ey_from_path,
+                                   double* log, double* final_state, double* metrics);
 
 /* Counters of the last solve_batch/rollout call on this handle. */
 typedef struct {

@@ -15,6 +15,9 @@ OPTIMAL, INFEASIBLE, UNBOUNDED, USERLIMIT, ERROR = 0, 1, 2, 3, 4
 STATUS_SYMBOLS = {0: "Optimal", 1: "Infeasible", 2: "Unbounded", 3: "UserLimit", 4: "Error"}
 HOST, DEVICE = 0, 1
 START_ZERO, START_ROLLOUT = 0, 1
+# the per-vehicle fields of rollout(..., metrics=True) (MPCB200_METRICS, include/mpc_b200.h), in column order
+ROLLOUT_METRICS = ("n_solved", "path_err_mean", "path_err_rms", "path_err_max", "heading_err_rms", "heading_err_max",
+                   "acc_rate_rms", "steer_rate_rms", "n_not_optimal", "iters_total", "s_last", "stop_period")
 
 
 class Config(C.Structure):
@@ -68,6 +71,8 @@ def lib():
     L.mpcb200_rollout.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_int32, C.c_double, dp, dp]
     L.mpcb200_rollout_w.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_int32, C.c_double, dp, dp, dp]
     L.mpcb200_rollout_frenet.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_double, C.c_double, C.c_int32, dp, dp]
+    L.mpcb200_rollout_metrics.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_int32, C.c_double, dp, dp, dp, dp]
+    L.mpcb200_rollout_frenet_metrics.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_double, C.c_double, C.c_int32, dp, dp, dp]
     L.mpcb200_get_stats.argtypes = [vp, C.POINTER(Stats)]
     L.mpcb200_fp64_peak.argtypes = [vp, dp]
     L.mpcb200_last_error.argtypes = [vp]
@@ -275,10 +280,12 @@ class Solver(object):
         dp = C.POINTER(C.c_double)
         self._check(lib().mpcb200_set_path(self._h, int(path_id), int(traj_table.shape[0]), *[c.ctypes.data_as(dp) for c in cols]))
 
-    def rollout(self, pose0, path_of, T, track_using_time=True, target_vel=1.0, want_log=True, weights=None):
+    def rollout(self, pose0, path_of, T, track_using_time=True, target_vel=1.0, want_log=True, weights=None, metrics=False):
         """Closed-loop Monte-Carlo rollout on the device (mpcb200_rollout).  pose0 (B,3); path_of (B,) in 0..2
         (ids given to set_path).  Returns log (T,B,8) = x,y,psi,v,acc_cmd,df_cmd,status,iters and final (B,8).
-        weights (B,8): each vehicle's cost weights for all its control periods (mpcb200_rollout_w), or None: the handle's."""
+        weights (B,8): each vehicle's cost weights for all its control periods (mpcb200_rollout_w), or None: the handle's.
+        metrics: also the per-vehicle tracking metrics accumulated on the device (mpcb200_rollout_metrics), out["metrics"] (B,12)
+        with the columns of ROLLOUT_METRICS; with want_log=False no log is transferred at all."""
         pose0 = np.ascontiguousarray(np.atleast_2d(pose0), dtype=np.float64)
         B = pose0.shape[0]
         path_of = np.ascontiguousarray(path_of, dtype=np.int32)
@@ -289,10 +296,15 @@ class Solver(object):
         dp = C.POINTER(C.c_double)
         args = [pose0.ctypes.data_as(dp), path_of.ctypes.data_as(C.POINTER(C.c_int32)), int(bool(track_using_time)), float(target_vel)]
         outs = [None if log is None else log.ctypes.data_as(dp), final.ctypes.data_as(dp)]
-        if weights is None:
+        w = None if weights is None else _weight_rows(weights, B, 8, "rollout")
+        if metrics:
+            met = np.empty((B, len(ROLLOUT_METRICS)))
+            self._check(lib().mpcb200_rollout_metrics(self._h, B, int(T), *args, None if w is None else w.ctypes.data_as(dp), *outs,
+                                                      met.ctypes.data_as(dp)))
+            return {"log": log, "final_state": final, "metrics": met}
+        if w is None:
             self._check(lib().mpcb200_rollout(self._h, B, int(T), *args, *outs))
         else:
-            w = _weight_rows(weights, B, 8, "rollout")
             self._check(lib().mpcb200_rollout_w(self._h, B, int(T), *args, w.ctypes.data_as(dp), *outs))
         return {"log": log, "final_state": final}
 
@@ -357,9 +369,10 @@ class FrenetSolver(Solver):
                                                            _ptr(w), _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), HOST))
         return {"u0": u0, "cost": cost, "status": status, "iters": iters, "traj": traj}
 
-    def rollout(self, pose0, path_of, T, window=40.0, target_vel=8.0, ey_from_path=True, want_log=True):
+    def rollout(self, pose0, path_of, T, window=40.0, target_vel=8.0, ey_from_path=True, want_log=True, metrics=False):
         """Closed loop on the Frenet-frame module on the device (mpcb200_rollout_frenet; what closed_loop.run_frenet does on the
-        host).  pose0 (B,3); path_of (B,) ids given to set_path.  Returns log (T,B,8) and final (B,8) like Solver.rollout."""
+        host).  pose0 (B,3); path_of (B,) ids given to set_path.  Returns log (T,B,8) and final (B,8) like Solver.rollout;
+        metrics: also out["metrics"] (B,12) as Solver.rollout (mpcb200_rollout_frenet_metrics)."""
         pose0 = np.ascontiguousarray(np.atleast_2d(pose0), dtype=np.float64)
         B = pose0.shape[0]
         path_of = np.ascontiguousarray(path_of, dtype=np.int32)
@@ -368,9 +381,13 @@ class FrenetSolver(Solver):
         log = np.empty((T, B, 8)) if want_log else None
         final = np.empty((B, 8))
         dp = C.POINTER(C.c_double)
-        self._check(lib().mpcb200_rollout_frenet(self._h, B, int(T), pose0.ctypes.data_as(dp), path_of.ctypes.data_as(C.POINTER(C.c_int32)),
-                                                 float(window), float(target_vel), int(bool(ey_from_path)),
-                                                 None if log is None else log.ctypes.data_as(dp), final.ctypes.data_as(dp)))
+        args = [pose0.ctypes.data_as(dp), path_of.ctypes.data_as(C.POINTER(C.c_int32)), float(window), float(target_vel),
+                int(bool(ey_from_path)), None if log is None else log.ctypes.data_as(dp), final.ctypes.data_as(dp)]
+        if metrics:
+            met = np.empty((B, len(ROLLOUT_METRICS)))
+            self._check(lib().mpcb200_rollout_frenet_metrics(self._h, B, int(T), *args, met.ctypes.data_as(dp)))
+            return {"log": log, "final_state": final, "metrics": met}
+        self._check(lib().mpcb200_rollout_frenet(self._h, B, int(T), *args))
         return {"log": log, "final_state": final}
 
     def solve_batch_device(self, B, state, k_coeffs, u_prev, u0, v_des=None, warm=None, cost=None, status=None, iters=None, traj=None,

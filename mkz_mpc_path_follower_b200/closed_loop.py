@@ -81,16 +81,76 @@ def module_load_solution(N, device=0):
     return _seed_cache[N]
 
 
+def _nearest_samples(traj_table, xy):
+    """Nearest path sample of each pose xy (M,2) over the whole path (np.argmin, first index on ties, as ref_gps_traj.py:136-137
+    and TeamSolver::nearest_sample): (index (M,), squared distance (M,))."""
+    XY = traj_table[:, 4:6]
+    d = (XY[None, :, 0] - xy[:, 0:1]) ** 2 + (XY[None, :, 1] - xy[:, 1:2]) ** 2
+    i = d.argmin(axis=1)
+    return i, d[np.arange(d.shape[0]), i]
+
+
 def path_errors(log, traj_table):
     """Tracking-quality metric of scripts/analysis/plot_path_tracking_error.py:21-34: distance to the
     nearest path sample for every logged pose.  log (T,B,8) -> (T,B)."""
-    XY = traj_table[:, 4:6]
     T, B = log.shape[0], log.shape[1]
     err = np.empty((T, B))
     for t in range(T):
-        d = (XY[None, :, 0] - log[t, :, 0:1]) ** 2 + (XY[None, :, 1] - log[t, :, 1:2]) ** 2
-        err[t] = np.sqrt(d.min(axis=1))
+        err[t] = np.sqrt(_nearest_samples(traj_table, log[t, :, 0:2])[1])
     return err
+
+
+def tracking_metrics(log, traj_table):
+    """Per-vehicle tracking metrics of a closed-loop log (T,B,8) on one path (the (n,7) table of GPSRefTrajectory.trajectory):
+    (B,12) in the order of capi.ROLLOUT_METRICS, as mpcb200_rollout_metrics / _frenet_metrics accumulate them on the device
+    (include/mpc_b200.h).  A period counts when a solve ran in it (status >= 0); e is the distance to the nearest path sample i of
+    the logged pose, h = mod(psi - psi_i + pi, 2 pi) - pi, the command rates are against the previous counting period's commands
+    (0 before the first).  The sums run in period order, so the device's results are reproduced to the last bit."""
+    T, B = log.shape[0], log.shape[1]
+    psi_p, s_p = traj_table[:, 3], traj_table[:, 6]
+    n, se, se2, emax, sh2, hmax, sda2, sdd2, nno, it, pa, pd = (np.zeros(B) for _ in range(12))
+    s_last = np.full(B, np.nan)
+    stop = np.full(B, -1.0)
+    for t in range(T):
+        status = log[t, :, 6]
+        stop[(status < 0) & (stop < 0)] = t
+        c = status >= 0
+        if not c.any():
+            continue
+        i, d = _nearest_samples(traj_table, log[t, c, 0:2])
+        e = np.sqrt(d)
+        h = np.mod(log[t, c, 2] - psi_p[i] + np.pi, 2.0 * np.pi) - np.pi
+        acc, dfc = log[t, c, 4], log[t, c, 5]
+        da, dd = acc - pa[c], dfc - pd[c]
+        n[c] += 1.0
+        se[c] += e
+        se2[c] += e * e
+        emax[c] = np.maximum(emax[c], e)
+        sh2[c] += h * h
+        hmax[c] = np.maximum(hmax[c], np.abs(h))
+        sda2[c] += da * da
+        sdd2[c] += dd * dd
+        nno[c] += status[c] != 0
+        it[c] += log[t, c, 7]
+        s_last[c] = s_p[i]
+        pa[c] = acc
+        pd[c] = dfc
+    out = np.zeros((B, 12))
+    m = n > 0
+    nm = n[m]
+    out[:, 0] = n
+    out[m, 1] = se[m] / nm
+    out[m, 2] = np.sqrt(se2[m] / nm)
+    out[m, 3] = emax[m]
+    out[m, 4] = np.sqrt(sh2[m] / nm)
+    out[m, 5] = hmax[m]
+    out[m, 6] = np.sqrt(sda2[m] / nm)
+    out[m, 7] = np.sqrt(sdd2[m] / nm)
+    out[m, 8] = nno[m]
+    out[m, 9] = it[m]
+    out[:, 10] = s_last
+    out[:, 11] = stop
+    return out
 
 
 def run_frenet(path_ids, pose0, T, N=8, window=40.0, target_vel=8.0, solver=None, ey_from_path=True):

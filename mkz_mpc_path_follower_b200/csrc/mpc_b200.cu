@@ -21,6 +21,7 @@
 #include <utility>
 
 using namespace mpcb200;
+static_assert(MET_FIELDS == MPCB200_METRICS, "rollout metrics: kernel and C ABI row sizes differ");
 
 namespace {
 
@@ -273,11 +274,37 @@ __global__ void rollout_final_kernel(const long long B, const long long Bp, cons
     for (int i = 0; i < 8; i++) final_state[8 * v + i] = veh[i * Bp + v];
 }
 
+// Tracking metrics of the per-period pipeline (mpcb200_rollout_metrics / _frenet_metrics), launched after the solve of period t:
+// warp = vehicle, metrics_period on the pose in veh (which the solve does not move), the published command veh[8..9], and the
+// solve's status and iterations unless the stop latch (XY: stop[v]; Frenet: stop = null) kept the vehicle from solving.  The
+// waypoint and reference kernels stay as they are, so the nearest sample is searched a second time here.
+__global__ void __launch_bounds__(128)
+rollout_metrics_kernel(const KCfg cfg, const RolloutArgs a, const long long Bp, const double* veh, const int* stop, const int* status,
+                       const int* iters, const int t) {
+    const long long warps = ((long long)gridDim.x * blockDim.x) >> 5;
+    TeamSolver<1> S(cfg, (smem_t)0);   // (one-warp teams use no shared memory in nearest_sample)
+    for (long long v = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; v < a.B; v += warps) {
+        const bool solved = !stop || !stop[v];
+        metrics_period(S, a.met + v, Bp, t, a.paths[a.path_of[v]], veh[v], veh[Bp + v], veh[2 * Bp + v], veh[8 * Bp + v], veh[9 * Bp + v],
+                       solved ? status[v] : -1, solved ? iters[v] : 0);
+        __syncwarp();
+    }
+}
+
+// [B][MET_FIELDS] rows from the [MET_K][stride] accumulators (both the fused kernels and the pipeline)
+__global__ void rollout_metrics_final_kernel(const long long B, const long long stride, const double* met, double* out) {
+    const long long v = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (v >= B) return;
+    metrics_finalize(met + v, (long)stride, out + (long long)MET_FIELDS * v);
+}
+
 #ifndef MPC_ROLLOUT_MIN_BLOCKS
 #define MPC_ROLLOUT_MIN_BLOCKS 3
 #endif
 // PW (this kernel and mpc_rollout_long_kernel): each vehicle's cost weights from args.w (mpcb200_rollout_w)
-template <int PW>
+// MET (these two and mpc_rollout_frenet_kernel): 1 = tracking metrics into args.met (mpcb200_rollout_metrics); a compile-time switch
+// like PW, so that the MET = 0 instantiations are the code they always were
+template <int PW, int MET = 0>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, MPC_ROLLOUT_MIN_BLOCKS)
 mpc_rollout_kernel(const KCfg cfg, const RolloutArgs args, unsigned long long* counter) {
     extern __shared__ double smem_all[];
@@ -292,12 +319,12 @@ mpc_rollout_kernel(const KCfg cfg, const RolloutArgs args, unsigned long long* c
         const unsigned long long b0 = next_group;
         __syncthreads();
         if (b0 >= (unsigned long long)args.B) break;
-        rollout_group<1, PW>(cfg, args, (long)b0, smem, px, WARPS_PER_BLOCK);
+        rollout_group<1, PW, MET>(cfg, args, (long)b0, smem, px, WARPS_PER_BLOCK);
     }
 }
 
 // Closed-loop rollouts at long horizons (32 <= N <= 95): one vehicle per block of W = 2 or 3 warps
-template <int W, int PW = 0>
+template <int W, int PW = 0, int MET = 0>
 __global__ void __launch_bounds__(W * 32, W == 2 ? 4 : 2)
 mpc_rollout_long_kernel(const KCfg cfg, const RolloutArgs args, unsigned long long* counter) {
     extern __shared__ double smem_all[];
@@ -311,13 +338,15 @@ mpc_rollout_long_kernel(const KCfg cfg, const RolloutArgs args, unsigned long lo
         const unsigned long long b0 = next_vehicle;
         __syncthreads();
         if (b0 >= (unsigned long long)args.B) break;
-        rollout_group<W, PW>(cfg, args, (long)b0, smem, px, 1);
+        rollout_group<W, PW, MET>(cfg, args, (long)b0, smem, px, 1);
     }
 }
 
 // Closed loop on the Frenet-frame module (gazebo_sim_mpc_cmd_pub_frenet.jl:112-153): four vehicles per block
+// met: [MET_K][B] accumulators of MET = 1 (rollout_group_frenet)
+template <int MET = 0>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 2)
-mpc_rollout_frenet_kernel(const KCfg cfg, const FrenetRolloutArgs args, unsigned long long* counter) {
+mpc_rollout_frenet_kernel(const KCfg cfg, const FrenetRolloutArgs args, unsigned long long* counter, double* met) {
     extern __shared__ double smem_all[];
     const int warp = threadIdx.x >> 5;
     const smem_t smem = smem_base(smem_all + (size_t)warp * smem_doubles_per_team(cfg.N, 1));
@@ -330,7 +359,7 @@ mpc_rollout_frenet_kernel(const KCfg cfg, const FrenetRolloutArgs args, unsigned
         const unsigned long long b0 = next_group;
         __syncthreads();
         if (b0 >= (unsigned long long)args.B) break;
-        rollout_group_frenet(cfg, args, (long)b0, smem, px, WARPS_PER_BLOCK);
+        rollout_group_frenet<MET>(cfg, args, (long)b0, smem, px, WARPS_PER_BLOCK, met);
     }
 }
 
@@ -373,6 +402,7 @@ struct mpcb200_handle {
     DevBuf d_genref;                  /* ... on a path: the generated waypoints [B][3][N+1] when the caller did not ask for them */
     DevBuf d_veh, d_vstop;            /* ... closed-loop fleets: vehicle state [12][Bp], stop latches */
     DevBuf d_w;                       /* per-problem weight rows of a weighted call (host pointers) */
+    DevBuf d_met, d_metout;           /* rollout tracking metrics: accumulators [MET_K][stride], rows [B][MET_FIELDS] */
     int blocks_per_sm_w = 0;          /* resident blocks per SM of the PW = 1 solve kernel of this handle (8 more doubles per team) */
     int rollout_blocks_per_sm_w = 0;  /* ... of the PW = 1 fused rollout kernel */
     int tpp_blocks_per_sm = 0;        /* resident blocks of mpc_solve_tpp_kernel per SM */
@@ -489,10 +519,10 @@ static TeamKernel team_kernel(const mpcb200_handle* h, int* threads) {
 
 /* the fused closed-loop kernel of an XY handle */
 typedef void (*RolloutKernel)(const KCfg, const RolloutArgs, unsigned long long*);
-template <int PW>
+template <int PW, int MET = 0>
 static RolloutKernel rollout_kernel(const mpcb200_handle* h) {
-    if (h->team_warps == 1) return mpc_rollout_kernel<PW>;
-    return (h->team_warps == 2) ? mpc_rollout_long_kernel<2, PW> : mpc_rollout_long_kernel<3, PW>;
+    if (h->team_warps == 1) return mpc_rollout_kernel<PW, MET>;
+    return (h->team_warps == 2) ? mpc_rollout_long_kernel<2, PW, MET> : mpc_rollout_long_kernel<3, PW, MET>;
 }
 
 /* dynamic shared memory of the fused rollout kernel: the teams and the plant exchange area (the XY handle's smem_bytes already
@@ -659,7 +689,7 @@ static int create_impl(mpcb200_handle** out, const mpcb200_config* cfg, int mode
         if (const char* e = getenv("MPCB200_FRENET_WPB")) { int v = atoi(e); if (v == 3 || v == 4) h->frenet_wpb = v; }  /* tuning aid */
         h->blocks_per_sm = (h->frenet_wpb == 3) ? b3 : b4;
         h->smem_bytes = h->frenet_wpb * team;
-        TRY_OR_FREE(prepare_kernel((const void*)mpc_rollout_frenet_kernel, h->device, WARPS_PER_BLOCK * 32, rollout_smem_bytes(h, false),
+        TRY_OR_FREE(prepare_kernel((const void*)mpc_rollout_frenet_kernel<0>, h->device, WARPS_PER_BLOCK * 32, rollout_smem_bytes(h, false),
                                    &h->frenet_rollout_blocks_per_sm));
     } else {
         /* one-warp XY teams: four per block, with the plant exchange area of the fused rollout kernel */
@@ -1302,6 +1332,7 @@ struct RolloutCall {
     int32_t track_using_time; const double* w;   /* XY: waypoints by time or arc length; [B][8] weight rows or null */
     double window; int32_t ey_from_path;          /* Frenet: length of the path ahead, e_y from the path or from the fit */
     double* log; double* final_state;             /* [T][B][8], [B][8] or null */
+    double* metrics;                              /* [B][MET_FIELDS] or null (the plain entry points) */
 };
 
 /* one device's share of a rollout: vehicles [lo, lo + n) of B; enqueue ... */
@@ -1330,6 +1361,9 @@ static int rollout_enqueue(mpcb200_handle* h, const RolloutCall& c, int64_t lo, 
     if ((rc = ensure(h, h->d_pathof, (size_t)n * sizeof(int32_t)))) return rc;
     if (c.log && (rc = ensure(h, h->d_log, (size_t)c.T * n * 8 * sizeof(double)))) return rc;
     if (c.final_state && (rc = ensure(h, h->d_final, (size_t)n * 8 * sizeof(double)))) return rc;
+    const long long Bp = (n + 31) / 32 * 32;   /* stride of the per-period pipeline's structure-of-arrays buffers */
+    if (c.metrics && ((rc = ensure(h, h->d_met, (size_t)MET_K * Bp * sizeof(double))) ||
+                      (rc = ensure(h, h->d_metout, (size_t)n * MET_FIELDS * sizeof(double))))) return rc;
     CUDA_TRY(h, cudaMemcpyAsync(h->d_pose.p, c.pose0 + 3 * lo, (size_t)n * 3 * sizeof(double), cudaMemcpyHostToDevice, s));
     CUDA_TRY(h, cudaMemcpyAsync(h->d_pathof.p, c.path_of + lo, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     h->stats.h2d_bytes += (size_t)n * (3 * sizeof(double) + sizeof(int32_t));
@@ -1350,6 +1384,7 @@ static int rollout_enqueue(mpcb200_handle* h, const RolloutCall& c, int64_t lo, 
     a.track_using_time = c.track_using_time; a.warm0 = (const double*)h->d_seed.p; a.w = c.w ? (const double*)h->d_w.p : nullptr;
     fa.ey_from_path = c.ey_from_path;
     fa.P1 = (const double*)h->d_fit.p; fa.P2 = fa.P1 + 4 * (size_t)h->fit_n1; fa.n1 = h->fit_n1; fa.n2 = h->fit_n2;
+    a.met = c.metrics ? (double*)h->d_met.p : nullptr;
     const KCfg kc = make_kcfg(h);
     /* large fleets at short horizons: one control period = plant / reference / thread-per-problem solve over the whole fleet.
      * Measured for the XY model at N = 8, 200 periods (profiles/r02_logs/r02_rollout_thresholds.log): a period of the pipeline takes
@@ -1357,7 +1392,6 @@ static int rollout_enqueue(mpcb200_handle* h, const RolloutCall& c, int64_t lo, 
      * 0.5 / 0.8 / 1.4 / 2.5 ms at 2,048 / 4,096 / 8,192 / 16,384 vehicles: the default rule switches at a quarter of the cold-start batch */
     const int64_t roll_from = h->tpp_default_rule ? h->tpp_min_batch / 4 : h->tpp_min_batch;
     if (h->tpp_min_batch > 0 && n >= roll_from) {
-        const long long Bp = (n + 31) / 32 * 32;
         /* blocks of 128 vehicles (two resident per SM): every vehicle solves at once and a block keeps its vehicles, so smaller
          * blocks mean less idle SMs in the last wave (16,384 vehicles: 0.89 instead of 1.07 ms per period; never slower) */
         const int tb = h->tpp_block < 128 ? h->tpp_block : 128;
@@ -1397,28 +1431,36 @@ static int rollout_enqueue(mpcb200_handle* h, const RolloutCall& c, int64_t lo, 
             else rollout_waypoints_kernel<<<wgrid, 128, 0, s>>>(kc, (long long)n, Bp, veh, a.path_of, rg, st, filt, stop, t == 0);
             sk<<<(int)sblocks, tb, 0, s>>>(kc, (long long)n, Bp, veh, stop, st, filt, (!c.model && t == 0) ? a.warm0 : nullptr, des_speed, out,
                                            a.log ? a.log + (size_t)t * n * 8 : nullptr, fref, t == 0);
+            if (a.met) rollout_metrics_kernel<<<wgrid, 128, 0, s>>>(kc, a, Bp, veh, stop, out.status, out.iters, t);
             CUDA_TRY(h, cudaGetLastError());
         }
         if (a.final_state) rollout_final_kernel<<<pgrid, 128, 0, s>>>((long long)n, Bp, veh, a.final_state);
+        if (a.met) rollout_metrics_final_kernel<<<pgrid, 128, 0, s>>>((long long)n, Bp, a.met, (double*)h->d_metout.p);
         CUDA_TRY(h, cudaGetLastError());
         CUDA_TRY(h, cudaEventRecord(h->ev1, s));
-        h->stats.kernel_launches += 3 * (int64_t)c.T + (a.final_state ? 1 : 0);
+        h->stats.kernel_launches += (a.met ? 4 : 3) * (int64_t)c.T + (a.final_state ? 1 : 0) + (a.met ? 1 : 0);
         return MPCB200_OK;
     }
     CUDA_TRY(h, cudaMemsetAsync(h->d_counter, 0, sizeof(unsigned long long), s));
     const int per_block = (h->team_warps == 1) ? WARPS_PER_BLOCK : 1;
     long long blocks_needed = (n + per_block - 1) / per_block;
-    const int bps = c.model ? h->frenet_rollout_blocks_per_sm : (c.w ? h->rollout_blocks_per_sm_w : h->rollout_blocks_per_sm);
-    long long max_blocks = (long long)h->num_sms * bps;
-    const int grid = (int)(blocks_needed < max_blocks ? blocks_needed : max_blocks);
+    int bps = c.model ? h->frenet_rollout_blocks_per_sm : (c.w ? h->rollout_blocks_per_sm_w : h->rollout_blocks_per_sm);
     const int threads = 32 * (h->team_warps == 1 ? WARPS_PER_BLOCK : h->team_warps);
     const size_t smem = rollout_smem_bytes(h, c.w != nullptr);
+    /* the MET = 1 instantiations: shared-memory limit and residency prepared here, by the calls that launch them */
+    const void* met_fn = !c.metrics ? nullptr : c.model ? (const void*)mpc_rollout_frenet_kernel<1>
+                                                         : (const void*)(c.w ? rollout_kernel<1, 1>(h) : rollout_kernel<0, 1>(h));
+    if (met_fn) CUDA_TRY(h, prepare_kernel(met_fn, h->device, threads, smem, &bps));
+    long long max_blocks = (long long)h->num_sms * bps;
+    const int grid = (int)(blocks_needed < max_blocks ? blocks_needed : max_blocks);
     CUDA_TRY(h, cudaEventRecord(h->ev0, s));
-    if (c.model) mpc_rollout_frenet_kernel<<<grid, threads, smem, s>>>(kc, fa, h->d_counter);
+    if (c.model) (c.metrics ? mpc_rollout_frenet_kernel<1> : mpc_rollout_frenet_kernel<0>)<<<grid, threads, smem, s>>>(kc, fa, h->d_counter, a.met);
+    else if (c.metrics) (c.w ? rollout_kernel<1, 1>(h) : rollout_kernel<0, 1>(h))<<<grid, threads, smem, s>>>(kc, a, h->d_counter);
     else (c.w ? rollout_kernel<1>(h) : rollout_kernel<0>(h))<<<grid, threads, smem, s>>>(kc, a, h->d_counter);
+    if (c.metrics) rollout_metrics_final_kernel<<<(int)((n + 127) / 128), 128, 0, s>>>((long long)n, (long long)n, a.met, (double*)h->d_metout.p);
     CUDA_TRY(h, cudaGetLastError());
     CUDA_TRY(h, cudaEventRecord(h->ev1, s));
-    h->stats.kernel_launches += 1;
+    h->stats.kernel_launches += c.metrics ? 2 : 1;
     return MPCB200_OK;
 }
 
@@ -1432,6 +1474,11 @@ static int rollout_collect(mpcb200_handle* h, const RolloutCall& c, int64_t lo, 
         h->stats.d2h_bytes += row * c.T;
     }
     if (c.final_state) { CUDA_TRY(h, cudaMemcpyAsync(c.final_state + (size_t)lo * 8, h->d_final.p, row, cudaMemcpyDeviceToHost, s)); h->stats.d2h_bytes += row; }
+    if (c.metrics) {
+        const size_t mrow = (size_t)n * MET_FIELDS * sizeof(double);
+        CUDA_TRY(h, cudaMemcpyAsync(c.metrics + (size_t)lo * MET_FIELDS, h->d_metout.p, mrow, cudaMemcpyDeviceToHost, s));
+        h->stats.d2h_bytes += mrow;
+    }
     CUDA_TRY(h, cudaStreamSynchronize(s));
     float ms = 0.f;
     CUDA_TRY(h, cudaEventElapsedTime(&ms, h->ev0, h->ev1));
@@ -1439,7 +1486,7 @@ static int rollout_collect(mpcb200_handle* h, const RolloutCall& c, int64_t lo, 
     return MPCB200_OK;
 }
 
-/* the body of mpcb200_rollout, mpcb200_rollout_w (w == NULL: the handle's weights) and mpcb200_rollout_frenet */
+/* the body of mpcb200_rollout, mpcb200_rollout_w (w == NULL: the handle's weights), mpcb200_rollout_frenet and their _metrics forms */
 static int rollout_impl(mpcb200_handle* h, const RolloutCall& c) {
     const char* who = c.who;
     if (!h) return MPCB200_EINVAL;
@@ -1470,18 +1517,33 @@ static int rollout_impl(mpcb200_handle* h, const RolloutCall& c) {
 
 int mpcb200_rollout(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, int32_t track_using_time,
                     double target_vel, double* log, double* final_state) {
-    return rollout_impl(h, {"mpcb200_rollout", 0, B, T, pose0, path_of, target_vel, track_using_time, nullptr, 0.0, 0, log, final_state});
+    return rollout_impl(h, {"mpcb200_rollout", 0, B, T, pose0, path_of, target_vel, track_using_time, nullptr, 0.0, 0, log, final_state, nullptr});
 }
 
 int mpcb200_rollout_w(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, int32_t track_using_time,
                       double target_vel, const double* w, double* log, double* final_state) {
     if (h && !w && B > 0 && T > 0) return fail(h, MPCB200_EINVAL, "mpcb200_rollout_w: w is required");
-    return rollout_impl(h, {"mpcb200_rollout_w", 0, B, T, pose0, path_of, target_vel, track_using_time, w, 0.0, 0, log, final_state});
+    return rollout_impl(h, {"mpcb200_rollout_w", 0, B, T, pose0, path_of, target_vel, track_using_time, w, 0.0, 0, log, final_state, nullptr});
 }
 
 int mpcb200_rollout_frenet(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, double window,
                            double target_vel, int32_t ey_from_path, double* log, double* final_state) {
-    return rollout_impl(h, {"mpcb200_rollout_frenet", 1, B, T, pose0, path_of, target_vel, 0, nullptr, window, ey_from_path, log, final_state});
+    return rollout_impl(h, {"mpcb200_rollout_frenet", 1, B, T, pose0, path_of, target_vel, 0, nullptr, window, ey_from_path, log, final_state,
+                            nullptr});
+}
+
+int mpcb200_rollout_metrics(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, int32_t track_using_time,
+                            double target_vel, const double* w, double* log, double* final_state, double* metrics) {
+    if (h && !metrics) return fail(h, MPCB200_EINVAL, "mpcb200_rollout_metrics: metrics is required");
+    return rollout_impl(h, {"mpcb200_rollout_metrics", 0, B, T, pose0, path_of, target_vel, track_using_time, w, 0.0, 0, log, final_state,
+                            metrics});
+}
+
+int mpcb200_rollout_frenet_metrics(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, double window,
+                                   double target_vel, int32_t ey_from_path, double* log, double* final_state, double* metrics) {
+    if (h && !metrics) return fail(h, MPCB200_EINVAL, "mpcb200_rollout_frenet_metrics: metrics is required");
+    return rollout_impl(h, {"mpcb200_rollout_frenet_metrics", 1, B, T, pose0, path_of, target_vel, 0, nullptr, window, ey_from_path, log,
+                            final_state, metrics});
 }
 
 int mpcb200_get_stats(mpcb200_handle* h, mpcb200_stats* out) {

@@ -1472,9 +1472,11 @@ struct TeamSolver {
     // get_waypoints (ref_gps_traj.py:131-218) for the whole team: thread k returns waypoint k (k <= N); returns stop_cmd.
     // Nearest sample over the whole path (:136-137), np.interp of X, Y, psi at t_closest + k dt -- or at
     // s_closest + (k + 1) dt v_target in distance mode (:175) --, heading unwrap (:204-218), stop_cmd (:198-200).
+    // bi_out (closed loops that score their tracking): receives the nearest sample on every lane.
     MPC_DEV bool get_waypoints(const PathTable& p, double traj_dt, double X, double Y, double yaw, bool use_vtarget,
-                               double v_target, double& xr, double& yr, double& pr) {
+                               double v_target, double& xr, double& yr, double& pr, int* bi_out = nullptr) {
         const int bi = nearest_sample(p, X, Y);
+        if (bi_out) *bi_out = bi;
         const double* absc = use_vtarget ? p.s : p.t;
         const double start = absc[bi];
         xr = yr = pr = 0.0;
@@ -2126,6 +2128,7 @@ struct RolloutArgs {
     long B;
     const double* warm0;    // [6N+4] or null: start point of every vehicle's FIRST solve (the module-load solution)
     const double* w;        // [B][8] or null: each vehicle's cost weights for all its control periods (checked by the host); null = KCfg::w
+    double* met;            // [MET_K][B]: tracking-metric accumulators (kernels built with MET = 1 only)
 };
 
 // atan2(y, x) for x > 0 and sincos for small arguments: the plant's slip angles and steering angle are
@@ -2152,6 +2155,90 @@ MPC_DEV void sincos_small(double x, double* s, double* c) {
 }
 
 MPC_DEV double py_mod(double a, double m) { double r = fmod(a, m); if (r != 0.0 && ((r < 0.0) != (m < 0.0))) r += m; return r; }
+
+// ---- Tracking metrics of a closed-loop rollout (mpcb200_rollout_metrics, mpcb200_rollout_frenet_metrics): running sums per vehicle,
+// updated once per control period by one lane, in a structure-of-arrays accumulator m[f * stride] (f < MET_K) that lives in global
+// memory, so that nothing of it stays in registers across the solve.  A period counts when a solve ran in it (status >= 0).  Every
+// operation is rounded like numpy's, and the sums run in period order, so closed_loop.tracking_metrics reproduces them on the host.
+#define MET_N 0      // counting periods
+#define MET_SE 1     // sum of e, the distance to the nearest path sample
+#define MET_SE2 2    // sum of e^2
+#define MET_EMAX 3   // max e
+#define MET_SH2 4    // sum of h^2, h = heading error wrapped to [-pi, pi)
+#define MET_HMAX 5   // max |h|
+#define MET_SDA2 6   // sum of (acc_cmd - previous acc_cmd)^2
+#define MET_SDD2 7   // sum of (df_cmd - previous df_cmd)^2
+#define MET_NNO 8    // counting periods whose status is not MPCB200_OPTIMAL
+#define MET_IT 9     // sum of iterations
+#define MET_S 10     // s of the nearest sample in the last counting period (NaN before the first)
+#define MET_STOP 11  // first period with status -1 (the stop latch), -1 if none
+#define MET_PA 12    // commands of the previous counting period (0 before the first, like the plant and u_prev)
+#define MET_PD 13
+#define MET_K 14
+#define MET_FIELDS 12   // MPCB200_METRICS: fields 0..11 of the finalised row, in the order of the raw accumulators above
+
+MPC_DEV double max_np(double a, double b) { return (b > a || b != b) ? b : a; }   // np.maximum: NaN propagates
+
+// One control period of one vehicle: t the period (0 starts the sums), i the nearest sample of the logged pose (x, y, psi) on path p
+// (read only when status >= 0), the published commands, the solve's status (-1: no solve) and iterations.
+MPC_DEV void metrics_update(double* m, long stride, int t, const PathTable& p, int i, double x, double y, double psi,
+                            double acc, double df, int status, int iters) {
+    double v[MET_K];
+    if (t == 0) {
+        for (int f = 0; f < MET_K; f++) v[f] = 0.0;
+        v[MET_S] = nan("");
+        v[MET_STOP] = -1.0;
+    } else {
+        for (int f = 0; f < MET_K; f++) v[f] = m[f * stride];
+    }
+    if (status < 0) {
+        if (v[MET_STOP] < 0.0) v[MET_STOP] = (double)t;
+    } else {
+        const double PI = 3.141592653589793;
+        const double dx = p.X[i] - x, dy = p.Y[i] - y, e = sqrt(add_rn(mul_rn(dx, dx), mul_rn(dy, dy)));
+        const double h = py_mod(psi - p.psi[i] + PI, 2.0 * PI) - PI;
+        const double da = acc - v[MET_PA], dd = df - v[MET_PD];
+        v[MET_N] = v[MET_N] + 1.0;
+        v[MET_SE] = add_rn(v[MET_SE], e);
+        v[MET_SE2] = add_rn(v[MET_SE2], mul_rn(e, e));
+        v[MET_EMAX] = max_np(v[MET_EMAX], e);
+        v[MET_SH2] = add_rn(v[MET_SH2], mul_rn(h, h));
+        v[MET_HMAX] = max_np(v[MET_HMAX], fabs(h));
+        v[MET_SDA2] = add_rn(v[MET_SDA2], mul_rn(da, da));
+        v[MET_SDD2] = add_rn(v[MET_SDD2], mul_rn(dd, dd));
+        if (status != 0) v[MET_NNO] = v[MET_NNO] + 1.0;
+        v[MET_IT] = v[MET_IT] + (double)iters;
+        v[MET_S] = p.s[i];
+        v[MET_PA] = acc; v[MET_PD] = df;
+    }
+    for (int f = 0; f < MET_K; f++) m[f * stride] = v[f];
+}
+
+// The MET_FIELDS fields of include/mpc_b200.h (MPCB200_METRICS) from one vehicle's accumulators
+MPC_DEV void metrics_finalize(const double* m, long stride, double* out) {
+    const double n = m[MET_N * stride];
+    const bool any = n > 0.0;
+    out[0] = n;
+    out[1] = any ? m[MET_SE * stride] / n : 0.0;
+    out[2] = any ? sqrt(m[MET_SE2 * stride] / n) : 0.0;
+    out[3] = any ? m[MET_EMAX * stride] : 0.0;
+    out[4] = any ? sqrt(m[MET_SH2 * stride] / n) : 0.0;
+    out[5] = any ? m[MET_HMAX * stride] : 0.0;
+    out[6] = any ? sqrt(m[MET_SDA2 * stride] / n) : 0.0;
+    out[7] = any ? sqrt(m[MET_SDD2 * stride] / n) : 0.0;
+    out[8] = any ? m[MET_NNO * stride] : 0.0;
+    out[9] = any ? m[MET_IT * stride] : 0.0;
+    out[10] = m[MET_S * stride];
+    out[11] = m[MET_STOP * stride];
+}
+
+// metrics_update where no waypoint computation hands over the nearest sample (the per-period pipeline): the vehicle's warp searches
+// it again.  A warp collective; status is the same on every lane.
+MPC_DEV void metrics_period(TeamSolver<1>& S, double* m, long stride, int t, const PathTable& p, double x, double y, double psi,
+                            double acc, double df, int status, int iters) {
+    const int i = (status >= 0) ? S.nearest_sample(p, x, y) : 0;
+    if (S.k == 0) metrics_update(m, stride, t, p, i, x, y, psi, acc, df, status, iters);
+}
 
 // vehicle_simulator.py:58-112, one 100 Hz publish period; st = X,Y,psi,vx,vy,wz,acc,df (every lane computes the same)
 MPC_DEV void plant_step(double* st, double acc_des, double df_des) {
@@ -2194,8 +2281,9 @@ MPC_DEV double sel8(const double* v, int i) {   // register-friendly v[i] for a 
 // warp would otherwise repeat the same 100 Euler sub-steps, atan2 and sincos included: 40 % of the
 // rollout's instructions); states and commands cross through `px` ([vehicle][10] doubles) around two
 // block barriers per control period.  Warps whose vehicle index is past the fleet only keep the barriers.
+// MET = 1 (mpcb200_rollout_metrics): the nearest sample of get_waypoints also feeds metrics_update, once per period, into a.met.
 #define ROLLOUT_PX 10   // X, Y, psi, vx, vy, wz, acc, df, acc_des, df_des
-template <int W, int PW = 0>
+template <int W, int PW = 0, int MET = 0>
 MPC_DEV void rollout_group(const KCfg& cfg, const RolloutArgs& a, long b0, smem_t smem, smem_t px, int nwarps) {
     TeamSolver<W, 0, PW> S(cfg, smem);
     const int k = S.k, N = cfg.N;
@@ -2234,7 +2322,8 @@ MPC_DEV void rollout_group(const KCfg& cfg, const RolloutArgs& a, long b0, smem_
         if (!valid) continue;
         for (int i = 0; i < 8; i++) st[i] = lds(px, pxw + SO(i));
         double xr, yr, pr;
-        const bool sc = S.get_waypoints(path, cfg.dt, st[0], st[1], st[2], !a.track_using_time, des_speed, xr, yr, pr);
+        int bi = 0;
+        const bool sc = S.get_waypoints(path, cfg.dt, st[0], st[1], st[2], !a.track_using_time, des_speed, xr, yr, pr, MET ? &bi : nullptr);
         S.set_ref(xr, yr, pr);
         if (sc) stop = true;   // latch, mpc_cmd_pub.jl:102-111
         int status = -1, iters = 0;
@@ -2254,6 +2343,7 @@ MPC_DEV void rollout_group(const KCfg& cfg, const RolloutArgs& a, long b0, smem_
             const double lv[8] = {st[0], st[1], st[2], st[3], acc_des, df_des, (double)status, (double)iters};
             a.log[((long)t * a.B + b) * 8 + k] = sel8(lv, k);
         }
+        if (MET && k == 0) metrics_update(a.met + b, a.B, t, path, bi, st[0], st[1], st[2], acc_des, df_des, status, iters);
     }
     if (valid && a.final_state && k < 8) a.final_state[b * 8 + k] = sel8(st, k);
     block_sync();
@@ -2326,9 +2416,10 @@ inline void cubic_fit_matrix(int n, double step, double* P) {
 // the host-built matrices P1, P2 times the samples: lanes stride the samples, the partial sums are reduced over the warp.  Used by
 // the fused closed-loop kernel (rollout_group_frenet) and by the per-period pipeline (rollout_frenet_ref_kernel).
 MPC_DEV void frenet_reference(TeamSolver<1, 1>& S, const PathTable& path, const FrenetRolloutArgs& a, double X, double Y, double yaw,
-                              double kc[4], double& ey, double& psi0) {
+                              double kc[4], double& ey, double& psi0, int* bi_out = nullptr) {
     const int k = S.k;
     const int bi = S.nearest_sample(path, X, Y);
+    if (bi_out) *bi_out = bi;
     const double s_i = path.s[bi];
     double sps, cps;
     mpc_sincos(yaw, &sps, &cps);
@@ -2360,7 +2451,11 @@ MPC_DEV void frenet_reference(TeamSolver<1, 1>& S, const PathTable& path, const 
     ey = a.ey_from_path ? -(-sp0 * xw0 + cp0 * yw0) : 0.0;
 }
 
-MPC_DEV void rollout_group_frenet(const KCfg& cfg, const FrenetRolloutArgs& a, long b0, smem_t smem, smem_t px, int nwarps) {
+// MET = 1 (mpcb200_rollout_frenet_metrics): the nearest sample of frenet_reference also feeds metrics_update, once per period, into
+// met = [MET_K][B] (an argument of its own: rollout_frenet_ref_kernel takes FrenetRolloutArgs by value, which therefore keeps its size)
+template <int MET = 0>
+MPC_DEV void rollout_group_frenet(const KCfg& cfg, const FrenetRolloutArgs& a, long b0, smem_t smem, smem_t px, int nwarps,
+                                  double* met = nullptr) {
     TeamSolver<1, 1> S(cfg, smem);
     const int k = S.k, N = cfg.N;
     const int w = thread_in_block() >> 5;
@@ -2388,7 +2483,8 @@ MPC_DEV void rollout_group_frenet(const KCfg& cfg, const FrenetRolloutArgs& a, l
         for (int i = 0; i < 8; i++) st[i] = lds(px, pxw + SO(i));
         // ---- the path ahead -> curvature polynomial, e_y, psi_start
         double kc[4], ey, psi0;
-        frenet_reference(S, path, a, st[0], st[1], st[2], kc, ey, psi0);
+        int bi = 0;
+        frenet_reference(S, path, a, st[0], st[1], st[2], kc, ey, psi0, MET ? &bi : nullptr);
         // ---- update_init_cond(0, e_y, -psi_start, v), update_reference(path, K_coeffs, des_speed), solve_model (:125-130)
         S.set_kpoly(kc[0], kc[1], kc[2], kc[3]);
         syncwarp();
@@ -2404,6 +2500,7 @@ MPC_DEV void rollout_group_frenet(const KCfg& cfg, const FrenetRolloutArgs& a, l
             const double lv[8] = {st[0], st[1], st[2], st[3], acc_des, df_des, (double)r.status, (double)r.iters};
             a.log[((long)t * a.B + b) * 8 + k] = sel8(lv, k);
         }
+        if (MET && k == 0) metrics_update(met + b, a.B, t, path, bi, st[0], st[1], st[2], acc_des, df_des, r.status, r.iters);
     }
     if (valid && a.final_state && k < 8) a.final_state[b * 8 + k] = sel8(st, k);
     block_sync();
