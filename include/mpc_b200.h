@@ -292,7 +292,7 @@ int mpcb200_rollout_frenet_metrics(mpcb200_handle* h, int64_t B, int32_t T, cons
 
 /* Counters of the last solve_batch/rollout call on this handle. */
 typedef struct {
-    int64_t kernel_launches;   /* kernels of this library launched by the call */
+    int64_t kernel_launches;   /* kernels of this library launched by the call (a radix sort counts as one) */
     int64_t h2d_bytes, d2h_bytes;
     float   kernel_ms;         /* device time of the solver kernel(s) (CUDA events), HOST mode only */
 } mpcb200_stats;

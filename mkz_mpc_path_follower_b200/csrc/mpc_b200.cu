@@ -8,6 +8,7 @@
 #include "mpc_kernel.cuh"
 #include "tpp_solver.cuh"
 
+#include <cub/device/device_radix_sort.cuh>
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -36,16 +37,27 @@ constexpr int WARPS_PER_BLOCK = 4;
 #ifndef MPC_MIN_BLOCKS
 #define MPC_MIN_BLOCKS 3
 #endif
-template <int PW>
+#ifndef MPC_ORDER_MIN_QUARTER_WAVES
+#define MPC_ORDER_MIN_QUARTER_WAVES 5   /* mpcb200_create: from how many quarter waves of resident teams a batch is ordered (0: all) */
+#endif
+//
+// ORD = 1: the queue is `order` (a permutation of 0 .. B-1, longest predicted solve first: queue_key_kernel and a radix sort),
+// and a warp solves problem order[counter] instead of problem counter.  Every problem still reads and writes its own index, so
+// the results are those of ORD = 0 bit for bit; only which warp solves a problem, and when, changes.  The team kernels take
+// `order` as their last parameter so that they share one launch signature; the ORD = 0 builds never read it.
+template <int PW, int ORD = 0>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, MPC_MIN_BLOCKS)
-mpc_solve_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const long long B, unsigned long long* counter) {
+mpc_solve_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const long long B, unsigned long long* counter, const int* order) {
     extern __shared__ double smem_all[];
     const int warp = threadIdx.x >> 5;
     const smem_t smem = smem_base(smem_all + (size_t)warp * smem_doubles_per_team(cfg.N, 0, PW));
     TeamSolver<1>::init_work(smem, cfg.N);
     for (;;) {
         unsigned long long b = 0;
-        if ((threadIdx.x & 31) == 0) b = atomicAdd(counter, 1ULL);
+        if ((threadIdx.x & 31) == 0) {
+            b = atomicAdd(counter, 1ULL);
+            if (ORD && b < (unsigned long long)B) b = (unsigned long long)order[b];
+        }
         b = __shfl_sync(0xffffffffu, b, 0);
         if (b >= (unsigned long long)B) break;
         solve_problem<1, 0, PW>(cfg, io, rg, (long)b, smem);
@@ -59,7 +71,7 @@ mpc_solve_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const long
 // mpcb200_create_frenet picks per horizon (see there)
 template <int WPB, int PW = 0>
 __global__ void __launch_bounds__(WPB * 32, WPB == 3 ? 3 : 2)
-mpc_solve_frenet_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const long long B, unsigned long long* counter) {
+mpc_solve_frenet_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const long long B, unsigned long long* counter, const int*) {
     extern __shared__ double smem_all[];
     const int warp = threadIdx.x >> 5;
     const smem_t smem = smem_base(smem_all + (size_t)warp * smem_doubles_per_team(cfg.N, 1, PW));
@@ -82,7 +94,7 @@ mpc_solve_frenet_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, con
 #endif
 template <int W, int MODEL = 0, int PW = 0>
 __global__ void __launch_bounds__(W * 32, MODEL ? 2 : (W == 2 ? MPC_LONG_MIN_BLOCKS2 : MPC_LONG_MIN_BLOCKS3))
-mpc_solve_long_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const long long B, unsigned long long* counter) {
+mpc_solve_long_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const long long B, unsigned long long* counter, const int*) {
     extern __shared__ double smem_all[];
     __shared__ unsigned long long next_problem;
     const smem_t smem = smem_base(smem_all);
@@ -94,6 +106,26 @@ mpc_solve_long_kernel(const KCfg cfg, const BatchPtrs io, const RefGen rg, const
         __syncthreads();
         if (b >= (unsigned long long)B) break;
         solve_problem<W, MODEL, PW>(cfg, io, rg, (long)b, smem);
+    }
+}
+
+// ---- Queue order of mpc_solve_kernel<PW, 1> for large cold-start batches (DESIGN §6, item 3).  From the all-zero start the iteration
+// counts spread from ~20 to the 200 cap (p50 42, p99 92 at N = 20), and one iteration costs a warp the same time whether its SM
+// is full or not, so a long solve taken late keeps the launch running after the queue is empty.  Taking the problems with the
+// longest predicted solve first leaves the short ones to fill the end.  The prediction is a linear score of raw inputs fitted by
+// least squares to the oracle's iteration counts (tools/queue_order_model.py: the bench batch to fit, the next 65,536 problems to
+// judge; R^2 0.18, but the longest solves come first): the vehicle's distance from the path frame's origin (log), the heading
+// change of the reference over the horizon, the previous steering and acceleration commands.  key[b] = the score in 16.16 fixed
+// point, clamped to [0, 256): the 24 bits the descending radix sort of (key, index) looks at.
+__global__ void __launch_bounds__(256)
+queue_key_kernel(const long long B, const int N, const double* state, const double* ref, const double* u_prev, unsigned* key, int* index) {
+    const long long nr = 3LL * (N + 1);
+    for (long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x; b < B; b += (long long)gridDim.x * blockDim.x) {
+        const double* rp = ref + nr * b + 2 * (N + 1);
+        const double s = 69.91 - 5.253 * log1p(hypot(state[4 * b], state[4 * b + 1])) + 0.7904 * fabs(rp[N] - rp[0])
+                         + 30.34 * fabs(u_prev[2 * b]) - 1.304 * u_prev[2 * b + 1];
+        key[b] = (s > 0.0) ? (unsigned)(fmin(s, 255.99) * 65536.0) : 0u;   // NaN inputs: last
+        index[b] = (int)b;
     }
 }
 
@@ -403,6 +435,9 @@ struct mpcb200_handle {
     DevBuf d_veh, d_vstop;            /* ... closed-loop fleets: vehicle state [12][Bp], stop latches */
     DevBuf d_w;                       /* per-problem weight rows of a weighted call (host pointers) */
     DevBuf d_met, d_metout;           /* rollout tracking metrics: accumulators [MET_K][stride], rows [B][MET_FIELDS] */
+    DevBuf d_order;                   /* queue order of large cold-start batches: keys, indices (in, out) and the sort's scratch */
+    int64_t order_min_batch = 1;      /* ... taken from this many problems on */
+    int blocks_per_sm_ord = 0;        /* resident blocks per SM of the queue-ordered one-warp XY solve kernel (mpc_solve_kernel<0, 1>) */
     int blocks_per_sm_w = 0;          /* resident blocks per SM of the PW = 1 solve kernel of this handle (8 more doubles per team) */
     int rollout_blocks_per_sm_w = 0;  /* ... of the PW = 1 fused rollout kernel */
     int tpp_blocks_per_sm = 0;        /* resident blocks of mpc_solve_tpp_kernel per SM */
@@ -506,7 +541,7 @@ static KCfg make_kcfg(const mpcb200_handle* h) {
 static int teams_per_block(const mpcb200_handle* h) { return (h->team_warps != 1) ? 1 : (h->model ? h->frenet_wpb : WARPS_PER_BLOCK); }
 
 /* the warp / block-per-problem solve kernel of a handle (model, team size, Frenet block size) and its threads per block */
-typedef void (*TeamKernel)(const KCfg, const BatchPtrs, const RefGen, const long long, unsigned long long*);
+typedef void (*TeamKernel)(const KCfg, const BatchPtrs, const RefGen, const long long, unsigned long long*, const int*);
 template <int PW>
 static TeamKernel team_kernel(const mpcb200_handle* h, int* threads) {
     *threads = 32 * h->team_warps;
@@ -697,6 +732,9 @@ static int create_impl(mpcb200_handle** out, const mpcb200_config* cfg, int mode
         int threads = 0;
         const void* fn = (const void*)team_kernel<0>(h, &threads);
         TRY_OR_FREE(prepare_kernel(fn, h->device, threads, h->smem_bytes, &h->blocks_per_sm));
+        if (!model && h->team_warps == 1) {   /* the queue-ordered build of the same kernel (same registers and footprint) */
+            TRY_OR_FREE(prepare_kernel((const void*)mpc_solve_kernel<0, 1>, h->device, threads, h->smem_bytes, &h->blocks_per_sm_ord));
+        }
         if (!model)
             TRY_OR_FREE(prepare_kernel((const void*)rollout_kernel<0>(h), h->device, threads, rollout_smem_bytes(h, false), &h->rollout_blocks_per_sm));
     }
@@ -725,6 +763,16 @@ static int create_impl(mpcb200_handle** out, const mpcb200_config* cfg, int mode
     }
     if (h->blocks_per_sm < 1) h->blocks_per_sm = 1;
     if (const char* e = getenv("MPCB200_BLOCKS_PER_SM")) { int v = atoi(e); if (v >= 1 && v < h->blocks_per_sm) h->blocks_per_sm = v; }  /* tuning aid */
+    /* the ordered kernel is the same solver with two more instructions; should it ever fit fewer blocks, its grid follows */
+    if (h->blocks_per_sm_ord < 1 || h->blocks_per_sm_ord > h->blocks_per_sm) h->blocks_per_sm_ord = h->blocks_per_sm;
+    /* cold-start batches of the one-warp XY kernel take their problems longest predicted solve first (queue_order) from 5/4
+     * waves of resident teams on (2,220 problems on a B200).  Measured at N = 20 against counter order, 7 alternated runs
+     * (profiles/r05_logs/queue_order_threshold.log; run-to-run spread 1-5 % at these sizes): 1,776 problems (one wave: every
+     * problem starts at once, the ~40 us of key kernel and sort are pure cost) +1.3 %, 1,900 +0.6 %, 2,048 -2.8 %, 2,304 -2.8 %,
+     * 2,664 -3.2 %, 3,072 -3.2 %, 3,552 -2.2 %; 8,192 -17 %, 65,536 -3.7 % (queue_order_ab.log).  Break-even lies between 1.07
+     * and 1.15 waves; the threshold keeps a margin above it for GPUs with other SM counts and for the spread */
+    h->order_min_batch = (int64_t)MPC_ORDER_MIN_QUARTER_WAVES * h->num_sms * h->blocks_per_sm_ord * WARPS_PER_BLOCK / 4;
+    if (h->order_min_batch < 1) h->order_min_batch = 1;
 #undef TRY_OR_FREE
     *out = h;
     return MPCB200_OK;
@@ -738,7 +786,7 @@ int mpcb200_destroy(mpcb200_handle* h) {
     DevBuf* bufs[] = {&h->d_state, &h->d_ref, &h->d_vdes, &h->d_uprev, &h->d_warm, &h->d_u0, &h->d_cost, &h->d_status, &h->d_iters, &h->d_traj,
                       &h->d_path[0], &h->d_path[1], &h->d_path[2], &h->d_pose, &h->d_pathof, &h->d_log, &h->d_final, &h->d_stop, &h->d_stage,
                       &h->d_rec, &h->d_resto, &h->d_seed, &h->d_fit, &h->d_tpp_state, &h->d_tpp_filt, &h->d_veh, &h->d_vstop, &h->d_genref,
-                      &h->d_w};
+                      &h->d_w, &h->d_order};
     for (DevBuf* b : bufs) if (b->p) cudaFree(b->p);
     if (h->d_counter) cudaFree(h->d_counter);
     if (h->d_roles) cudaFree(h->d_roles);
@@ -775,6 +823,28 @@ int mpcb200_set_stream(mpcb200_handle* h, void* s) {
     h->stream = s ? (cudaStream_t)s : h->own_stream;
     drop_graphs(h);
     return MPCB200_OK;
+}
+
+/* the queue order of mpc_solve_kernel<0, 1>: a key per problem (queue_key_kernel), then a stable descending radix sort of
+ * (key, index) over the key's 24 bits; *order = the sorted indices, in h->d_order (sized at the first large batch) */
+static int queue_order(mpcb200_handle* h, int64_t B, const BatchPtrs& io, const int** order) {
+    const int n = (int)B;
+    size_t sort_bytes = 0;
+    CUDA_TRY(h, cub::DeviceRadixSort::SortPairsDescending(nullptr, sort_bytes, (const unsigned*)nullptr, (unsigned*)nullptr,
+                                                          (const int*)nullptr, (int*)nullptr, n, 0, 24, h->stream));
+    const size_t arr = ((size_t)n * sizeof(int) + 255) / 256 * 256;
+    int rc;
+    if ((rc = ensure(h, h->d_order, 4 * arr + sort_bytes))) return rc;
+    char* base = (char*)h->d_order.p;
+    unsigned* key_in = (unsigned*)base; unsigned* key_out = (unsigned*)(base + arr);
+    int* idx_in = (int*)(base + 2 * arr); int* idx_out = (int*)(base + 3 * arr);
+    const long long kb = (B + 255) / 256, kmax = (long long)h->num_sms * 8;
+    queue_key_kernel<<<(int)(kb < kmax ? kb : kmax), 256, 0, h->stream>>>((long long)B, h->cfg.N, io.state, io.ref, io.u_prev, key_in, idx_in);
+    CUDA_TRY(h, cudaGetLastError());
+    CUDA_TRY(h, cub::DeviceRadixSort::SortPairsDescending(base + 4 * arr, sort_bytes, key_in, key_out, idx_in, idx_out, n, 0, 24, h->stream));
+    h->stats.kernel_launches += 2;   /* the key kernel and the sort (one call of cub's radix sort, which launches several kernels) */
+    *order = idx_out;
+    return 0;
 }
 
 static int launch_solve(mpcb200_handle* h, int64_t B, const BatchPtrs& io, const RefGen& rg, unsigned long long* zeroed_counter = nullptr) {
@@ -834,14 +904,24 @@ static int launch_solve(mpcb200_handle* h, int64_t B, const BatchPtrs& io, const
     }
     const int tpb = teams_per_block(h);
     const bool pw = io.w != nullptr;
+    /* longest predicted solve first (queue_key_kernel): XY one-warp teams, references from the caller, cold starts with the
+     * handle's weights -- what the score was fitted on; warm and rollout starts take a few iterations each, no tail to cut */
+    const bool ordered = B >= h->order_min_batch && B <= INT32_MAX && !zeroed_counter && !h->model && h->team_warps == 1 &&
+                         !rg.path_of && !io.warm && !pw && h->cfg.start_mode == MPCB200_START_ZERO;
     long long blocks_needed = (B + tpb - 1) / tpb;
-    long long max_blocks = (long long)h->num_sms * (pw ? h->blocks_per_sm_w : h->blocks_per_sm);
+    long long max_blocks = (long long)h->num_sms * (pw ? h->blocks_per_sm_w : (ordered ? h->blocks_per_sm_ord : h->blocks_per_sm));
     int grid = (int)(blocks_needed < max_blocks ? blocks_needed : max_blocks);
     if (grid < 1) grid = 1;
     int threads = 0;
-    const TeamKernel tk = pw ? team_kernel<1>(h, &threads) : team_kernel<0>(h, &threads);
+    TeamKernel tk = pw ? team_kernel<1>(h, &threads) : team_kernel<0>(h, &threads);
     const size_t smem = h->smem_bytes + (pw ? (size_t)tpb * 8 * sizeof(double) : 0);
-    tk<<<grid, threads, smem, h->stream>>>(make_kcfg(h), io, rg, (long long)B, counter);
+    const int* order = nullptr;
+    if (ordered) {
+        int rc;
+        if ((rc = queue_order(h, B, io, &order))) return rc;
+        tk = mpc_solve_kernel<0, 1>;
+    }
+    tk<<<grid, threads, smem, h->stream>>>(make_kcfg(h), io, rg, (long long)B, counter, order);
     CUDA_TRY(h, cudaGetLastError());
     h->stats.kernel_launches += 1;
     return 0;
