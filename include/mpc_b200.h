@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define MPCB200_VERSION 4
+#define MPCB200_VERSION 5
 
 /* error codes */
 #define MPCB200_OK          0
@@ -285,10 +285,19 @@ int mpcb200_solve_batch_frenet_w(mpcb200_handle* h, int64_t B, const double* sta
 int mpcb200_rollout_frenet(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of,
                            double window, double target_vel, int32_t ey_from_path, double* log, double* final_state);
 /* mpcb200_rollout_frenet with the tracking metrics of mpcb200_rollout_metrics (every period counts; stop_period is always -1).
- * Per-vehicle weights are not available for Frenet rollouts: mpcb200_rollout_metrics refuses a Frenet handle (MPCB200_EINVAL). */
+ * mpcb200_rollout_metrics refuses a Frenet handle (MPCB200_EINVAL); per-vehicle weights are mpcb200_rollout_frenet_w's. */
 int mpcb200_rollout_frenet_metrics(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of,
                                    double window, double target_vel, int32_t ey_from_path,
                                    double* log, double* final_state, double* metrics);
+/* mpcb200_rollout_frenet with one cost-weight row per vehicle, w [B][7] in the update_cost order of MKZMPCPathFollowerFrenet.jl
+ * (cey, cep, cev, cda, cdd, ca, cd), used in every control period of that vehicle (a Frenet closed-loop tuning sweep in one call).
+ * w is required (NULL with B > 0 and T > 0 is MPCB200_EINVAL); rows are checked as by mpcb200_solve_batch_frenet_w with host
+ * pointers.  metrics [B][MPCB200_METRICS] or NULL: when given, filled as mpcb200_rollout_frenet_metrics fills it.  Everything else
+ * -- host pointers, N <= 31, window, the fused / per-period switch, the first solve from all zeros, devices[0] of a multi-GPU
+ * handle -- is that of mpcb200_rollout_frenet. */
+int mpcb200_rollout_frenet_w(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of,
+                             double window, double target_vel, int32_t ey_from_path, const double* w,
+                             double* log, double* final_state, double* metrics);
 
 /* Counters of the last solve_batch/rollout call on this handle. */
 typedef struct {

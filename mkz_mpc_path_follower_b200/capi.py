@@ -73,6 +73,7 @@ def lib():
     L.mpcb200_rollout_frenet.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_double, C.c_double, C.c_int32, dp, dp]
     L.mpcb200_rollout_metrics.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_int32, C.c_double, dp, dp, dp, dp]
     L.mpcb200_rollout_frenet_metrics.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_double, C.c_double, C.c_int32, dp, dp, dp]
+    L.mpcb200_rollout_frenet_w.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_double, C.c_double, C.c_int32, dp, dp, dp, dp]
     L.mpcb200_get_stats.argtypes = [vp, C.POINTER(Stats)]
     L.mpcb200_fp64_peak.argtypes = [vp, dp]
     L.mpcb200_last_error.argtypes = [vp]
@@ -369,10 +370,12 @@ class FrenetSolver(Solver):
                                                            _ptr(w), _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj), HOST))
         return {"u0": u0, "cost": cost, "status": status, "iters": iters, "traj": traj}
 
-    def rollout(self, pose0, path_of, T, window=40.0, target_vel=8.0, ey_from_path=True, want_log=True, metrics=False):
+    def rollout(self, pose0, path_of, T, window=40.0, target_vel=8.0, ey_from_path=True, want_log=True, metrics=False, weights=None):
         """Closed loop on the Frenet-frame module on the device (mpcb200_rollout_frenet; what closed_loop.run_frenet does on the
         host).  pose0 (B,3); path_of (B,) ids given to set_path.  Returns log (T,B,8) and final (B,8) like Solver.rollout;
-        metrics: also out["metrics"] (B,12) as Solver.rollout (mpcb200_rollout_frenet_metrics)."""
+        metrics: also out["metrics"] (B,12) as Solver.rollout (mpcb200_rollout_frenet_metrics).
+        weights (B,7) in set_cost's order (cey, cep, cev, cda, cdd, ca, cd): each vehicle's cost weights for all its control
+        periods (mpcb200_rollout_frenet_w, with or without metrics), or None: the handle's."""
         pose0 = np.ascontiguousarray(np.atleast_2d(pose0), dtype=np.float64)
         B = pose0.shape[0]
         path_of = np.ascontiguousarray(path_of, dtype=np.int32)
@@ -383,6 +386,15 @@ class FrenetSolver(Solver):
         dp = C.POINTER(C.c_double)
         args = [pose0.ctypes.data_as(dp), path_of.ctypes.data_as(C.POINTER(C.c_int32)), float(window), float(target_vel),
                 int(bool(ey_from_path)), None if log is None else log.ctypes.data_as(dp), final.ctypes.data_as(dp)]
+        if weights is not None:
+            w = _weight_rows(weights, B, 7, "rollout")
+            met = np.empty((B, len(ROLLOUT_METRICS))) if metrics else None
+            self._check(lib().mpcb200_rollout_frenet_w(self._h, B, int(T), *args[:5], w.ctypes.data_as(dp), *args[5:],
+                                                       None if met is None else met.ctypes.data_as(dp)))
+            out = {"log": log, "final_state": final}
+            if metrics:
+                out["metrics"] = met
+            return out
         if metrics:
             met = np.empty((B, len(ROLLOUT_METRICS)))
             self._check(lib().mpcb200_rollout_frenet_metrics(self._h, B, int(T), *args, met.ctypes.data_as(dp)))

@@ -239,7 +239,7 @@ rollout_waypoints_kernel(const KCfg cfg, const long long B, const long long Bp, 
 // MODEL 0: reference samples already in the slots, stop latch, the first solve from the module-load solution `warm0`.
 // MODEL 1 (closed loop of the Frenet node, gazebo_sim_mpc_cmd_pub_frenet.jl:112-153): `fref` = [6][Bp] curvature polynomial (4),
 // e_y, psi_start per vehicle from rollout_frenet_ref_kernel; state (0, e_y, -psi_start, v); the first solve from all zeros.
-// PW: each vehicle's cost weights from out.w (mpcb200_rollout_w), the slot keeps its vehicle and so its row
+// PW: each vehicle's cost weights from out.w (mpcb200_rollout_w, mpcb200_rollout_frenet_w), the slot keeps its vehicle and so its row
 template <int MODEL, int PW = 0>
 __global__ void __launch_bounds__(MPC_TPP_BLOCK, MPC_TPP_MIN_BLOCKS)
 rollout_solve_tpp_kernel(const KCfg cfg, const long long B, const long long Bp, double* veh, const int* stop, double* tpp_state, double* tpp_filt,
@@ -248,7 +248,7 @@ rollout_solve_tpp_kernel(const KCfg cfg, const long long B, const long long Bp, 
     const bool valid = v < B;
     const TppMemT<MODEL> mem(tpp_state, tpp_filt, cfg.N, (long)(valid ? v : 0));
     TppSolverT<MODEL, PW> sv(cfg, mem);
-    if (PW && valid && out.w) sv.wr = out.w + 8 * v;
+    if (PW && valid && out.w) sv.wr = out.w + (MODEL ? 7 : 8) * v;
     const bool stopped = valid && !MODEL && stop[v] != 0;
     bool live = valid && !stopped;
     double st4[4] = {0.0, 0.0, 0.0, 0.0};
@@ -376,13 +376,14 @@ mpc_rollout_long_kernel(const KCfg cfg, const RolloutArgs args, unsigned long lo
 
 // Closed loop on the Frenet-frame module (gazebo_sim_mpc_cmd_pub_frenet.jl:112-153): four vehicles per block
 // met: [MET_K][B] accumulators of MET = 1 (rollout_group_frenet)
-template <int MET = 0>
+// PW: each vehicle's cost weights from w = [B][7] (mpcb200_rollout_frenet_w); an argument after met so that the PW = 0 kernels keep theirs
+template <int MET = 0, int PW = 0>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 2)
-mpc_rollout_frenet_kernel(const KCfg cfg, const FrenetRolloutArgs args, unsigned long long* counter, double* met) {
+mpc_rollout_frenet_kernel(const KCfg cfg, const FrenetRolloutArgs args, unsigned long long* counter, double* met, const double* w) {
     extern __shared__ double smem_all[];
     const int warp = threadIdx.x >> 5;
-    const smem_t smem = smem_base(smem_all + (size_t)warp * smem_doubles_per_team(cfg.N, 1));
-    const smem_t px = smem_base(smem_all + (size_t)WARPS_PER_BLOCK * smem_doubles_per_team(cfg.N, 1));
+    const smem_t smem = smem_base(smem_all + (size_t)warp * smem_doubles_per_team(cfg.N, 1, PW));
+    const smem_t px = smem_base(smem_all + (size_t)WARPS_PER_BLOCK * smem_doubles_per_team(cfg.N, 1, PW));
     __shared__ unsigned long long next_group;
     TeamSolver<1, 1>::init_work(smem, cfg.N);
     for (;;) {
@@ -391,7 +392,7 @@ mpc_rollout_frenet_kernel(const KCfg cfg, const FrenetRolloutArgs args, unsigned
         const unsigned long long b0 = next_group;
         __syncthreads();
         if (b0 >= (unsigned long long)args.B) break;
-        rollout_group_frenet<MET>(cfg, args, (long)b0, smem, px, WARPS_PER_BLOCK, met);
+        rollout_group_frenet<MET, PW>(cfg, args, (long)b0, smem, px, WARPS_PER_BLOCK, met, w);
     }
 }
 
@@ -563,7 +564,7 @@ static RolloutKernel rollout_kernel(const mpcb200_handle* h) {
 /* dynamic shared memory of the fused rollout kernel: the teams and the plant exchange area (the XY handle's smem_bytes already
  * holds it at N <= 31; the Frenet kernel always runs WARPS_PER_BLOCK vehicles per block, whatever frenet_wpb is) */
 static size_t rollout_smem_bytes(const mpcb200_handle* h, bool pw) {
-    if (h->model) return WARPS_PER_BLOCK * ((size_t)smem_doubles_per_team(h->cfg.N, 1) + ROLLOUT_PX) * sizeof(double);
+    if (h->model) return WARPS_PER_BLOCK * ((size_t)smem_doubles_per_team(h->cfg.N, 1, pw) + ROLLOUT_PX) * sizeof(double);
     return h->smem_bytes + (h->team_warps == 1 ? 0 : ROLLOUT_PX * sizeof(double)) + (pw ? (size_t)teams_per_block(h) * 8 * sizeof(double) : 0);
 }
 
@@ -1402,14 +1403,14 @@ static int ensure_seed(mpcb200_handle* h) {
     return rc;
 }
 
-/* one closed-loop call: mpcb200_rollout and mpcb200_rollout_w (model 0) or mpcb200_rollout_frenet (model 1) */
+/* one closed-loop call: mpcb200_rollout and mpcb200_rollout_w (model 0) or mpcb200_rollout_frenet and mpcb200_rollout_frenet_w (model 1) */
 struct RolloutCall {
     const char* who;
     int model;
     int64_t B; int32_t T;
     const double* pose0; const int32_t* path_of;
     double target_vel;
-    int32_t track_using_time; const double* w;   /* XY: waypoints by time or arc length; [B][8] weight rows or null */
+    int32_t track_using_time; const double* w;   /* XY: waypoints by time or arc length; [B][8] ([B][7] Frenet) weight rows or null */
     double window; int32_t ey_from_path;          /* Frenet: length of the path ahead, e_y from the path or from the fit */
     double* log; double* final_state;             /* [T][B][8], [B][8] or null */
     double* metrics;                              /* [B][MET_FIELDS] or null (the plain entry points) */
@@ -1448,9 +1449,10 @@ static int rollout_enqueue(mpcb200_handle* h, const RolloutCall& c, int64_t lo, 
     CUDA_TRY(h, cudaMemcpyAsync(h->d_pathof.p, c.path_of + lo, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     h->stats.h2d_bytes += (size_t)n * (3 * sizeof(double) + sizeof(int32_t));
     if (c.w) {
-        if ((rc = ensure(h, h->d_w, (size_t)n * 8 * sizeof(double)))) return rc;
-        CUDA_TRY(h, cudaMemcpyAsync(h->d_w.p, c.w + 8 * lo, (size_t)n * 8 * sizeof(double), cudaMemcpyHostToDevice, s));
-        h->stats.h2d_bytes += (size_t)n * 8 * sizeof(double);
+        const size_t nw = c.model ? 7 : 8;
+        if ((rc = ensure(h, h->d_w, (size_t)n * nw * sizeof(double)))) return rc;
+        CUDA_TRY(h, cudaMemcpyAsync(h->d_w.p, c.w + nw * lo, (size_t)n * nw * sizeof(double), cudaMemcpyHostToDevice, s));
+        h->stats.h2d_bytes += (size_t)n * nw * sizeof(double);
     }
     /* the kernel arguments of both models; only those of c.model are launched with */
     RolloutArgs a;
@@ -1488,7 +1490,8 @@ static int rollout_enqueue(mpcb200_handle* h, const RolloutCall& c, int64_t lo, 
         BatchPtrs out;
         memset(&out, 0, sizeof(out));
         out.u0 = (double*)h->d_u0.p; out.status = (int*)h->d_status.p; out.iters = (int*)h->d_iters.p; out.w = a.w;
-        auto sk = c.model ? rollout_solve_tpp_kernel<1, 0> : (a.w ? rollout_solve_tpp_kernel<0, 1> : rollout_solve_tpp_kernel<0, 0>);
+        auto sk = c.model ? (a.w ? rollout_solve_tpp_kernel<1, 1> : rollout_solve_tpp_kernel<1, 0>)
+                          : (a.w ? rollout_solve_tpp_kernel<0, 1> : rollout_solve_tpp_kernel<0, 0>);
         RefGen rg;
         memset(&rg, 0, sizeof(rg));
         fill_paths(h, rg.paths);
@@ -1527,14 +1530,17 @@ static int rollout_enqueue(mpcb200_handle* h, const RolloutCall& c, int64_t lo, 
     int bps = c.model ? h->frenet_rollout_blocks_per_sm : (c.w ? h->rollout_blocks_per_sm_w : h->rollout_blocks_per_sm);
     const int threads = 32 * (h->team_warps == 1 ? WARPS_PER_BLOCK : h->team_warps);
     const size_t smem = rollout_smem_bytes(h, c.w != nullptr);
-    /* the MET = 1 instantiations: shared-memory limit and residency prepared here, by the calls that launch them */
-    const void* met_fn = !c.metrics ? nullptr : c.model ? (const void*)mpc_rollout_frenet_kernel<1>
-                                                         : (const void*)(c.w ? rollout_kernel<1, 1>(h) : rollout_kernel<0, 1>(h));
-    if (met_fn) CUDA_TRY(h, prepare_kernel(met_fn, h->device, threads, smem, &bps));
+    auto fk = c.metrics ? (c.w ? mpc_rollout_frenet_kernel<1, 1> : mpc_rollout_frenet_kernel<1, 0>)
+                        : (c.w ? mpc_rollout_frenet_kernel<0, 1> : mpc_rollout_frenet_kernel<0, 0>);
+    /* the MET = 1 and the Frenet PW = 1 instantiations: shared-memory limit and residency prepared here, by the calls that launch them */
+    const void* prep_fn = nullptr;
+    if (c.model && (c.metrics || c.w)) prep_fn = (const void*)fk;
+    else if (!c.model && c.metrics) prep_fn = (const void*)(c.w ? rollout_kernel<1, 1>(h) : rollout_kernel<0, 1>(h));
+    if (prep_fn) CUDA_TRY(h, prepare_kernel(prep_fn, h->device, threads, smem, &bps));
     long long max_blocks = (long long)h->num_sms * bps;
     const int grid = (int)(blocks_needed < max_blocks ? blocks_needed : max_blocks);
     CUDA_TRY(h, cudaEventRecord(h->ev0, s));
-    if (c.model) (c.metrics ? mpc_rollout_frenet_kernel<1> : mpc_rollout_frenet_kernel<0>)<<<grid, threads, smem, s>>>(kc, fa, h->d_counter, a.met);
+    if (c.model) fk<<<grid, threads, smem, s>>>(kc, fa, h->d_counter, a.met, a.w);
     else if (c.metrics) (c.w ? rollout_kernel<1, 1>(h) : rollout_kernel<0, 1>(h))<<<grid, threads, smem, s>>>(kc, a, h->d_counter);
     else (c.w ? rollout_kernel<1>(h) : rollout_kernel<0>(h))<<<grid, threads, smem, s>>>(kc, a, h->d_counter);
     if (c.metrics) rollout_metrics_final_kernel<<<(int)((n + 127) / 128), 128, 0, s>>>((long long)n, (long long)n, a.met, (double*)h->d_metout.p);
@@ -1566,7 +1572,8 @@ static int rollout_collect(mpcb200_handle* h, const RolloutCall& c, int64_t lo, 
     return MPCB200_OK;
 }
 
-/* the body of mpcb200_rollout, mpcb200_rollout_w (w == NULL: the handle's weights), mpcb200_rollout_frenet and their _metrics forms */
+/* the body of mpcb200_rollout, mpcb200_rollout_w (w == NULL: the handle's weights), mpcb200_rollout_frenet, mpcb200_rollout_frenet_w
+ * and the _metrics forms */
 static int rollout_impl(mpcb200_handle* h, const RolloutCall& c) {
     const char* who = c.who;
     if (!h) return MPCB200_EINVAL;
@@ -1580,7 +1587,7 @@ static int rollout_impl(mpcb200_handle* h, const RolloutCall& c) {
     if (!c.pose0 || !c.path_of) return fail(h, MPCB200_EINVAL, "%s: pose0 and path_of are required", who);
     int rc;
     if ((rc = check_path_ids(h, who, "vehicle", c.B, c.path_of))) return rc;
-    if (c.w && (rc = check_weight_rows(h, who, "vehicle", c.B, c.w, 8))) return rc;
+    if (c.w && (rc = check_weight_rows(h, who, "vehicle", c.B, c.w, c.model ? 7 : 8))) return rc;
     /* a vehicle stays on one GPU for all T steps: contiguous slices of the fleet, every device at once.  Frenet fleets run on
      * devices[0] only, as mpc_b200.h documents */
     mpcb200_handle* dev[8];
@@ -1610,6 +1617,13 @@ int mpcb200_rollout_frenet(mpcb200_handle* h, int64_t B, int32_t T, const double
                            double target_vel, int32_t ey_from_path, double* log, double* final_state) {
     return rollout_impl(h, {"mpcb200_rollout_frenet", 1, B, T, pose0, path_of, target_vel, 0, nullptr, window, ey_from_path, log, final_state,
                             nullptr});
+}
+
+int mpcb200_rollout_frenet_w(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, double window,
+                             double target_vel, int32_t ey_from_path, const double* w, double* log, double* final_state, double* metrics) {
+    if (h && !w && B > 0 && T > 0) return fail(h, MPCB200_EINVAL, "mpcb200_rollout_frenet_w: w is required");
+    return rollout_impl(h, {"mpcb200_rollout_frenet_w", 1, B, T, pose0, path_of, target_vel, 0, w, window, ey_from_path, log, final_state,
+                            metrics});
 }
 
 int mpcb200_rollout_metrics(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of, int32_t track_using_time,

@@ -2415,7 +2415,8 @@ inline void cubic_fit_matrix(int n, double step, double* P) {
 // fitted cubics every 0.25 m fitted by a cubic (:44-58), psi_start = atan2(Y'(0), X'(0)) (:84) and e_y.  Both least-squares fits are
 // the host-built matrices P1, P2 times the samples: lanes stride the samples, the partial sums are reduced over the warp.  Used by
 // the fused closed-loop kernel (rollout_group_frenet) and by the per-period pipeline (rollout_frenet_ref_kernel).
-MPC_DEV void frenet_reference(TeamSolver<1, 1>& S, const PathTable& path, const FrenetRolloutArgs& a, double X, double Y, double yaw,
+template <int PW = 0>
+MPC_DEV void frenet_reference(TeamSolver<1, 1, PW>& S, const PathTable& path, const FrenetRolloutArgs& a, double X, double Y, double yaw,
                               double kc[4], double& ey, double& psi0, int* bi_out = nullptr) {
     const int k = S.k;
     const int bi = S.nearest_sample(path, X, Y);
@@ -2452,11 +2453,13 @@ MPC_DEV void frenet_reference(TeamSolver<1, 1>& S, const PathTable& path, const 
 }
 
 // MET = 1 (mpcb200_rollout_frenet_metrics): the nearest sample of frenet_reference also feeds metrics_update, once per period, into
-// met = [MET_K][B] (an argument of its own: rollout_frenet_ref_kernel takes FrenetRolloutArgs by value, which therefore keeps its size)
-template <int MET = 0>
+// met = [MET_K][B] (an argument of its own: rollout_frenet_ref_kernel takes FrenetRolloutArgs by value, which therefore keeps its size).
+// PW = 1 (mpcb200_rollout_frenet_w): each vehicle's cost weights from wrow = [B][7] (row_weight; an argument of its own for the same
+// reason), staged behind the team's area at wt_offset(N, 1), slot 0 (no weight on s) = 0
+template <int MET = 0, int PW = 0>
 MPC_DEV void rollout_group_frenet(const KCfg& cfg, const FrenetRolloutArgs& a, long b0, smem_t smem, smem_t px, int nwarps,
-                                  double* met = nullptr) {
-    TeamSolver<1, 1> S(cfg, smem);
+                                  double* met = nullptr, const double* wrow = nullptr) {
+    TeamSolver<1, 1, PW> S(cfg, smem);
     const int k = S.k, N = cfg.N;
     const int w = thread_in_block() >> 5;
     const long b = b0 + w;
@@ -2464,6 +2467,7 @@ MPC_DEV void rollout_group_frenet(const KCfg& cfg, const FrenetRolloutArgs& a, l
     const int pxw = SO(w * ROLLOUT_PX);
     const PathTable& path = a.paths[valid ? a.path_of[b] : 0];
     if (k < 8) sts(px, pxw + SO(k), (valid && k < 3) ? a.pose0[3 * b + k] : 0.0);
+    if (PW && k < 8) sts(smem, SO(wt_offset(N, 1) + k), (valid && wrow) ? row_weight(wrow, b, k, 1) : cfg.w[k]);   // the vehicle keeps its row
     double st[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     double acc_des = 0.0, df_des = 0.0, up_d = 0.0, up_a = 0.0;
     S.L.sx = S.L.sy = S.L.sp = S.L.sv = S.L.ua = S.L.ud = 0.0;   // start = 0.0, then the previous solution
