@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define MPCB200_VERSION 5
+#define MPCB200_VERSION 6
 
 /* error codes */
 #define MPCB200_OK          0
@@ -259,7 +259,8 @@ int mpcb200_rollout_metrics(mpcb200_handle* h, int64_t B, int32_t T, const doubl
  *       update_current_input(c_swa, c_acc) (:151-154)        -> u_prev   [B][2]
  *       solve_model() (:173-183)                             -> u0 [B][2] (acc, d_f), status, cost, iters
  *       get_solver_results() (:188-207)                      -> traj [B][6N+4] = s[N+1], ey[N+1], v[N+1], epsi[N+1], d_f[N], acc[N]
- *   warm as in mpcb200_solve_batch.  mpcb200_solve_batch / _on_path / _rollout refuse a Frenet handle.
+ *   warm as in mpcb200_solve_batch.  mpcb200_solve_batch / _on_path / _rollout refuse a Frenet handle; the Frenet form of
+ *   _on_path is mpcb200_solve_batch_frenet_on_path below.
  */
 int mpcb200_create_frenet(mpcb200_handle** out, const mpcb200_config* cfg);
 int mpcb200_set_cost_frenet(mpcb200_handle* h, const double w[7]);
@@ -298,6 +299,34 @@ int mpcb200_rollout_frenet_metrics(mpcb200_handle* h, int64_t B, int32_t T, cons
 int mpcb200_rollout_frenet_w(mpcb200_handle* h, int64_t B, int32_t T, const double* pose0, const int32_t* path_of,
                              double window, double target_vel, int32_t ey_from_path, const double* w,
                              double* log, double* final_state, double* metrics);
+
+/*
+ * Frenet-frame batch from vehicle poses, the open-loop form of one period of mpcb200_rollout_frenet: for each problem the node's
+ * reference step (gazebo_sim_mpc_cmd_pub_frenet.jl:112-130 with nav_msgs_path_frenet.py:44-86: nearest path sample, the next
+ * `window` metres resampled every 0.5 m in the vehicle frame, cubic fits of X(s) and Y(s), their curvature every 0.25 m fitted
+ * by a cubic, psi_start and e_y) computed on the device exactly as mpcb200_rollout_frenet computes it, then the solve.  Replaces
+ * the node's get_reference_frenet + update_init_cond / update_reference / update_current_input + solve_model sequence.
+ *   pose          [B][4]  X, Y, psi, v (the node's state_est)
+ *   path_of       [B]     path ids given to mpcb200_set_path
+ *   window        length of the path ahead in metres, in [4, 500]; target_vel, ey_from_path as in mpcb200_rollout_frenet
+ *   v_des         [B] or NULL = target_vel for every problem
+ *   u_prev, warm, u0, cost, status, iters, traj as in mpcb200_solve_batch_frenet
+ *   w             [B][7] Frenet weight rows as in mpcb200_solve_batch_frenet_w, or NULL = the handle's weights
+ *   k_coeffs_out  [B][4] or NULL: K(s), highest degree first
+ *   state_out     [B][4] or NULL: (0, e_y, -psi_start, v) as given to the solver
+ * u0, cost, status, iters, traj and warm are bit-identical to those of mpcb200_solve_batch_frenet (or _w with w) called with the
+ * returned state_out and k_coeffs_out: the solve is the same kernel in the same layout on those rows.  pose, path_of, u_prev and
+ * u0 are required; any horizon of a Frenet handle; host pointers are sliced over a multi-GPU handle like every host solve call,
+ * device pointers run on devices[0].  A handle from mpcb200_create and a window outside [4, 500] (or NaN) are MPCB200_EINVAL.
+ * With MPCB200_HOST pointers an unset path id or a negative or NaN weight is refused (MPCB200_EINVAL, naming the problem); with
+ * MPCB200_DEVICE pointers that problem alone comes back with status MPCB200_ERROR, zero commands, cost 0 and 0 iterations, and
+ * for an unset path id NaN in its k_coeffs_out and state_out rows.  Three kernel launches (reference, solve, answers for unset ids).
+ */
+int mpcb200_solve_batch_frenet_on_path(mpcb200_handle* h, int64_t B, const double* pose, const int32_t* path_of,
+                                       double window, double target_vel, int32_t ey_from_path,
+                                       const double* v_des, const double* u_prev, double* warm, const double* w,
+                                       double* u0, double* cost, int32_t* status, int32_t* iters, double* traj,
+                                       double* k_coeffs_out, double* state_out, int32_t mem_space);
 
 /* Counters of the last solve_batch/rollout call on this handle. */
 typedef struct {

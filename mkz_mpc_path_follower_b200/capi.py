@@ -67,6 +67,7 @@ def lib():
     L.mpcb200_solve_batch_frenet.argtypes = [vp, C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int32]
     L.mpcb200_solve_batch_frenet_w.argtypes = [vp, C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int32]
     L.mpcb200_solve_batch_on_path.argtypes = [vp, C.c_int64, vp, vp, C.c_int32, C.c_double, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, C.c_int32]
+    L.mpcb200_solve_batch_frenet_on_path.argtypes = [vp, C.c_int64, vp, vp, C.c_double, C.c_double, C.c_int32] + [vp] * 11 + [C.c_int32]
     L.mpcb200_set_path.argtypes = [vp, C.c_int32, C.c_int32, dp, dp, dp, dp, dp]
     L.mpcb200_rollout.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_int32, C.c_double, dp, dp]
     L.mpcb200_rollout_w.argtypes = [vp, C.c_int64, C.c_int32, dp, ip, C.c_int32, C.c_double, dp, dp, dp]
@@ -401,6 +402,55 @@ class FrenetSolver(Solver):
             return {"log": log, "final_state": final, "metrics": met}
         self._check(lib().mpcb200_rollout_frenet(self._h, B, int(T), *args))
         return {"log": log, "final_state": final}
+
+    def solve_batch_on_path(self, pose, path_of, u_prev, window=40.0, target_vel=8.0, ey_from_path=True, v_des=None, warm=None,
+                            want_traj=False, want_ref=False, weights=None):
+        """mpcb200_solve_batch_frenet_on_path: the node's reference step (nearest sample, the next `window` metres of the path set
+        with set_path, the curvature fit, psi_start, e_y) on the device from each pose, then the solve.  pose (B,4) = X, Y, psi, v;
+        path_of (B,) ids given to set_path; v_des (B,) or None = target_vel; warm, weights as in solve_batch.  Returns the
+        solve_batch dict; with want_ref also "k_coeffs" (B,4) and "state" (B,4) = (0, e_y, -psi_start, v), the solver's inputs."""
+        N = self.N
+        pose = np.ascontiguousarray(pose, dtype=np.float64)
+        B = pose.shape[0]
+        path_of = np.ascontiguousarray(path_of, dtype=np.int32)
+        u_prev = np.ascontiguousarray(u_prev, dtype=np.float64)
+        if pose.shape != (B, 4) or path_of.shape != (B,) or u_prev.shape != (B, 2):
+            raise ValueError("solve_batch_on_path: expected pose (B,4), path_of (B,), u_prev (B,2)")
+        if v_des is not None:
+            v_des = np.ascontiguousarray(v_des, dtype=np.float64)
+            if v_des.shape != (B,):
+                raise ValueError("solve_batch_on_path: v_des must be (B,)")
+        if warm is not None:
+            if not (isinstance(warm, np.ndarray) and warm.dtype == np.float64 and warm.flags.c_contiguous
+                    and warm.shape == (B, 6 * N + 4)):
+                raise ValueError("solve_batch_on_path: warm must be a C-contiguous float64 (B,6N+4) array (updated in place)")
+        w = None if weights is None else _weight_rows(weights, B, 7, "solve_batch_on_path")
+        u0 = np.empty((B, 2)); cost = np.empty(B)
+        status = np.empty(B, dtype=np.int32); iters = np.empty(B, dtype=np.int32)
+        traj = np.empty((B, 6 * N + 4)) if want_traj else None
+        k_coeffs = np.empty((B, 4)) if want_ref else None
+        state = np.empty((B, 4)) if want_ref else None
+        self._check(lib().mpcb200_solve_batch_frenet_on_path(self._h, B, _ptr(pose), _ptr(path_of), float(window), float(target_vel),
+                                                             int(bool(ey_from_path)), _ptr(v_des), _ptr(u_prev), _ptr(warm), _ptr(w),
+                                                             _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj),
+                                                             _ptr(k_coeffs), _ptr(state), HOST))
+        out = {"u0": u0, "cost": cost, "status": status, "iters": iters, "traj": traj}
+        if want_ref:
+            out["k_coeffs"] = k_coeffs
+            out["state"] = state
+        return out
+
+    def solve_batch_on_path_device(self, B, pose, path_of, u_prev, u0, window=40.0, target_vel=8.0, ey_from_path=True, v_des=None,
+                                   warm=None, cost=None, status=None, iters=None, traj=None, k_coeffs_out=None, state_out=None,
+                                   weights=None):
+        """solve_batch_on_path with device pointers (torch CUDA tensors, float64 / int32, contiguous); only enqueues on the
+        handle's stream.  An unset path id or a bad weight row gives that problem status ERROR (and, for the path id, NaN rows in
+        k_coeffs_out / state_out)."""
+        w = None if weights is None else _weight_rows_device(weights, B, 7, "solve_batch_on_path_device")
+        self._check(lib().mpcb200_solve_batch_frenet_on_path(self._h, B, _ptr(pose), _ptr(path_of), float(window), float(target_vel),
+                                                             int(bool(ey_from_path)), _ptr(v_des), _ptr(u_prev), _ptr(warm), _ptr(w),
+                                                             _ptr(u0), _ptr(cost), _ptr(status), _ptr(iters), _ptr(traj),
+                                                             _ptr(k_coeffs_out), _ptr(state_out), DEVICE))
 
     def solve_batch_device(self, B, state, k_coeffs, u_prev, u0, v_des=None, warm=None, cost=None, status=None, iters=None, traj=None,
                            weights=None):

@@ -300,6 +300,23 @@ rollout_frenet_ref_kernel(const KCfg cfg, const FrenetRolloutArgs a, const long 
     }
 }
 
+// ---- mpcb200_solve_batch_frenet_on_path: the reference of every problem first (warp = problem, frenet_on_path_problem: the
+// node's reference step from the pose) into k_out / state_out = [B][4]; the solve kernels then read those rows as an ordinary
+// Frenet batch (launch_solve), so the results are those of mpcb200_solve_batch_frenet on the returned inputs by construction.
+// vdes_out [B] or null: target_vel for every problem when the caller gives no v_des.  The reference is not fused into the solve
+// kernels: that would be a new build of every (WPB, PW) and long-team solve instantiation (DESIGN §3.4).
+__global__ void __launch_bounds__(128)
+on_path_frenet_ref_kernel(const KCfg cfg, const FrenetRolloutArgs a, const double* pose, double* k_out, double* state_out,
+                          double* vdes_out, const double target_vel) {
+    const long long warps = ((long long)gridDim.x * blockDim.x) >> 5;
+    TeamSolver<1, 1> S(cfg, (smem_t)0);   // (one-warp teams: collectives are shuffles only)
+    for (long long b = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; b < a.B; b += warps) {
+        frenet_on_path_problem(S, a, pose, (long)b, k_out, state_out);
+        if (vdes_out && (threadIdx.x & 31) == 0) vdes_out[b] = target_vel;
+        __syncwarp();
+    }
+}
+
 __global__ void rollout_final_kernel(const long long B, const long long Bp, const double* veh, double* final_state) {
     const long long v = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (v >= B) return;
@@ -948,15 +965,22 @@ struct SolveArgs {
     double* u0; double* cost; int32_t* status; int32_t* iters; double* traj;
     double* ref_out; int32_t* stop; double* rec;
     const double* w;   /* [B][8] ([B][7] Frenet) per-problem weights, or NULL: the handle's */
+    /* mpcb200_solve_batch_frenet_on_path (frenet_on_path set; state and ref are NULL): the poses [B][4], the length of the path
+     * ahead, e_y from the path or 0, and where K(s) and the solver's state go ([B][4] each, or NULL) */
+    const double* pose; double window; int32_t ey_from_path;
+    double* k_out; double* state_out;
+    bool frenet_on_path;
 };
 
 /* doubles per weight row of a handle's model */
 static size_t weight_row(int model) { return model ? 7 : 8; }
 
 /* The per-problem arrays of a solve call, one table entry each.  The order is that of the packed small-batch layout
- * (solve_small_host): inputs, then warm (in and out), then outputs. */
+ * (solve_small_host): inputs, then warm (in and out), then outputs.  The last three belong to mpcb200_solve_batch_frenet_on_path
+ * only, which never takes the packed path; the other calls never give them, so they leave the packed layout and the graph
+ * key of those calls as they were. */
 enum ArrayId { A_STATE, A_REF, A_PATH_OF, A_U_PREV, A_V_DES, A_W, A_WARM, A_U0, A_COST, A_TRAJ, A_STATUS, A_ITERS, A_REC, A_REF_OUT, A_STOP,
-               A_COUNT };
+               A_POSE, A_K_OUT, A_STATE_OUT, A_COUNT };
 enum { DIR_IN = 1, DIR_OUT = 2, DIR_INOUT = 3 };
 /* an array's slot in the packed small-batch layout: there when the caller gives the array (PACK_GIVEN); always there and
  * copied, the kernel getting it only when given (PACK_SLOT); always there and always written by the kernel (PACK_ALWAYS), so
@@ -991,6 +1015,9 @@ static void call_arrays(mpcb200_handle* h, const SolveArgs& a, int64_t lo, CallA
         {(char*)a.rec, 4 * d, DIR_OUT, PACK_GIVEN, &h->d_rec},
         {(char*)a.ref_out, nr, DIR_OUT, PACK_GIVEN, &h->d_ref},
         {(char*)a.stop, i4, DIR_OUT, PACK_GIVEN, &h->d_stop},
+        {(char*)a.pose, 4 * d, DIR_IN, PACK_GIVEN, &h->d_pose},
+        {(char*)a.k_out, 4 * d, DIR_OUT, PACK_GIVEN, &h->d_ref},       /* (the call has no ref and no state) */
+        {(char*)a.state_out, 4 * d, DIR_OUT, PACK_GIVEN, &h->d_state},
     };
     for (int i = 0; i < A_COUNT; i++) {
         t[i] = all[i];
@@ -1004,6 +1031,61 @@ static BatchPtrs batch_ptrs(void* const p[A_COUNT], int* resto, RefGen& rg) {
     return BatchPtrs{(const double*)p[A_STATE], (const double*)p[A_REF], (const double*)p[A_V_DES], (const double*)p[A_U_PREV],
                      (double*)p[A_WARM], (double*)p[A_U0], (double*)p[A_COST], (int*)p[A_STATUS], (int*)p[A_ITERS], (double*)p[A_TRAJ],
                      (double*)p[A_REC], resto, (const double*)p[A_W]};
+}
+
+/* The two least-squares fit matrices of the Frenet reference on this handle's device, [4][n1] then [4][n2] in d_fit, rebuilt and
+ * uploaded when the window changes: grids of nav_msgs_path_frenet.py:63,79, arange(0, window, 0.5) and arange(0, window, 0.25) */
+static int ensure_fit(mpcb200_handle* h, const char* who, double window) {
+    if (h->fit_window == window) return MPCB200_OK;
+    int n1, n2, rc;
+    fit_grid_sizes(window, &n1, &n2);
+    double* P = (double*)malloc(sizeof(double) * 4 * ((size_t)n1 + n2));
+    if (!P) return fail(h, MPCB200_ENOMEM, "%s: out of host memory", who);
+    cubic_fit_matrix(n1, 0.5, P); cubic_fit_matrix(n2, 0.25, P + 4 * (size_t)n1);
+    rc = ensure(h, h->d_fit, sizeof(double) * 4 * ((size_t)n1 + n2));
+    if (!rc) {
+        cudaError_t e = cudaMemcpyAsync(h->d_fit.p, P, sizeof(double) * 4 * ((size_t)n1 + n2), cudaMemcpyHostToDevice, h->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+        if (e != cudaSuccess) rc = fail(h, MPCB200_ECUDA, "%s: %s", who, cudaGetErrorString(e));
+    }
+    free(P);
+    if (rc) return rc;
+    h->fit_window = window; h->fit_n1 = n1; h->fit_n2 = n2;
+    return MPCB200_OK;
+}
+
+/* mpcb200_solve_batch_frenet_on_path on one device: on_path_frenet_ref_kernel, launch_solve on the rows it wrote (an ordinary
+ * Frenet batch: the kernel and layout mpcb200_solve_batch_frenet would take), then on_path_invalid_kernel for the problems whose
+ * path id was never set.  p: the call's arrays on this device, io / rg as batch_ptrs made them from p (rg: this device's tables) */
+static int launch_frenet_on_path(mpcb200_handle* h, int64_t B, const SolveArgs& a, void* const p[A_COUNT], BatchPtrs io, const RefGen& rg) {
+    int rc;
+    if ((rc = ensure_fit(h, a.who, a.window))) return rc;
+    const size_t rows = (size_t)B * 4 * sizeof(double);
+    double* k_out = (double*)p[A_K_OUT];
+    double* state_out = (double*)p[A_STATE_OUT];
+    double* vdes = nullptr;
+    if (!k_out) { if ((rc = ensure(h, h->d_ref, rows))) return rc; k_out = (double*)h->d_ref.p; }
+    if (!state_out) { if ((rc = ensure(h, h->d_state, rows))) return rc; state_out = (double*)h->d_state.p; }
+    if (!io.v_des) { if ((rc = ensure(h, h->d_vdes, (size_t)B * sizeof(double)))) return rc; vdes = (double*)h->d_vdes.p; }
+    FrenetRolloutArgs fa;
+    memset(&fa, 0, sizeof(fa));
+    for (int i = 0; i < 3; i++) fa.paths[i] = rg.paths[i];
+    fa.path_of = rg.path_of; fa.B = (long)B; fa.ey_from_path = a.ey_from_path;
+    fa.P1 = (const double*)h->d_fit.p; fa.P2 = fa.P1 + 4 * (size_t)h->fit_n1; fa.n1 = h->fit_n1; fa.n2 = h->fit_n2;
+    const long long wblocks = (B + 3) / 4, wmax = (long long)h->num_sms * 16;
+    on_path_frenet_ref_kernel<<<(int)(wblocks < wmax ? wblocks : wmax), 128, 0, h->stream>>>(make_kcfg(h), fa, (const double*)p[A_POSE],
+                                                                                             k_out, state_out, vdes, a.target_vel);
+    CUDA_TRY(h, cudaGetLastError());
+    h->stats.kernel_launches += 1;
+    io.state = state_out; io.ref = k_out;
+    if (vdes) io.v_des = vdes;
+    RefGen none;
+    memset(&none, 0, sizeof(none));
+    if ((rc = launch_solve(h, B, io, none))) return rc;
+    on_path_invalid_kernel<<<(int)((B + 127) / 128), 128, 0, h->stream>>>((long long)B, rg, io);
+    CUDA_TRY(h, cudaGetLastError());
+    h->stats.kernel_launches += 1;
+    return MPCB200_OK;
 }
 
 /* contiguous slice of `total` owned by part `i` of `parts`; sizes differ by at most one (same rule as sharding.shard_range) */
@@ -1166,7 +1248,7 @@ static int host_enqueue(mpcb200_handle* h, int64_t B, const SolveArgs& a, int64_
     if (a.path_of) fill_paths(h, rg.paths);   /* this device's copies of the tables */
     const BatchPtrs io = batch_ptrs(p, (int*)h->d_resto.p, rg);
     CUDA_TRY(h, cudaEventRecord(h->ev0, s));
-    if ((rc = launch_solve(h, B, io, rg))) return rc;
+    if ((rc = a.frenet_on_path ? launch_frenet_on_path(h, B, a, p, io, rg) : launch_solve(h, B, io, rg))) return rc;
     CUDA_TRY(h, cudaEventRecord(h->ev1, s));
     return MPCB200_OK;
 }
@@ -1195,7 +1277,8 @@ static int sub_fail(mpcb200_handle* h, mpcb200_handle* d, int rc) {
     return rc;
 }
 
-/* common body of mpcb200_solve_batch* (ref given) and mpcb200_solve_batch_on_path (path_of given) */
+/* common body of mpcb200_solve_batch* (ref given), mpcb200_solve_batch_on_path (path_of given) and mpcb200_solve_batch_frenet_on_path
+ * (pose and path_of given) */
 static int solve_batch_impl(mpcb200_handle* h, int64_t B, const SolveArgs& a, int32_t mem_space) {
     const char* who = a.who;
     if (!h) return MPCB200_EINVAL;
@@ -1205,9 +1288,11 @@ static int solve_batch_impl(mpcb200_handle* h, int64_t B, const SolveArgs& a, in
     h->last_B = B; h->last_sharded = false; h->resto_on_host = false;
     if (B == 0) return MPCB200_OK;
     const bool on_path = (a.path_of != nullptr);
-    if (!a.state || (!a.ref && !on_path) || !a.u_prev || (!a.u0 && !a.rec))
+    if (a.frenet_on_path) {
+        if (!a.pose || !a.path_of || !a.u_prev || !a.u0) return fail(h, MPCB200_EINVAL, "%s: pose, path_of, u_prev and u0 are required", who);
+    } else if (!a.state || (!a.ref && !on_path) || !a.u_prev || (!a.u0 && !a.rec))
         return fail(h, MPCB200_EINVAL, "%s: state, %s, u_prev and %s are required", who, on_path ? "path_of" : "ref", a.rec ? "rec" : "u0");
-    if (on_path && h->model) return fail(h, MPCB200_EINVAL, "%s: not available for the Frenet-frame variant", who);
+    if (on_path && h->model && !a.frenet_on_path) return fail(h, MPCB200_EINVAL, "%s: not available for the Frenet-frame variant", who);
     int rc;
     if (a.w && mem_space == MPCB200_HOST && (rc = check_weight_rows(h, who, "problem", B, a.w, weight_row(h->model)))) return rc;
     CUDA_TRY(h, cudaSetDevice(h->device));
@@ -1226,7 +1311,7 @@ static int solve_batch_impl(mpcb200_handle* h, int64_t B, const SolveArgs& a, in
         void* p[A_COUNT];
         for (int i = 0; i < A_COUNT; i++) p[i] = t[i].host;
         const BatchPtrs io = batch_ptrs(p, (int*)h->d_resto.p, rg);
-        return launch_solve(h, B, io, rg);
+        return a.frenet_on_path ? launch_frenet_on_path(h, B, a, p, io, rg) : launch_solve(h, B, io, rg);
     }
     if (!on_path && B <= SMALL_BATCH) return solve_small_host(h, B, a);
     mpcb200_handle* dev[8];
@@ -1338,6 +1423,18 @@ int mpcb200_solve_batch_on_path(mpcb200_handle* h, int64_t B, const double* stat
     return solve_batch_impl(h, B, a, mem_space);
 }
 
+int mpcb200_solve_batch_frenet_on_path(mpcb200_handle* h, int64_t B, const double* pose, const int32_t* path_of, double window,
+                                       double target_vel, int32_t ey_from_path, const double* v_des, const double* u_prev, double* warm,
+                                       const double* w, double* u0, double* cost, int32_t* status, int32_t* iters, double* traj,
+                                       double* k_coeffs_out, double* state_out, int32_t mem_space) {
+    const char* who = "mpcb200_solve_batch_frenet_on_path";
+    if (h && !h->model) return fail(h, MPCB200_EINVAL, "%s: the handle was not created with mpcb200_create_frenet", who);
+    if (h && !(window >= 4.0 && window <= 500.0)) return fail(h, MPCB200_EINVAL, "%s: window %.3g m outside [4, 500]", who, window);
+    const SolveArgs a{who, nullptr, nullptr, path_of, 0, target_vel, v_des, u_prev, warm, u0, cost, status, iters, traj, nullptr, nullptr,
+                      nullptr, w, pose, window, ey_from_path, k_coeffs_out, state_out, true};
+    return solve_batch_impl(h, B, a, mem_space);
+}
+
 int mpcb200_set_path(mpcb200_handle* h, int32_t path_id, int32_t n, const double* t, const double* X, const double* Y,
                      const double* psi, const double* s) {
     if (!h) return MPCB200_EINVAL;
@@ -1422,22 +1519,7 @@ static int rollout_enqueue(mpcb200_handle* h, const RolloutCall& c, int64_t lo, 
     cudaStream_t s = h->stream;
     int rc;
     if (!c.model && (rc = ensure_seed(h))) return rc;
-    if (c.model && h->fit_window != c.window) {   /* grids of nav_msgs_path_frenet.py:63,79: arange(0, window, 0.5) and arange(0, window, 0.25) */
-        int n1, n2;
-        fit_grid_sizes(c.window, &n1, &n2);
-        double* P = (double*)malloc(sizeof(double) * 4 * ((size_t)n1 + n2));
-        if (!P) return fail(h, MPCB200_ENOMEM, "%s: out of host memory", c.who);
-        cubic_fit_matrix(n1, 0.5, P); cubic_fit_matrix(n2, 0.25, P + 4 * (size_t)n1);
-        rc = ensure(h, h->d_fit, sizeof(double) * 4 * ((size_t)n1 + n2));
-        if (!rc) {
-            cudaError_t e = cudaMemcpyAsync(h->d_fit.p, P, sizeof(double) * 4 * ((size_t)n1 + n2), cudaMemcpyHostToDevice, s);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-            if (e != cudaSuccess) rc = fail(h, MPCB200_ECUDA, "%s: %s", c.who, cudaGetErrorString(e));
-        }
-        free(P);
-        if (rc) return rc;
-        h->fit_window = c.window; h->fit_n1 = n1; h->fit_n2 = n2;
-    }
+    if (c.model && (rc = ensure_fit(h, c.who, c.window))) return rc;
     if ((rc = ensure(h, h->d_pose, (size_t)n * 3 * sizeof(double)))) return rc;
     if ((rc = ensure(h, h->d_pathof, (size_t)n * sizeof(int32_t)))) return rc;
     if (c.log && (rc = ensure(h, h->d_log, (size_t)c.T * n * 8 * sizeof(double)))) return rc;

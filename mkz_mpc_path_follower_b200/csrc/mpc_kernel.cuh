@@ -2452,6 +2452,28 @@ MPC_DEV void frenet_reference(TeamSolver<1, 1, PW>& S, const PathTable& path, co
     ey = a.ey_from_path ? -(-sp0 * xw0 + cp0 * yw0) : 0.0;
 }
 
+// mpcb200_solve_batch_frenet_on_path, one problem (warp = problem; on_path_frenet_ref_kernel): frenet_reference on the pose
+// (X, Y, psi, v) = pose[4b..4b+3] and path a.paths[a.path_of[b]], then K(s) into k_out[4b..] and the solver's state
+// (0, e_y, -psi_start, v) into state_out[4b..] -- the inputs of update_init_cond / update_reference
+// (gazebo_sim_mpc_cmd_pub_frenet.jl:125-126).  A path id that was never set gives NaN in both rows (on_path_invalid_kernel
+// answers the problem after the solve).  Of `a` only paths, path_of, P1, P2, n1, n2 and ey_from_path are read.
+MPC_DEV void frenet_on_path_problem(TeamSolver<1, 1>& S, const FrenetRolloutArgs& a, const double* pose, long b, double* k_out,
+                                    double* state_out) {
+    const int k = S.k;
+    const int pid = a.path_of[b];
+    double cv[8];
+    for (int i = 0; i < 8; i++) cv[i] = nan("");
+    if (!(pid < 0 || pid > 2 || a.paths[pid].n < 2)) {
+        const double* p = pose + 4 * b;
+        double kc[4], ey, psi0;
+        frenet_reference(S, a.paths[pid], a, p[0], p[1], p[2], kc, ey, psi0);
+        cv[0] = kc[0]; cv[1] = kc[1]; cv[2] = kc[2]; cv[3] = kc[3];
+        cv[4] = 0.0; cv[5] = ey; cv[6] = -psi0; cv[7] = p[3];
+    }
+    if (k < 4) k_out[4 * b + k] = sel8(cv, k);
+    else if (k < 8) state_out[4 * b + (k - 4)] = sel8(cv, k);
+}
+
 // MET = 1 (mpcb200_rollout_frenet_metrics): the nearest sample of frenet_reference also feeds metrics_update, once per period, into
 // met = [MET_K][B] (an argument of its own: rollout_frenet_ref_kernel takes FrenetRolloutArgs by value, which therefore keeps its size).
 // PW = 1 (mpcb200_rollout_frenet_w): each vehicle's cost weights from wrow = [B][7] (row_weight; an argument of its own for the same
